@@ -13,16 +13,25 @@ Prints ONE JSON line (contract in the task statement): value = device-resident t
 e2e = the same cycle through the public API with frames in pinned HOST memory (H2D of every
 frame and D2H of the actions/loss inside the timed region), roofline = the dominant kernel
 timed live with CUDA events, cpu_baseline = the CPU port of the reference path on this box.
+
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+also writes what the last timed cycle of the device-resident arm computed as DIR/<name>.npy
+(see dump_outputs).  Frames, weights, random starts and action draws are all seeded, so the same
+arguments give the same inputs on every run and two builds can be compared output for output.
 """
 import argparse
 import importlib
 import json
 import os
+import random
 import statistics
 import subprocess
 import sys
 import threading
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -188,6 +197,34 @@ def run_reference(args, rank):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, net, T, B, A):
+    """Write what one A3C cycle hands back, float32, as out_dir/<name>.npy: the actions sampled at
+    its t_max env steps, the logits / policy / values of its rollout forward ([T, B, ...]), the
+    loss sums, the gradient its backward produced and the parameters and RMSProp state its update
+    left.  Above DUMP_BYTES in all, the per-env arrays keep a fixed, seeded sample of the envs,
+    whose indices go to env_index.npy.  The loss sums are accumulated with float atomics, so they
+    may differ in the last bits from run to run; the other arrays repeat bit for bit."""
+    out = {"params": net.params, "rms": net.rms, "grads": net.grads, "loss_sums": net.loss_sums}
+    out = {k: v.float().cpu().numpy() for k, v in out.items()}
+    rollout = {"actions": net.sampled_action.view(T, B), "logits": net.policy_logits.view(T, B, A),
+               "policy": net.policy.view(T, B, A), "value": net.value.view(T, B)}
+    rollout = {k: v.float().cpu().numpy() for k, v in rollout.items()}
+    fixed = sum(v.nbytes for v in out.values()) + 4096                # + room for the .npy headers
+    per_env = sum(v[:, :1].nbytes for v in rollout.values())
+    if fixed + B * per_env > DUMP_BYTES:
+        keep = (DUMP_BYTES - fixed) // (per_env + 8)
+        idx = np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+        rollout = {k: v[:, idx] for k, v in rollout.items()}
+        out["env_index"] = idx.astype(np.float64)
+    out.update(rollout)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def workload_config(args, ref=False):
     return {"workload": "A3C full update, %d envs/GPU, conv16-conv32-fc256, %d-action head, "
                         "t_max %d, history 4, shared RMSProp (BASELINE.json configs[2]/[3])"
@@ -220,7 +257,13 @@ def main():
     ap.add_argument("--collective", default=None, choices=[None, "auto", "p2p", "library", "torch"],
                     help="gradient exchange at N>1 (default: config.collective = auto)")
     ap.add_argument("--pool", type=int, default=0, help="steps of synthetic frames kept (0: t_max, capped to ~24 GB)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -283,6 +326,7 @@ def main():
         env = pkg.GymEnvironment(cfg, env=pkg.SyntheticAtari(B, A, seed=123 + rank, pool=pool,
                                                              device=dev, host=host), device=dev)
         agent = pkg.Agent(cfg, env, device=dev)
+        random.seed(cfg.seed)                    # the random-start no-ops of new_random_game
         agent.before_train()
         return agent, env
 
@@ -458,6 +502,8 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     ms_total, launches, replays = timed(agent, env, sampler=sampler)
     clocks = sampler.finish() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, net, T, B, A)
     value = world * B * T * K / (ms_total * 1e-3)
     timed_in = "timed region (K1 launched between events, everything else replayed from CUDA graphs)"
     if dominant == "arl_preprocess_push" and in_graph and k1_graph_events:
