@@ -60,7 +60,7 @@ constexpr int64_t kPrepW1 = kPrepFcW + kPrepFcWBytes;             // conv1 fwd: 
 constexpr int64_t kPrepW1Bytes = 12800;
 constexpr int64_t kPrepW2F = kPrepW1 + kPrepW1Bytes;              // conv2 fwd: [hi | lo] image | bias
 constexpr int64_t kPrepW2FBytes = 33408;
-constexpr int64_t kPrepW2D = kPrepW2F + kPrepW2FBytes;            // conv2 dgrad: transposed [hi | lo] image
+constexpr int64_t kPrepW2D = kPrepW2F + kPrepW2FBytes;            // conv2 bwd: transposed fp16 [hi | lo] image
 constexpr int64_t kPrepW2DBytes = 33024;
 constexpr int64_t kPrepFcWT = kPrepW2D + kPrepW2DBytes;           // l4_w TRANSPOSED as a split block [256 rows][2592]
 constexpr int64_t kPrepBytes = kPrepFcWT + kPrepFcWBytes;

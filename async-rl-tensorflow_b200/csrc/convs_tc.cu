@@ -12,13 +12,16 @@
 //
 //   conv1 fwd  : X rows from the u8 ring (exact in bf16 -> hi image only), W1 resident
 //   conv2 fwd  : X2 rows from a1 (bf16 hi+lo), W2 resident
-//   conv2 dgrad: the transposed conv.  Output pixels of one parity class (y&1, x&1) use 4 taps
-//                of the zero-padded dy2 grid Z[11,11,32]; the 4 classes share the Z image and
-//                differ only in the resident weights -> 4 accumulator sets per stage
+//   conv2 bwd  : ONE kernel, one dy2 image (fp16 hi+lo) per tile serves both MMAs.  Input
+//                gradient = the transposed conv: output pixels of one parity class (y&1, x&1) use
+//                4 taps of dy2 on the X2 grid itself (its zero rows are the padding); the 4 classes
+//                share the image and differ only in the resident weights.  Weight gradient: see
+//                wgrads; its accumulator lives across the CTA's tiles.
 //   wgrads     : dW[(tap,ch), co] = sum_P X[P+shift][ch] * dyz[P][co] reduces over ROWS, so the
 //                same row-major images serve as MN-major operands (k = row index); tap b is a
 //                second copy of the image shifted by one row, tap a a descriptor row offset.
-//                Work is split over row ranges; partials are summed in a fixed order.
+//                Work is split over row ranges (conv1) or CTAs (conv2); partials are summed in a
+//                fixed order.
 #include <stdlib.h>
 
 #include "gemm_tc.cuh"
@@ -72,17 +75,15 @@ struct PixelGrid {
   }
 };
 
-// Streams the pixels of grid rows [z0, z0+ROWS) (rows >= z_end count as zero) into a hi/lo image
-// pair whose 16-B vector (row r, chunk kc) sits at kc*PL + r*16; FP16 chooses the element format of
-// the pair (fp16 hi + lo next to fp16 activations, bf16 hi + lo next to bf16 weights: the two
-// operands of one MMA must share a format).  U float4 loads are in flight per
-// lane before the first one is consumed (U * gsize >= the whole window => one latency per stage).
-// acc (optional) accumulates the column sums of what was stored: a lane owns floats
-// (glane % CF4)*4 .. +3 of every pixel it touches.
-template <class G, int CF4, int ROWS, int PL, int U, bool ACC, bool FP16>
+// Streams the pixels of grid rows [z0, z0+ROWS) (z0 may be negative: rows before the first sample
+// are zero) into an fp16 hi + lo image pair whose 16-B vector (row r, chunk kc) sits at
+// kc*PL + r*16.  U float4 loads are in flight per lane before the first one is consumed
+// (U * gsize >= the whole window => one latency per stage).  acc accumulates the column sums of
+// the window rows r >= SUM_FROM: a lane owns floats (glane % CF4)*4 .. +3 of every pixel it touches.
+template <class G, int CF4, int ROWS, int PL, int U, int SUM_FROM>
 __device__ __forceinline__ void stream_pixels(uint8_t* hi, uint8_t* lo, const float* __restrict__ src,
-                                              int z0, int z_end, int num_samples, int glane,
-                                              int gsize, float (&acc)[4]) {
+                                              int z0, int num_samples, int glane, int gsize,
+                                              float (&acc)[4]) {
   const int p0 = G::lower_pixel(z0);
   const int p_total = num_samples * G::PP;
   constexpr int SPAN = ROWS + 2 * G::WIDTH + 2;              // lower_pixel undershoots by <= 2*PW
@@ -102,7 +103,7 @@ __device__ __forceinline__ void stream_pixels(uint8_t* hi, uint8_t* lo, const fl
         const int z = G::grid_of_pixel(pix);
         if (z >= z0 && z < z0 + ROWS) {
           rr[u] = z - z0;
-          if (z < z_end) x[u] = __ldg(s4 + f);
+          x[u] = __ldg(s4 + f);
         }
       }
     }
@@ -110,9 +111,8 @@ __device__ __forceinline__ void stream_pixels(uint8_t* hi, uint8_t* lo, const fl
     for (int u = 0; u < U; ++u) {
       if (rr[u] < 0) continue;
       const int off = (q >> 1) * PL + rr[u] * 16 + (q & 1) * 8;
-      if (FP16) tc::store_half_split_h(hi, lo, off, x[u]);
-      else tc::store_half_split(hi, lo, off, x[u]);
-      if (ACC) { acc[0] += x[u].x; acc[1] += x[u].y; acc[2] += x[u].z; acc[3] += x[u].w; }
+      tc::store_half_split_h(hi, lo, off, x[u]);
+      if (rr[u] >= SUM_FROM) { acc[0] += x[u].x; acc[1] += x[u].y; acc[2] += x[u].z; acc[3] += x[u].w; }
     }
   }
   // rows of the window that no pixel maps to (grid padding, beyond the last sample)
@@ -128,7 +128,6 @@ __device__ __forceinline__ void stream_pixels(uint8_t* hi, uint8_t* lo, const fl
 }
 
 using GridDy2 = PixelGrid<10, 100, 9, 9, 0, 8>;       // dy2 [N,81,32] on the conv2 X2 grid
-using GridZ   = PixelGrid<11, 121, 9, 9, 1, 8>;       // dy2 zero-padded by one (transposed conv)
 
 // resident operand image: built once per parameter change by arl_prepare_weights (build_image of
 // the policy), copied into shared memory by the producer threads in the kernel prologue
@@ -206,8 +205,8 @@ __device__ __forceinline__ void x1_store(uint8_t* img, const uint4 (&w)[U], int 
 }
 
 // ---- a1 in HBM: fp16, blocked ("a1s") -----------------------------------------------------------
-// conv1's output is only ever consumed as a tensor-core operand (conv2 forward / conv2 wgrad)
-// and as a relu mask (conv2 dgrad), so it is stored the way those kernels want it -- ONE fp16 per
+// conv1's output is only ever consumed as a tensor-core operand (conv2 forward / backward) and as
+// the relu mask of conv2's input gradient, so it is stored the way those kernels want it -- ONE fp16 per
 // value (12 800 bytes per sample, half of fp32 [20,20,16]) in space-to-depth order:
 //   a1s[n][kc = (i*2+j)*2 + chalf][q = yp*10 + xp][8 channels]     (16-B vectors)
 // with pixel (y,x) = (2yp+i, 2xp+j) and channels chalf*8 .. chalf*8+7.  A run of X2 rows of one
@@ -508,18 +507,9 @@ struct Conv2Fwd : tc::PolicyBase {
   }
 };
 
-// =================================== conv2 input gradient =====================================
-struct Conv2DgradArgs {
-  const uint8_t* w_img;  // prepared: transposed bf16 [hi | lo] image of l2_w
-  const uint8_t* a1s;    // relu mask of conv1: sign of its fp16 output
-  const float* dy2;      // [N, 81, 32]
-  uint8_t* dy1s;         // conv1 output gradient, one fp16 per value on the conv1 X grid ("dy1s", see below)
-  float* bias_partials;  // [grid * 8 epilogue warps][16]: column sums of dy1 (= the conv1 bias gradient)
-  int64_t rows;          // 121 * num_samples
-  int num_samples;
-};
+// =================================== conv2 backward ===========================================
 // dy1s: the gradient w.r.t. conv1's output is only ever the B operand of the conv1 weight-gradient
-// MMA (rows of the 21-wide X grid = the reduction index), so conv2 dgrad stores it the way that
+// MMA (rows of the 21-wide X grid = the reduction index), so conv2 backward stores it the way that
 // kernel fetches it with cp.async.bulk -- ONE fp16 per value (x tensor_scale, saturating):
 //   dy1s[co group (2)][grid row n*441 + y*21 + x][8 channels]      (16-B vectors)
 // with the rows y = 20 / x = 20 (no conv1 output there) written as zeros: 14 112 B per sample.
@@ -527,124 +517,7 @@ struct Conv2DgradArgs {
 // of this kernel's epilogue), 2e-4 in tests/precision_study.py's "fp16 a1 + d_a1" row; round 1
 // kept a bf16 hi + lo pair (28 224 B).
 constexpr int kDy1sRows = 441;
-struct Conv2Dgrad : tc::PolicyBase {
-  using Args = Conv2DgradArgs;
-  static constexpr int GW = 11, GROWS = 121, TROWS = 140;
-  static constexpr int PL = 146 * 16, IMG = 4 * PL;           // 32 co = 4 chunks
-  // the relu-mask epilogue waits on HBM: two epilogue sets; 8 producer warps (17 warps in all ->
-  // 96 registers per thread, 8 float4 mask loads in flight per epilogue lane)
-  static constexpr int EPI_SETS = 2, PROD_WARPS = 8, STAGES = 4, STAGE_BYTES = 2 * IMG;
-  // resident W2^T image: rows = part*64 + cls*16 + c (N = 128: the 4 parity classes share the A
-  // tile of a tap, and lo follows hi), 16 k-chunk planes (tap*4 + co8)
-  static constexpr int PLB = 129 * 16, RES_BYTES = 16 * PLB;
-  static constexpr int ACC_COLS = 128, OUT_COLS = 64, LO_DELTA = 64, SEG = 32;   // 4 classes x 16 ch
-  static constexpr bool CUSTOM_EPI = true;
-  static __device__ __forceinline__ int acc_col(int c) { return c; }
-  static __device__ __forceinline__ int num_items(const Args& g) { return (int)((g.rows + 127) / 128); }
-  static __device__ __forceinline__ TileCoord coord(const Args&, int item) { return row_tile(item); }
-  static __device__ __forceinline__ int num_stages(const Args&, const TileCoord&) { return 1; }
-  static __device__ __forceinline__ void load_resident(const Args& g, uint8_t* res, int ptid, int nthr) {
-    copy_image<RES_BYTES>(res, g.w_img, ptid, nthr);
-  }
-  static __device__ __forceinline__ void build_image(const float* params, uint8_t* res, int ptid, int nthr) {
-    const float* w2 = params + 4112;
-    for (int ch = ptid; ch < 4 * 16 * 16; ch += nthr) {
-      const int c = ch & 15, kc = (ch >> 4) & 15, cls = ch >> 8;   // kc = tap*4 + co8
-      const int tap = kc >> 2, co8 = kc & 3;
-      const int kh = (cls >> 1) + 2 * (tap >> 1), kw = (cls & 1) + 2 * (tap & 1);
-      float x[8];
-      load8(w2 + ((kh * 4 + kw) * 16 + c) * 32 + co8 * 8, x);
-      tc::store_chunk_split(res, res + 64 * 16, kc * PLB + (cls * 16 + c) * 16, x);
-    }
-  }
-  static __device__ __forceinline__ void load_stage(const Args& g, const TileCoord& t, int,
-                                                    uint8_t* st, int glane, int gsize, Prod&) {
-    float unused[4];
-    const int z0 = t.mt * 128;
-    stream_pixels<GridZ, 8, TROWS, PL, 7, false, false>(st, st + IMG, g.dy2, z0, z0 + TROWS, g.num_samples,
-                                                         glane, gsize, unused);
-  }
-  static __device__ __forceinline__ void issue(const Args&, const TileCoord&, int, uint32_t st,
-                                               uint32_t res, uint32_t d) {
-    constexpr uint32_t idesc128 = tc::make_idesc(128), idesc64 = tc::make_idesc(64);
-#pragma unroll
-    const uint64_t da0 = tc::make_sdesc(st, PL), db0 = tc::make_sdesc(res, PLB);   // one derivation per stage
-#pragma unroll
-    for (int tap = 0; tap < 4; ++tap) {
-      // output (yy,xx) of every class reads Z row P + 12 - 11*dkh - dkw
-      const uint32_t aoff = (12 - 11 * (tap >> 1) - (tap & 1)) * 16;
-#pragma unroll
-      for (int k16 = 0; k16 < 2; ++k16) {
-        const uint64_t da_hi = tc::sdesc_advance(da0, aoff + 2 * k16 * PL);
-        const uint64_t da_lo = tc::sdesc_advance(da0, aoff + IMG + 2 * k16 * PL);
-        const uint64_t db = tc::sdesc_advance(db0, (tap * 4 + 2 * k16) * PLB);
-        tc::umma_f16(d, da_hi, db, idesc128, (tap | k16) != 0 ? 1u : 0u);  // z_hi . [wT_hi | wT_lo]
-        tc::umma_f16(d, da_lo, db, idesc64, 1u);                            // z_lo . wT_hi
-      }
-    }
-  }
-  // epilogue: lane = row (yy, xx) of the 11-wide grid = the 2x2 block of dy1 pixels (2yy+dy, 2xx+dx),
-  // accumulator columns cls*16 + c with cls = dy*2 + dx.  Per pixel and channel half: relu mask
-  // (sign of a1's hi part, prefetched before the accumulator wait), bias-gradient sums, bf16 split,
-  // one hi and one lo vector into dy1s.  Rows yy = 10 / xx = 10 write the zero rows y = 20 / x = 20.
-  // Lanes of a warp write 16-B vectors 32 B apart, the dx = 0/1 stores interleave: 8 lines each.
-  struct EpiPre { uint4 m[8]; };
-  struct EpiState { float b[16]; };
-  static __device__ __forceinline__ void epi_begin(EpiState& s) {
-#pragma unroll
-    for (int c = 0; c < 16; ++c) s.b[c] = 0.f;
-  }
-  static __device__ __forceinline__ void epi_prefetch(const Args& g, const TileCoord& t, int row, EpiPre& pre) {
-    const int pr = t.mt * 128 + row, n = pr / GROWS;
-    const int q = pr - n * GROWS, yy = q / GW, xx = q - yy * GW;
-    const bool ok = n < g.num_samples && yy < 10 && xx < 10;
-    const uint8_t* p = g.a1s + (int64_t)n * kA1sSample + (yy * 10 + xx) * 16;     // plane = cls*2 + chalf (fp16 a1)
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-      pre.m[i] = ok ? __ldg(reinterpret_cast<const uint4*>(p + i * kA1sPlane)) : make_uint4(0u, 0u, 0u, 0u);
-  }
-  static __device__ __forceinline__ void custom_epilogue(const Args& g, const TileCoord& t, const uint8_t*,
-                                                         uint32_t taddr, int row, EpiPre& pre, EpiState& st) {
-    const int pr = t.mt * 128 + row, n = pr / GROWS;
-    const int q = pr - n * GROWS, yy = q / GW, xx = q - yy * GW;
-    const bool live = n < g.num_samples;
-    const int64_t R = (int64_t)g.num_samples * kDy1sRows;
-#pragma unroll
-    for (int cls = 0; cls < 4; ++cls) {
-      const int y = 2 * yy + (cls >> 1), x = 2 * xx + (cls & 1);
-#pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        float v[8];
-        tc::tmem_ld8_sum(taddr + cls * 16 + half * 8, taddr + 64 + cls * 16 + half * 8, v);
-        if (!live || y > 20 || x > 20) continue;
-        uint4 hv = make_uint4(0u, 0u, 0u, 0u);
-        if (y < 20 && x < 20) {
-          const uint4 m = pre.m[cls * 2 + half];
-          const uint32_t w[4] = {m.x, m.y, m.z, m.w};
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            if ((int16_t)(w[i] & 0xFFFFu) <= 0) v[2 * i] = 0.f;        // fp16 > 0 <=> its bits as int16 > 0
-            if ((int32_t)w[i] < 0x10000) v[2 * i + 1] = 0.f;
-          }
-#pragma unroll
-          for (int e = 0; e < 8; ++e) st.b[half * 8 + e] += v[e];
-          hv = make_uint4(tc::pack_h2(v[0], v[1]), tc::pack_h2(v[2], v[3]), tc::pack_h2(v[4], v[5]),
-                          tc::pack_h2(v[6], v[7]));
-        }
-        *reinterpret_cast<uint4*>(g.dy1s + ((int64_t)half * R + (int64_t)n * kDy1sRows + y * 21 + x) * 16) = hv;
-      }
-    }
-  }
-  static __device__ __forceinline__ void epi_end(const Args& g, EpiState& st, int warp, int lane) {
-#pragma unroll
-    for (int c = 0; c < 16; ++c) {
-      const float s = warp_sum(st.b[c]);
-      if (lane == 0) g.bias_partials[((size_t)blockIdx.x * 8 + warp) * 16 + c] = s;
-    }
-  }
-};
 
-// =================================== weight gradients =========================================
 // work item `item` (= its partial slice `ks`) covers the row range number `range`
 __device__ __forceinline__ TileCoord range_tile(int item, int64_t rows, int k_chunk, int range) {
   TileCoord t;
@@ -666,96 +539,219 @@ __device__ __forceinline__ void bias_partial_store(float* dst_row, float (&acc)[
     *reinterpret_cast<float4*>(dst_row + lane * 4) = make_float4(acc[0], acc[1], acc[2], acc[3]);
 }
 
-struct Conv2WgradArgs {
-  const uint8_t* a1s;    // fp16 blocked conv1 output
-  const float* dy2;
-  float* partials;       // [items][8192]
-  float* bias_partials;  // [items * PROD_WARPS][32]  column sums of dy2 (= db2), per producer warp
-  int64_t rows;          // 100 * num_samples
-  int num_samples, k_chunk, items;
-  int reverse;           // item i takes row range items-1-i (see serpentine())
+struct Conv2BwdArgs {
+  const uint8_t* w_img;   // prepared: transposed fp16 [hi | lo] image of l2_w
+  const uint8_t* a1s;     // fp16 blocked conv1 output: weight-gradient operand and relu mask
+  const float* dy2;       // [N, 81, 32]
+  uint8_t* dy1s;          // conv1 output gradient (see dy1s above)
+  float* partials;        // [grid][8192]: dW2 of each CTA's tiles
+  float* bias2_partials;  // [grid * PROD_WARPS][32]: column sums of dy2 (= db2), per producer warp
+  float* bias1_partials;  // [grid * 8 epilogue warps][16]: column sums of dy1 (= db1)
+  int64_t rows;           // 100 * num_samples
+  int num_samples;
+  int reverse;            // walk the row tiles from the last to the first (see serpentine())
 };
-struct Conv2Wgrad : tc::PolicyBase {
-  using Args = Conv2WgradArgs;
-  struct Prod { float acc[4]; };    // running column sums of dy2 (bias gradient)
-  // dW2[(a,b) tap][ch][co] = sum_P X2[P + a*10 + b][ch] * dy2[P][co] over the rows P of the X2 grid.
-  // Both operands are fp16: X2 is bulk-copied from a1s as it is (one fp16 per value), dy2 is
-  // converted by the producers into an fp16 hi + lo pair concatenated along N (the gradient keeps
-  // its two terms: a single fp16 term left l1_b / l2_w at 1e-3 against the oracle).  Tap b is
-  // folded into M: a second bulk copy of the X2 image shifted by one row fills planes 8..15, so
-  // rows b*64 + ch of the accumulator are tap b; tap a is a row offset of the A descriptor and its
-  // own block of 64 accumulator columns.  One N = 64 MMA per tap a and 16 rows: 16 per stage
-  // (round 1: 32, with X2 as a hi/lo pair stacked along M).
+// Weight and input gradient of conv2 in one pass over 128-row tiles of the 10-wide X2 grid.  A
+// stage holds the tile's X2 rows [p0, p0 + 140) (+ the copy shifted by one row), bulk-copied from
+// a1s, and dy2 rows [p0 - 11, p0 + 128) converted ONCE into an fp16 hi + lo pair.  Both MMAs read
+// that one dy image:
+//   input gradient (transposed conv): output block (yy, xx) of parity class (dy, dx), tap (th, tw)
+//     reads dy2 pixel (yy - th, xx - tw) = grid row P - 10*th - tw, with kh = dy + 2*th,
+//     kw = dx + 2*tw.  Every out-of-range pixel lands on a zero row of the grid (px = 9 / py = 9 of
+//     this or the previous sample, or before sample 0), so no padded grid is needed.  dy is the
+//     K-major A operand (M = rows, K = co) at a row offset of 11 - 10*th - tw; the resident W2^T
+//     image is B with rows part*64 + cls*16 + c (N = 128: the 4 parity classes and the lo part
+//     share the A tile of a tap): z_hi . [wT_hi | wT_lo] + z_lo . wT_hi into the tile's accumulator.
+//   weight gradient: dW2[(a,b) tap][ch][co] = sum_P X2[P + a*10 + b][ch] * dy2[P][co].  Tap b is
+//     folded into M (planes 8..15 = the shifted copy), tap a is a row offset of the A descriptor;
+//     dy rows [p0, p0 + 128) are the MN-major B operand [dy_hi | dy_lo] (N = 64), accumulated over
+//     all the CTA's tiles in a CTA-lifetime accumulator that the epilogue warps drain once.
+// The relu mask the input gradient's epilogue needs is a1s row P of the 8 planes = rows this CTA's
+// bulk copies have just brought into L2.
+struct Conv2Bwd : tc::PolicyBase {
+  using Args = Conv2BwdArgs;
+  struct Prod { float acc[4]; };    // running column sums of dy2 over the CTA's tiles (bias gradient)
   static constexpr int GW = 10, GROWS = 100, TROWS = 140;
-  static constexpr int PLA = (TROWS + 1) * 16, A_IMG = 8 * PLA;    // one copy: 8 channel groups
-  static constexpr int PLB = 130 * 16, B_IMG = 4 * PLB;            // dy2: 4 co groups per part
-  static constexpr int PROD_WARPS = 18, STAGES = 3, STAGE_BYTES = 2 * A_IMG + 2 * B_IMG, RES_BYTES = 0;
-  // accumulator columns: a*64 + part*32 + co
-  static constexpr int ACC_COLS = 128, OUT_COLS = 64, LO_DELTA = 32, SEG = 32;
-  static __device__ __forceinline__ int acc_col(int c) { return (c >> 5) * 64 + (c & 31); }
-  static __device__ __forceinline__ int num_items(const Args& g) { return g.items; }
+  static constexpr int HALO = 11, DROWS = kTileM + HALO;           // dy rows [p0 - 11, p0 + 128)
+  static constexpr int PLA = (TROWS + 1) * 16, A_IMG = 8 * PLA;    // X2: one copy = 8 channel groups
+  // dy: 4 co groups per part; 142 rows: the producers' 8-byte stores of the 4 chunks of a row fall
+  // into distinct banks (PLD % 128 = 96)
+  static constexpr int PLD = 142 * 16, D_IMG = 4 * PLD;
+  // 4 producer warps per stage stream the 159-pixel dy window in one round of 10 float4 per lane;
+  // two epilogue sets: the mask loads of one tile overlap the read-out of the previous one.
+  // 21 warps -> 96 registers per thread
+  static constexpr int EPI_SETS = 2, PROD_WARPS = 12, STAGES = 3, STAGE_BYTES = 2 * A_IMG + 2 * D_IMG;
+  static constexpr int PLB = 129 * 16, RES_BYTES = 16 * PLB;       // W2^T: 16 k-chunk planes (tap*4 + co8)
+  // tile accumulator: cls*16 + c (hi products), + 64 (lo); CTA accumulator: a*64 + part*32 + co
+  static constexpr int ACC_COLS = 128, OUT_COLS = 64, LO_DELTA = 64, SEG = 32, PERSIST_COLS = 128;
+  static constexpr bool CUSTOM_EPI = true, PROD_PER_CTA = true;
+  static __device__ __forceinline__ int acc_col(int c) { return c; }
+  static __device__ __forceinline__ int num_items(const Args& g) { return (int)((g.rows + 127) / 128); }
   static __device__ __forceinline__ TileCoord coord(const Args& g, int item) {
-    return range_tile(item, g.rows, g.k_chunk, g.reverse ? g.items - 1 - item : item);
+    TileCoord t = row_tile(g.reverse ? num_items(g) - 1 - item : item);
+    t.ks = item;                      // == blockIdx.x: the CTA's first tile (starts dW2 at zero)
+    return t;
   }
-  static __device__ __forceinline__ int num_stages(const Args&, const TileCoord& t) {
-    return (t.k_end - t.k_begin + 127) / 128;
+  static __device__ __forceinline__ int num_stages(const Args&, const TileCoord&) { return 1; }
+  static __device__ __forceinline__ void load_resident(const Args& g, uint8_t* res, int ptid, int nthr) {
+    copy_image<RES_BYTES>(res, g.w_img, ptid, nthr);
   }
-  static __device__ __forceinline__ void load_resident(const Args&, uint8_t*, int, int) {}
+  static __device__ __forceinline__ void build_image(const float* params, uint8_t* res, int ptid, int nthr) {
+    const float* w2 = params + 4112;
+    for (int ch = ptid; ch < 4 * 16 * 16; ch += nthr) {
+      const int c = ch & 15, kc = (ch >> 4) & 15, cls = ch >> 8;   // kc = tap*4 + co8
+      const int tap = kc >> 2, co8 = kc & 3;
+      const int kh = (cls >> 1) + 2 * (tap >> 1), kw = (cls & 1) + 2 * (tap & 1);
+      float x[8];
+      load8(w2 + ((kh * 4 + kw) * 16 + c) * 32 + co8 * 8, x);
+      tc::store_chunk_split_h(res, res + 64 * 16, kc * PLB + (cls * 16 + c) * 16, x);
+    }
+  }
   static __device__ __forceinline__ void prod_begin(Prod& ps) {
     ps.acc[0] = ps.acc[1] = ps.acc[2] = ps.acc[3] = 0.f;
   }
-  static __device__ __forceinline__ void load_stage(const Args& g, const TileCoord& t, int s,
+  static __device__ __forceinline__ void load_stage(const Args& g, const TileCoord& t, int,
                                                     uint8_t* st, int glane, int gsize, Prod& ps) {
-    const int p0 = t.k_begin + s * 128;
-    // A: X2 rows p0 .. p0+139 (and the copy shifted by one row) arrive by cp.async.bulk
-    // (bulk_stage); only the rows beyond the last sample need zeros here
+    const int p0 = t.mt * 128;
+    // X2 rows arrive by cp.async.bulk (bulk_stage); only the rows beyond the last sample need zeros
     a1s_zero_tail<TROWS, PLA, 16>(st, p0, g.num_samples, glane, gsize);
-    // B: dy2 on the 10-wide grid, zero at y'=9 / x'=9 and outside [k_begin, k_end)
-    uint8_t* b_hi = st + 2 * A_IMG;
-    stream_pixels<GridDy2, 8, 128, PLB, 7, true, true>(b_hi, b_hi + B_IMG, g.dy2, p0, t.k_end, g.num_samples,
-                                                       glane, gsize, ps.acc);
+    // dy2 on the 10-wide grid; the bias sums skip the 11 halo rows (the previous tile's)
+    uint8_t* d_hi = st + 2 * A_IMG;
+    stream_pixels<GridDy2, 8, DROWS, PLD, 10, HALO>(d_hi, d_hi + D_IMG, g.dy2, p0 - HALO, g.num_samples,
+                                                   glane, gsize, ps.acc);
   }
-  // 8 lanes of the stage's 192 (every 24th) own one plane each
-  static __device__ __forceinline__ bool bulk_stage(const Args& g, const TileCoord& t, int s, uint8_t* st,
+  // 8 lanes of the stage's 128 (every 16th) own one a1s plane each
+  static __device__ __forceinline__ bool bulk_stage(const Args& g, const TileCoord& t, int, uint8_t* st,
                                                     int glane, int, uint64_t* full) {
-    if (glane % 24 != 0) return false;
-    const int p0 = t.k_begin + s * 128, kc = glane / 24;             // 0..7
+    if (glane % 16 != 0) return false;
+    const int p0 = t.mt * 128, kc = glane / 16;                      // 0..7
     mbar_expect_tx(full, a1s_bulk_bytes<TROWS, true>(p0, g.num_samples));
     a1s_bulk_issue<TROWS, PLA, true>(st, g.a1s, p0, g.num_samples, kc, full);
     return true;
   }
   static __device__ __forceinline__ void prod_end(const Args& g, const TileCoord& t, Prod& ps, int pw,
                                                   int lane) {
-    bias_partial_store<8>(g.bias_partials + ((size_t)t.ks * PROD_WARPS + pw) * 32, ps.acc, lane);
+    bias_partial_store<8>(g.bias2_partials + ((size_t)t.ks * PROD_WARPS + pw) * 32, ps.acc, lane);
   }
-  static __device__ __forceinline__ void issue(const Args&, const TileCoord&, int s, uint32_t st,
-                                               uint32_t, uint32_t d) {
-    constexpr uint32_t idesc = tc::make_idesc_h(64, true, true);     // [x ; x shifted] . [dy_hi | dy_lo]
-    // one descriptor derivation per stage
-    const uint64_t da0 = tc::make_sdesc(st, 128, PLA), db0 = tc::make_sdesc(st + 2 * A_IMG, 128, PLB);
+  static __device__ __forceinline__ void issue(const Args&, const TileCoord& t, int, uint32_t st,
+                                               uint32_t res, uint32_t d, uint32_t dw) {
+    const uint32_t dy = st + 2 * A_IMG;
+    {                                                                // input gradient
+      constexpr uint32_t idesc128 = tc::make_idesc_h(128), idesc64 = tc::make_idesc_h(64);
+      const uint64_t da0 = tc::make_sdesc(dy, PLD), db0 = tc::make_sdesc(res, PLB);
 #pragma unroll
-    for (int a = 0; a < 2; ++a) {
+      for (int tap = 0; tap < 4; ++tap) {
+        const uint32_t aoff = (HALO - GW * (tap >> 1) - (tap & 1)) * 16;
 #pragma unroll
-      for (int k16 = 0; k16 < 8; ++k16) {
-        const uint64_t da = tc::sdesc_advance(da0, (a * GW + k16 * 16) * 16);
-        const uint64_t db = tc::sdesc_advance(db0, k16 * 256);
-        tc::umma_f16(d + a * 64, da, db, idesc, (s | k16) != 0 ? 1u : 0u);
+        for (int k16 = 0; k16 < 2; ++k16) {
+          const uint64_t da_hi = tc::sdesc_advance(da0, aoff + 2 * k16 * PLD);
+          const uint64_t da_lo = tc::sdesc_advance(da0, aoff + D_IMG + 2 * k16 * PLD);
+          const uint64_t db = tc::sdesc_advance(db0, (tap * 4 + 2 * k16) * PLB);
+          tc::umma_f16(d, da_hi, db, idesc128, (tap | k16) != 0 ? 1u : 0u);  // z_hi . [wT_hi | wT_lo]
+          tc::umma_f16(d, da_lo, db, idesc64, 1u);                            // z_lo . wT_hi
+        }
+      }
+    }
+    {                                                                // weight gradient
+      constexpr uint32_t idesc = tc::make_idesc_h(64, true, true);   // [x ; x shifted] . [dy_hi | dy_lo]
+      const uint64_t da0 = tc::make_sdesc(st, 128, PLA), db0 = tc::make_sdesc(dy + HALO * 16, 128, PLD);
+      const bool first = t.ks == (int)blockIdx.x;
+#pragma unroll
+      for (int a = 0; a < 2; ++a) {
+#pragma unroll
+        for (int k16 = 0; k16 < 8; ++k16) {
+          const uint64_t da = tc::sdesc_advance(da0, (a * GW + k16 * 16) * 16);
+          const uint64_t db = tc::sdesc_advance(db0, k16 * 256);
+          tc::umma_f16(dw + a * 64, da, db, idesc, (first && k16 == 0) ? 0u : 1u);
+        }
       }
     }
   }
-  // row = b*64 + ch, ch = (i*2+j)*16 + cin ; segment a = 32 co of tap (kh = 2a+i, kw = 2b+j)
-  static __device__ __forceinline__ float* row_ptr(const Args& g, const TileCoord& t, int row) {
-    const int b = row >> 6, ch = row & 63, ij = ch >> 4, cin = ch & 15;
-    return g.partials + (size_t)t.ks * 8192 + (((ij >> 1) * 4 + 2 * b + (ij & 1)) * 16 + cin) * 32;
+  // input-gradient epilogue: lane = row (yy, xx) of the 10-wide grid = the 2x2 block of dy1 pixels
+  // (2yy+dy, 2xx+dx), accumulator columns cls*16 + c with cls = dy*2 + dx.  Per pixel and channel
+  // half: relu mask (sign of a1, prefetched before the accumulator wait), bias-gradient sums, one
+  // fp16 vector into dy1s.  The lanes of the last block row / column (yy = 9 / xx = 9) also write
+  // the zero rows y = 20 / x = 20, so every byte of dy1s is written on every call.
+  struct EpiPre { uint4 m[8]; };
+  struct EpiState { float b[16]; };
+  static __device__ __forceinline__ void epi_begin(EpiState& s) {
+#pragma unroll
+    for (int c = 0; c < 16; ++c) s.b[c] = 0.f;
   }
-  static __device__ __forceinline__ int64_t seg_offset(const Args&, const TileCoord&, int a) {
-    return a * 8 * 16 * 32;
+  static __device__ __forceinline__ void epi_prefetch(const Args& g, const TileCoord& t, int row, EpiPre& pre) {
+    const int pr = t.mt * 128 + row, n = pr / GROWS, q = pr - n * GROWS;
+    const bool ok = n < g.num_samples;
+    const uint8_t* p = g.a1s + (int64_t)n * kA1sSample + q * 16;     // plane = cls*2 + chalf (fp16 a1)
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+      pre.m[i] = ok ? __ldg(reinterpret_cast<const uint4*>(p + i * kA1sPlane)) : make_uint4(0u, 0u, 0u, 0u);
+  }
+  static __device__ __forceinline__ void custom_epilogue(const Args& g, const TileCoord& t, const uint8_t*,
+                                                         uint32_t taddr, int row, EpiPre& pre, EpiState& st) {
+    const int pr = t.mt * 128 + row, n = pr / GROWS;
+    const int q = pr - n * GROWS, yy = q / GW, xx = q - yy * GW;
+    const bool live = n < g.num_samples;
+    const int64_t R = (int64_t)g.num_samples * kDy1sRows;
+    uint8_t* d0 = g.dy1s + (int64_t)n * kDy1sRows * 16;
+#pragma unroll
+    for (int cls = 0; cls < 4; ++cls) {
+      const int y = 2 * yy + (cls >> 1), x = 2 * xx + (cls & 1);
+#pragma unroll
+      for (int half = 0; half < 2; ++half) {
+        float v[8];
+        tc::tmem_ld8_sum(taddr + cls * 16 + half * 8, taddr + 64 + cls * 16 + half * 8, v);
+        if (!live) continue;
+        const uint4 m = pre.m[cls * 2 + half];
+        const uint32_t w[4] = {m.x, m.y, m.z, m.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          if ((int16_t)(w[i] & 0xFFFFu) <= 0) v[2 * i] = 0.f;        // fp16 > 0 <=> its bits as int16 > 0
+          if ((int32_t)w[i] < 0x10000) v[2 * i + 1] = 0.f;
+        }
+#pragma unroll
+        for (int e = 0; e < 8; ++e) st.b[half * 8 + e] += v[e];
+        *reinterpret_cast<uint4*>(d0 + (half * R + y * 21 + x) * 16) =
+            make_uint4(tc::pack_h2(v[0], v[1]), tc::pack_h2(v[2], v[3]), tc::pack_h2(v[4], v[5]),
+                       tc::pack_h2(v[6], v[7]));
+      }
+    }
+    if (live && (yy == 9 || xx == 9)) {
+      const uint4 z = make_uint4(0u, 0u, 0u, 0u);
+#pragma unroll
+      for (int half = 0; half < 2; ++half) {
+        uint4* dh = reinterpret_cast<uint4*>(d0 + half * R * 16);
+        if (yy == 9) { dh[20 * 21 + 2 * xx] = z; dh[20 * 21 + 2 * xx + 1] = z; }
+        if (xx == 9) { dh[(2 * yy) * 21 + 20] = z; dh[(2 * yy + 1) * 21 + 20] = z; }
+        if (yy == 9 && xx == 9) dh[20 * 21 + 20] = z;
+      }
+    }
+  }
+  static __device__ __forceinline__ void epi_end(const Args& g, EpiState& st, int warp, int lane) {
+#pragma unroll
+    for (int c = 0; c < 16; ++c) {
+      const float s = warp_sum(st.b[c]);
+      if (lane == 0) g.bias1_partials[((size_t)blockIdx.x * 8 + warp) * 16 + c] = s;
+    }
+  }
+  // weight gradient, once per CTA: epilogue set a drains tap a.  Accumulator row = b*64 + ch with
+  // ch = (i*2+j)*16 + cin; tap (kh = 2a+i, kw = 2b+j); columns a*64 + co (hi) and + 32 (lo)
+  static __device__ __forceinline__ void persist_epilogue(const Args& g, uint32_t taddr, int row, int a) {
+    const int b = row >> 6, ch = row & 63, ij = ch >> 4, cin = ch & 15;
+    float* dst = g.partials + (size_t)blockIdx.x * 8192 + (size_t)a * 8 * 16 * 32 +
+                 (((ij >> 1) * 4 + 2 * b + (ij & 1)) * 16 + cin) * 32;
+#pragma unroll
+    for (int c8 = 0; c8 < 4; ++c8) {
+      float v[8];
+      tc::tmem_ld8_sum(taddr + a * 64 + c8 * 8, taddr + a * 64 + 32 + c8 * 8, v);
+      reinterpret_cast<float4*>(dst + c8 * 8)[0] = make_float4(v[0], v[1], v[2], v[3]);
+      reinterpret_cast<float4*>(dst + c8 * 8)[1] = make_float4(v[4], v[5], v[6], v[7]);
+    }
   }
 };
 
 struct Conv1WgradArgs {
   RingGeo geo;
-  const uint8_t* dy1s;   // fp16 on the X grid, written by conv2 dgrad (see dy1s above)
+  const uint8_t* dy1s;   // fp16 on the X grid, written by conv2 backward (see dy1s above)
   float* partials;       // [items][4096]
   int64_t rows;          // 441 * num_samples
   int num_samples, k_chunk, items;
@@ -852,7 +848,7 @@ struct Conv1Wgrad : tc::PolicyBase {
   }
 };
 
-// arl_prepare_weights: CTA 0 / 1 / 2 builds the resident image of conv1 fwd / conv2 fwd / conv2 dgrad
+// arl_prepare_weights: CTA 0 / 1 / 2 builds the resident image of conv1 fwd / conv2 fwd / conv2 bwd
 // in shared memory (the same code the kernels used to run in their prologues) and writes it out
 __global__ void __launch_bounds__(256) build_images_kernel(const float* __restrict__ params, uint8_t* prepared) {
   extern __shared__ __align__(128) uint8_t img[];
@@ -866,19 +862,21 @@ __global__ void __launch_bounds__(256) build_images_kernel(const float* __restri
     Conv2Fwd::build_image(params, img, tid, 256);
     bytes = Conv2Fwd::RES_BYTES; out += kPrepW2F;
   } else {
-    Conv2Dgrad::build_image(params, img, tid, 256);
-    bytes = Conv2Dgrad::RES_BYTES; out += kPrepW2D;
+    Conv2Bwd::build_image(params, img, tid, 256);
+    bytes = Conv2Bwd::RES_BYTES; out += kPrepW2D;
   }
   __syncthreads();
   for (int i = tid; i < bytes / 16; i += 256) reinterpret_cast<uint4*>(out)[i] = reinterpret_cast<const uint4*>(img)[i];
 }
 static_assert(Conv1Fwd::RES_BYTES <= kPrepW1Bytes && Conv2Fwd::RES_BYTES <= kPrepW2FBytes &&
-                  Conv2Dgrad::RES_BYTES <= kPrepW2DBytes, "prepared-weight layout");
+                  Conv2Bwd::RES_BYTES <= kPrepW2DBytes, "prepared-weight layout");
 
 // Serpentine sweep: consecutive kernels of a chain walk the samples in OPPOSITE directions, so a
 // kernel starts with the rows its predecessor touched last -- the ones still in the 126 MB L2 --
 // instead of the ones evicted longest ago.  forward: conv1 up, conv2 DOWN; backward: fc dgrad up,
-// conv2 wgrad DOWN, conv2 dgrad up, conv1 wgrad DOWN.  ARL_SERPENTINE=0 turns it off (A/B runs).
+// conv2 backward DOWN, conv1 wgrad DOWN.  (conv1 wgrad gives each CTA one contiguous row range, so
+// its direction hardly changes which rows are read first: up measured the same, 244 us per cycle
+// at 4096 envs x t_max 5 on one B200.)  ARL_SERPENTINE=0 turns it off (A/B runs).
 bool serpentine() {
   static const bool on = [] { const char* e = getenv("ARL_SERPENTINE"); return !(e && e[0] == '0'); }();
   return on;
@@ -982,28 +980,23 @@ extern "C" int arl_conv2_backward(const float* prepared, const float* a1, const 
     ARL_CUDA(cudaMemsetAsync(grads + 4096, 0, (16 + 8192 + 32) * sizeof(float), st));   // l1_b | l2_w | l2_b
     return ARL_OK;
   }
-  Conv2WgradArgs w;
-  w.a1s = reinterpret_cast<const uint8_t*>(a1);
-  w.dy2 = d_a2;
-  w.partials = (float*)workspace;
-  w.rows = num_samples * 100;
-  w.num_samples = (int)num_samples;
-  w.items = split_rows(w.rows, num_sms(), &w.k_chunk);
-  w.reverse = serpentine() ? 1 : 0;
-  w.bias_partials = (float*)workspace + (size_t)w.items * 8192;
-  int rc = tc::launch<Conv2Wgrad>(w, w.items, st);
+  Conv2BwdArgs g;
+  g.w_img = reinterpret_cast<const uint8_t*>(prepared) + kPrepW2D;
+  g.a1s = reinterpret_cast<const uint8_t*>(a1);
+  g.dy2 = d_a2;
+  g.dy1s = reinterpret_cast<uint8_t*>(d_a1);
+  g.rows = num_samples * 100;
+  g.num_samples = (int)num_samples;
+  g.reverse = serpentine() ? 1 : 0;
+  const int items = (int)((g.rows + 127) / 128), grid = items < num_sms() ? items : num_sms();
+  g.partials = (float*)workspace;
+  g.bias2_partials = g.partials + (size_t)grid * 8192;
+  g.bias1_partials = g.bias2_partials + (size_t)grid * Conv2Bwd::PROD_WARPS * 32;
+  int rc = tc::launch<Conv2Bwd>(g, items, st);
   if (rc) return rc;
-  rc = reduce_partials_scaled(w.partials, g2, w.items, 8192, grad_unscale, st);
+  rc = reduce_partials_scaled(g.partials, g2, grid, 8192, grad_unscale, st);                     // l2_w
   if (rc) return rc;
-  // l2_b = column sums of d_a2, accumulated by the wgrad producers while they stream d_a2
-  rc = reduce_partials_scaled(w.bias_partials, g2 + 8192, w.items * Conv2Wgrad::PROD_WARPS, 32, grad_unscale, st);
+  rc = reduce_partials_scaled(g.bias2_partials, g2 + 8192, grid * Conv2Bwd::PROD_WARPS, 32, grad_unscale, st);   // l2_b
   if (rc) return rc;
-  // dgrad; its epilogue also sums the columns of d_a1 = the conv1 bias gradient l1_b
-  float* db1 = (float*)workspace + (size_t)w.items * (8192 + Conv2Wgrad::PROD_WARPS * 32);
-  Conv2DgradArgs d{reinterpret_cast<const uint8_t*>(prepared) + kPrepW2D, reinterpret_cast<const uint8_t*>(a1),
-                   d_a2, reinterpret_cast<uint8_t*>(d_a1), db1, num_samples * 121, (int)num_samples};
-  const int items = (int)((d.rows + 127) / 128);
-  rc = tc::launch<Conv2Dgrad>(d, items, st);
-  if (rc) return rc;
-  return reduce_partials_scaled(db1, grads + 4096, (items < num_sms() ? items : num_sms()) * 8, 16, grad_unscale, st);
+  return reduce_partials_scaled(g.bias1_partials, grads + 4096, grid * 8, 16, grad_unscale, st);   // l1_b
 }

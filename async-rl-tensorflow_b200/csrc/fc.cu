@@ -363,7 +363,7 @@ extern "C" int arl_fc_backward(const float* prepared, const float* a2, int64_t a
                                 ARL_FC, ARL_FC, (M + 7) / 8);
   const tc::SplitMat ws = mat(prepared, ARL_A2_ELEMS, ARL_A2_ELEMS, ARL_FC / 8);
   // wgrad first (dW [2592,256] = a2^T . d_h, 7 split-K slices x 21 row tiles = 147 items), dgrad
-  // LAST: the next kernel of the chain (conv2 wgrad) starts with the d_a2 rows dgrad wrote last
+  // LAST: the next kernel of the chain (conv2 backward) starts with the d_a2 rows dgrad wrote last
   float* part = (float*)workspace;
   tc::BulkGemmArgs g = {};
   g.A = a2s; g.B = dhsT; g.mask = mat(nullptr, 0, 1, 0);

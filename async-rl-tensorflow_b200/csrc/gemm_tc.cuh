@@ -267,15 +267,6 @@ __device__ __forceinline__ void store_chunk_split(uint8_t* hi_img, uint8_t* lo_i
   *reinterpret_cast<uint4*>(hi_img + off) = h;
   *reinterpret_cast<uint4*>(lo_img + off) = l;
 }
-// 4 consecutive k of one row: 8 B of hi and 8 B of lo
-__device__ __forceinline__ void store_half_split(uint8_t* hi_img, uint8_t* lo_img, int off,
-                                                 const float4& x) {
-  uint2 h, l;
-  split2(x.x, x.y, h.x, l.x);
-  split2(x.z, x.w, h.y, l.y);
-  *reinterpret_cast<uint2*>(hi_img + off) = h;
-  *reinterpret_cast<uint2*>(lo_img + off) = l;
-}
 // ---- fp16 storage (round 2: tensors that are only ever tensor-core operands are kept as ONE fp16
 // value instead of a bf16 hi + lo pair: 2^-12 relative per element, measured 2.5e-4 / 4.4e-4 on
 // logits / gradients against the float64 oracle -- tests/precision_study.py; plain bf16 fails the
@@ -421,6 +412,16 @@ struct PolicyBase {
   static constexpr bool HAS_AUX = false;       // finish() needs an operand from HBM (bias, relu mask)
   static constexpr bool AUX_ROW_INVARIANT = true;   // ... that depends on the column only (bias)
   struct Prod {};
+  // PROD_PER_CTA: Prod lives across all the items of the CTA (prod_begin before the first,
+  // prod_end after the last, with a TileCoord whose ks = blockIdx.x) instead of one item
+  static constexpr bool PROD_PER_CTA = false;
+  // PERSIST_COLS > 0: a second accumulator of that many TMEM columns (after the NUM_ACC per-item
+  // ones) that lives across all the items of the CTA.  issue() gets its address as a 7th argument;
+  // the MMA warp commits it after the CTA's last stage, and the epilogue warps then read it out
+  // once: persist_epilogue(g, taddr (lane quadrant of the warp), row, epilogue set)
+  static constexpr int PERSIST_COLS = 0;
+  template <class Args>
+  static __device__ __forceinline__ void persist_epilogue(const Args&, uint32_t, int, int) {}
   template <class Pr>
   static __device__ __forceinline__ void prod_begin(Pr&) {}
   // PREFETCH: the producer requests the global data of its NEXT stage (into registers held in
@@ -482,7 +483,8 @@ struct Smem {
   static constexpr int EPI_OFF = BAR_OFF + 512;                 // up to 2*16 + 4 mbarriers + TMEM slot
   static constexpr int EPI_ROW = (P::SEG + 4) * 4;              // staged row, padded: conflict-free
   static constexpr int EPI_WARP = 32 * EPI_ROW + 32 * 8 + 32 * 8;   // staging + 32 row pointers + 32 row aux offsets
-  static constexpr int TOTAL = EPI_OFF + epi_warps<P>() * EPI_WARP;
+  // a custom epilogue writes its output itself and never touches the staging area
+  static constexpr int TOTAL = EPI_OFF + (P::CUSTOM_EPI ? 0 : epi_warps<P>() * EPI_WARP);
 };
 
 template <class P>
@@ -501,12 +503,14 @@ __global__ void __launch_bounds__(cta_threads<P>(), 1) tc_kernel(typename P::Arg
   constexpr int NUM_ACC = P::EPI_SETS > 2 ? P::EPI_SETS : 2;
   uint64_t* tfull = empty + STAGES;      // [NUM_ACC]
   uint64_t* tempty = tfull + NUM_ACC;    // [NUM_ACC]
-  uint32_t* tmem_base_slot = reinterpret_cast<uint32_t*>(tempty + NUM_ACC);
+  uint64_t* pfull = tempty + NUM_ACC;    // PERSIST_COLS > 0: the CTA-lifetime accumulator is final
+  uint32_t* tmem_base_slot = reinterpret_cast<uint32_t*>(pfull + 1);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  constexpr uint32_t kTmemCols = NUM_ACC * P::ACC_COLS <= 32 ? 32 : NUM_ACC * P::ACC_COLS <= 64 ? 64
-                               : NUM_ACC * P::ACC_COLS <= 128 ? 128 : NUM_ACC * P::ACC_COLS <= 256 ? 256 : 512;
-  static_assert(NUM_ACC * P::ACC_COLS <= 512 && P::ACC_COLS % 16 == 0, "TMEM budget");
+  constexpr int kAccCols = NUM_ACC * P::ACC_COLS + P::PERSIST_COLS;
+  constexpr uint32_t kTmemCols = kAccCols <= 32 ? 32 : kAccCols <= 64 ? 64 : kAccCols <= 128 ? 128
+                               : kAccCols <= 256 ? 256 : 512;
+  static_assert(kAccCols <= 512 && P::ACC_COLS % 16 == 0 && P::PERSIST_COLS % 16 == 0, "TMEM budget");
   static_assert(P::EPI_SETS == 1 || P::EPI_SETS == 2 || P::EPI_SETS == 4, "EPI_SETS");
 
   if (tid == 0) {
@@ -518,6 +522,7 @@ __global__ void __launch_bounds__(cta_threads<P>(), 1) tc_kernel(typename P::Arg
       mbar_init(&tfull[a], 1);
       mbar_init(&tempty[a], 128);
     }
+    if (P::PERSIST_COLS > 0) mbar_init(pfull, 1);
     fence_mbar_init();
   }
   if (warp == kMmaWarp) tmem_alloc(tmem_base_slot, kTmemCols);
@@ -544,11 +549,12 @@ __global__ void __launch_bounds__(cta_threads<P>(), 1) tc_kernel(typename P::Arg
     const int pg = pw / WPS, glane = (pw % WPS) * 32 + lane;
     uint8_t* st = smem + pg * P::STAGE_BYTES;
     int i = 0;                                         // running stage index over all items
+    typename P::Prod ps;
+    if (P::PROD_PER_CTA) P::prod_begin(ps);
     for (int item = blockIdx.x; item < items; item += gridDim.x) {
       const TileCoord tc = P::coord(g, item);
       const int ns = P::num_stages(g, tc);
-      typename P::Prod ps;
-      P::prod_begin(ps);
+      if (!P::PROD_PER_CTA) P::prod_begin(ps);
       bool first = true;
       for (int s = 0; s < ns; ++s, ++i) {
         if (i % STAGES != pg) continue;
@@ -560,7 +566,12 @@ __global__ void __launch_bounds__(cta_threads<P>(), 1) tc_kernel(typename P::Arg
         if (!P::bulk_stage(g, tc, s, st, glane, 32 * WPS, &full[pg])) mbar_arrive(&full[pg]);
         if (P::PREFETCH && s + STAGES < ns) P::prefetch_stage(g, tc, s + STAGES, glane, 32 * WPS, ps);
       }
-      P::prod_end(g, tc, ps, pw, lane);
+      if (!P::PROD_PER_CTA) P::prod_end(g, tc, ps, pw, lane);
+    }
+    if (P::PROD_PER_CTA) {
+      TileCoord cta{};
+      cta.ks = blockIdx.x;
+      P::prod_end(g, cta, ps, pw, lane);
     }
   } else if (warp == kMmaWarp) {
     // ===================== MMA issuer (one thread) =====================
@@ -579,12 +590,20 @@ __global__ void __launch_bounds__(cta_threads<P>(), 1) tc_kernel(typename P::Arg
           mbar_wait_sleep(&full[stage], (i / STAGES) & 1);
           tc_fence_after();
           if (elect_one()) {
-            P::issue(g, tc, s, smem_u32(smem + stage * P::STAGE_BYTES), res_addr, d_tmem);
+            if constexpr (P::PERSIST_COLS > 0)
+              P::issue(g, tc, s, smem_u32(smem + stage * P::STAGE_BYTES), res_addr, d_tmem,
+                       tmem_base + NUM_ACC * P::ACC_COLS);
+            else
+              P::issue(g, tc, s, smem_u32(smem + stage * P::STAGE_BYTES), res_addr, d_tmem);
             umma_commit(&empty[stage]);      // frees the smem stage when these MMAs retire
           }
           __syncwarp();
         }
         if (elect_one()) umma_commit(&tfull[acc]);       // accumulator ready for the epilogue
+        __syncwarp();
+      }
+      if (P::PERSIST_COLS > 0) {
+        if (elect_one()) umma_commit(pfull);             // after the CTA's last stage
         __syncwarp();
       }
     }
@@ -695,6 +714,12 @@ __global__ void __launch_bounds__(cta_threads<P>(), 1) tc_kernel(typename P::Arg
       }
       tc_fence_before();
       mbar_arrive(&tempty[acc]);
+    }
+    if constexpr (P::PERSIST_COLS > 0) {
+      mbar_wait_backoff<64>(pfull, 0);
+      tc_fence_after();
+      P::persist_epilogue(g, tmem_base + ((uint32_t)(quad * 32) << 16) + NUM_ACC * P::ACC_COLS,
+                          quad * 32 + lane, set);
     }
     P::epi_end(g, est, warp, lane);
   }

@@ -21,7 +21,8 @@ ENTRY_OF = [
     ("BulkGemm<128, 32, 0, 0, 2", "arl_fc_backward"),    # fc dgrad
     ("BulkGemm<128, 64, 1, 1, 0", "arl_fc_backward"),    # fc wgrad (earlier form)
     ("BulkGemm<256, 32, 1, 0, 0", "arl_fc_backward"),    # fc wgrad
-    ("Conv2Wgrad", "arl_conv2_backward"),
+    ("Conv2Bwd", "arl_conv2_backward"),
+    ("Conv2Wgrad", "arl_conv2_backward"),                # (earlier form: two kernels)
     ("Conv2Dgrad", "arl_conv2_backward"),
     ("Conv1Wgrad", "arl_conv1_backward"),
 ]
