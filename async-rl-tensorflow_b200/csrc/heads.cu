@@ -23,20 +23,60 @@ __device__ __forceinline__ void tc_split2(float a, float b, uint32_t& hi, uint32
 int reduce_partials(const float* partials, float* out, int num_partials, int n,
                     cudaStream_t stream);
 
+// Philox4x32-10: second output word of the same block (used by the epsilon-greedy draw)
+__device__ __forceinline__ void philox_two(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
+                                           uint32_t k0, uint32_t k1, uint32_t& x0, uint32_t& x1) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+    const uint32_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
+    c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
+    k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+  }
+  x0 = c0; x1 = c1;
+}
+
 // ------------------------------- heads forward --------------------------------------------
 // One warp per sample: lane l holds h[8l .. 8l+7] (the warp reads the 1-KB row as 32-byte pieces),
 // the weights sit in shared memory as wt[(j*8 + e)*32 + l] = W[k = 8l + e][j] (conflict-free),
 // every output is 8 FMAs per lane + a butterfly sum; lane j keeps logit j, the softmax runs
 // across the lanes.  (First version: 16 samples per CTA staged in shared memory, one thread per
 // (sample, output) walking 256 k serially: 10 us per 4096 samples, latency-bound.)
+//
+// The action draw after the heads is chosen by the last argument's type: SampleDraw (network.py:72,
+// the A3C policy sample) or EgreedyDraw (agent.py:141-151 on the logits, the n-step Q learner of
+// arl_forward_egreedy).  SampleDraw carries nothing and its branch is the only one compiled in, so the
+// A3C path pays nothing for the second kind.
+struct SampleDraw {
+  static constexpr bool kEgreedy = false;
+};
+struct EgreedyDraw {
+  static constexpr bool kEgreedy = true;
+  float ep;                                          // used when step_dev == nullptr
+  double ep_start, ep_end, ep_end_t, learn_start;    // used with step_dev (agent.py:142-144)
+};
+
+// agent.py:142-144  ep_end + max(0., (ep_start - ep_end) * (ep_end_t - max(0., step - learn_start))
+// / ep_end_t), in double, one correctly rounded operation at a time in Python's order (the _rn
+// intrinsics keep the compiler from contracting a multiply and an add), then rounded to float once:
+// the float the host computes as c_float(Agent.ep), bit for bit
+__device__ __forceinline__ float egreedy_epsilon(const EgreedyDraw& d, int64_t step) {
+  const double s = __dsub_rn((double)step, d.learn_start);
+  const double m = s > 0.0 ? s : 0.0;
+  const double f = __ddiv_rn(__dmul_rn(__dsub_rn(d.ep_start, d.ep_end), __dsub_rn(d.ep_end_t, m)), d.ep_end_t);
+  return __double2float_rn(__dadd_rn(d.ep_end, f > 0.0 ? f : 0.0));
+}
+
 constexpr int kHfThreads = 256;
+template <class Draw>
 __global__ void __launch_bounds__(kHfThreads)
 heads_fwd_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
                  const float* __restrict__ qw, const float* __restrict__ qb,
                  const float* __restrict__ h, float* __restrict__ logits,
                  float* __restrict__ probs, float* __restrict__ value, int64_t num_samples, int A,
                  int32_t* __restrict__ actions, uint64_t env_id_base, uint64_t step, uint64_t seed,
-                 const int64_t* __restrict__ step_dev, int wait_first) {
+                 const int64_t* __restrict__ step_dev, int wait_first, Draw draw) {
   extern __shared__ __align__(16) float sm[];   // [A+1][8][32]
   // wait_first: the kernel before this one in the stream may have written the parameters (a
   // stand-alone arl_heads_forward right after an update): nothing is read before the wait
@@ -55,6 +95,8 @@ heads_fwd_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
   // touched only after it has completed
   if (!wait_first) pdl_wait();
   if (actions != nullptr && step_dev != nullptr) step += (uint64_t)*step_dev;
+  float ep = 0.f;
+  if constexpr (Draw::kEgreedy) ep = step_dev != nullptr ? egreedy_epsilon(draw, (int64_t)step) : draw.ep;
   const int64_t stride = (int64_t)gridDim.x * (kHfThreads / 32);
   for (int64_t n = (int64_t)blockIdx.x * (kHfThreads / 32) + warp; n < num_samples; n += stride) {
     const float4* hp = reinterpret_cast<const float4*>(h + n * 256) + lane * 2;
@@ -82,7 +124,22 @@ heads_fwd_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
       probs[n * A + lane] = pj;
     }
     if (lane == 0) value[n] = zv + qb0;
-    if (actions != nullptr) {
+    if constexpr (Draw::kEgreedy) {
+      // the draw of egreedy_actions_kernel on the logits just written: Philox block (env, step_lo,
+      // step_hi, 1), word 0 -> u < ep, word 1 -> uniform action, else argmax (ties -> lowest index)
+      uint32_t x0, x1;
+      philox_two((uint32_t)(env_id_base + (uint64_t)n), (uint32_t)step, (uint32_t)(step >> 32), 1u,
+                 (uint32_t)seed, (uint32_t)(seed >> 32), x0, x1);
+      const float u = (float)(x0 >> 8) * 5.9604644775390625e-08f;     // 2^-24
+      int a = 0;
+      float best = __shfl_sync(0xffffffffu, z, 0);
+      for (int j = 1; j < A; ++j) {
+        const float q = __shfl_sync(0xffffffffu, z, j);
+        if (q > best) { best = q; a = j; }
+      }
+      if (u < ep) a = (int)(((uint64_t)x1 * (uint64_t)A) >> 32);
+      if (lane == 0) actions[n] = a;
+    } else if (actions != nullptr) {
       // network.py:72 in the same launch: the draw of sample_actions_kernel (Philox4x32-10 keyed by
       // the global env id and the step; inverse CDF over the float32 running sum in index order)
       const uint32_t x = philox_first((uint32_t)(env_id_base + (uint64_t)n), (uint32_t)step,
@@ -104,20 +161,6 @@ heads_fwd_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
 }
 
 // ------------------------------- action selection -----------------------------------------
-// second output word of the same block (used by the epsilon-greedy draw)
-__device__ __forceinline__ void philox_two(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
-                                           uint32_t k0, uint32_t k1, uint32_t& x0, uint32_t& x1) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-    const uint32_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
-    c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
-    k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-  }
-  x0 = c0; x1 = c1;
-}
-
 // step_dev (optional): the step counter lives in device memory (a captured CUDA graph cannot carry
 // a host value that changes on every launch); the Philox step is then *step_dev + step
 __global__ void sample_actions_kernel(const float* __restrict__ probs, int32_t* __restrict__ actions,
@@ -415,7 +458,9 @@ __global__ void observe_store_kernel(const float* __restrict__ reward, const uin
 }
 
 int heads_init() {
-  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<SampleDraw>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)((ARL_MAX_ACTIONS + 1) * 256 * sizeof(float))));
+  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<EgreedyDraw>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)((ARL_MAX_ACTIONS + 1) * 256 * sizeof(float))));
   return ARL_OK;
 }
@@ -437,10 +482,28 @@ int heads_forward_sample(const float* params, int action_size, const float* h, f
   // up to 4 CTAs per SM: one env step of 4096 samples is ONE round of warps (two rounds cost a second
   // exposed load latency)
   const int grid = (int)(ctas < 4LL * num_sms() ? ctas : 4LL * num_sms());
-  ARL_CUDA(launch_pdl(heads_fwd_kernel, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
+  ARL_CUDA(launch_pdl(heads_fwd_kernel<SampleDraw>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
                       params + L.off[T_PB], params + L.off[T_QW], params + L.off[T_QB], h, logits, probs, value,
                       num_samples, action_size, actions, (uint64_t)env_id_base, (uint64_t)step, seed, step_dev,
-                      after_fc ? 0 : 1));
+                      after_fc ? 0 : 1, SampleDraw{}));
+  ARL_LAUNCH_CHECK("heads_fwd_kernel");
+  return ARL_OK;
+}
+
+// heads + softmax + the epsilon-greedy draw, launched behind the fc256 kernel (arl_forward_egreedy)
+int heads_forward_egreedy(const float* params, int action_size, const float* h, float* logits, float* probs,
+                          float* value, int32_t* actions, int64_t env_id_base, int64_t step,
+                          const int64_t* step_dev, uint64_t seed, float ep, double ep_start, double ep_end,
+                          double ep_end_t, double learn_start, int64_t num_samples, cudaStream_t st) {
+  const ParamLayout L = param_layout(action_size);
+  const size_t smem = (size_t)(action_size + 1) * 256 * sizeof(float);
+  const int64_t ctas = (num_samples + kHfThreads / 32 - 1) / (kHfThreads / 32);
+  const int grid = (int)(ctas < 4LL * num_sms() ? ctas : 4LL * num_sms());
+  const EgreedyDraw draw = {ep, ep_start, ep_end, ep_end_t, learn_start};
+  ARL_CUDA(launch_pdl(heads_fwd_kernel<EgreedyDraw>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
+                      params + L.off[T_PB], params + L.off[T_QW], params + L.off[T_QB], h, logits, probs, value,
+                      num_samples, action_size, actions, (uint64_t)env_id_base, (uint64_t)step, seed, step_dev,
+                      0, draw));
   ARL_LAUNCH_CHECK("heads_fwd_kernel");
   return ARL_OK;
 }

@@ -78,18 +78,22 @@ class Agent(BaseModel):
         self.update_count = 0
         # loss_mode 'async_q' = the learner the reference actually runs (SURVEY D1): Q head,
         # epsilon-greedy, 1-step targets from a target network (agent.py:141-207, 298-314)
+        # loss_mode 'nstep_q' = the paper's asynchronous n-step Q-learning: the same Q head,
+        # epsilon-greedy schedule and target network, n-step returns bootstrapped from
+        # max_a Q(s_T; theta^-) -- the A3C cycle with another loss kernel, on the graph-replayed path
         self.loss_mode = getattr(config, 'loss_mode', 'a3c')
-        if self.loss_mode not in ('a3c', 'async_q'):
-            raise ValueError("loss_mode must be 'a3c' or 'async_q', got %r" % (self.loss_mode,))
-        if self.loss_mode == 'async_q':
-            self.network.make_target()
+        if self.loss_mode not in ('a3c', 'async_q', 'nstep_q'):
+            raise ValueError("loss_mode must be 'a3c', 'async_q' or 'nstep_q', got %r" % (self.loss_mode,))
+        self.has_target = self.loss_mode in ('async_q', 'nstep_q')
+        if self.has_target:
+            self.network.make_target(one_step=self.loss_mode == 'async_q')
             self._last_target_sync = 0
         # CUDA graphs of the loop (SURVEY a16): the device work of ``predict`` and of ``observe``
         # (+ the learner step at the end of a rollout) is captured once per distinct set of launch
         # arguments -- rollout slot, ring position, frame / reward buffers -- and replayed from then
         # on.  The two host values that change on every step, the Philox step and the step the
         # learning rate is annealed on, are read from ``step_dev`` (device memory) instead.
-        self.cuda_graphs = bool(getattr(config, 'cuda_graphs', True)) and self.loss_mode == 'a3c'
+        self.cuda_graphs = bool(getattr(config, 'cuda_graphs', True)) and self.loss_mode in ('a3c', 'nstep_q')
         self.max_graphs = int(getattr(config, 'max_graphs', 1024))
         self.graph_warmup_updates = 2                            # eager cycles first (lazy init, autotune)
         self.step_dev = torch.zeros(1, dtype=torch.int64, device=self.device)
@@ -108,7 +112,7 @@ class Agent(BaseModel):
         self.history.add(self.env.frames, replicate=self.history_length)
         self.t = 0
         self.update_target_q_network()                           # main.py:92
-        if self.loss_mode == 'async_q':
+        if self.has_target:
             self._last_target_sync = self.T
         return self.env.frames, 0, 0, self.env.terminal, range(self.step, self.max_step)
 
@@ -164,7 +168,7 @@ class Agent(BaseModel):
                 self.env.new_random_game(mask=terminal)
             if self.update_count != before:                      # agent.py:199-201
                 sums = self.network.loss_sums
-                if self.loss_mode == 'async_q':
+                if self.has_target:                              # async_q, nstep_q: {sum delta^2, sum Q}
                     n = float(self.t_max * B)
                     acc['loss'] += sums[0] / n
                     acc['q'] += sums[1] / n
@@ -221,6 +225,9 @@ class Agent(BaseModel):
         path = self.network.save_model(checkpoint_dir=d, step=self.step_op)
         if self.loss_mode == 'async_q':
             torch.save(self.network.target_params.cpu(), os.path.join(d, "target-%d.pt" % self.step_op))
+        elif self.loss_mode == 'nstep_q':                         # + where the sync schedule stands
+            torch.save({"target": self.network.target_params.cpu(), "last_target_sync": self._last_target_sync},
+                       os.path.join(d, "target-%d.pt" % self.step_op))
         return path
 
     def load_checkpoint(self, checkpoint_dir=None):
@@ -229,10 +236,14 @@ class Agent(BaseModel):
         if not self.network.load_model(checkpoint_dir=d):
             return False
         self.step_op = self.network.loaded_step
-        if self.loss_mode == 'async_q':
+        if self.has_target:
             p = os.path.join(d, "target-%d.pt" % self.step_op)
             if os.path.exists(p):
-                self.network.target_params.copy_(torch.load(p).to(self.device))
+                saved = torch.load(p)
+                if isinstance(saved, dict):                      # nstep_q
+                    self._last_target_sync = int(saved["last_target_sync"])
+                    saved = saved["target"]
+                self.network.target_params.copy_(saved.to(self.device))
             else:
                 self.network.update_target()
         return True
@@ -281,12 +292,19 @@ class Agent(BaseModel):
             net.forward(self.history, t)
             ep = self.ep if test_ep is None else test_ep
             return net.egreedy(t, self.step, self.seed, ep, self.env_id_base)
+        if self.loss_mode == 'nstep_q' and test_ep is not None:   # a fixed epsilon: eager
+            return net.forward_egreedy(self.history, t, self.seed, self.env_id_base, step=self.step, ep=test_ep)
         self._sync_step_dev()
         refresh = net._fc_w_stale()
 
         def launches():                                        # forward + heads + Philox draw
-            net.forward_sample(self.history, t, 0, self.seed, self.env_id_base, step_dev=self.step_dev,
-                               refresh=refresh)
+            if self.loss_mode == 'nstep_q':                    # agent.py:142-149, epsilon from step_dev
+                net.forward_egreedy(self.history, t, self.seed, self.env_id_base, step_dev=self.step_dev,
+                                    ep_sched=(self.ep_start, self.ep_end, self.ep_end_t, self.learn_start),
+                                    refresh=refresh)
+            else:
+                net.forward_sample(self.history, t, 0, self.seed, self.env_id_base, step_dev=self.step_dev,
+                                   refresh=refresh)
         self._run(('predict', t, self.history.head, refresh), launches)
         return net.sampled_action[net._rows(t)]
 
@@ -296,7 +314,8 @@ class Agent(BaseModel):
         History seeded with 4 copies of the first screen (agent.py:365-366), then predict / act
         (is_training=False: no life-loss terminal) / add until every env has finished its episode
         or ``n_step`` steps have passed.  Action selection: epsilon-greedy with ``test_ep``
-        (default ep_end, agent.py:352-353) in async_q mode, a sample from the policy in a3c mode.
+        (default ep_end, agent.py:352-353) in async_q / nstep_q mode, a sample from the policy in
+        a3c mode.
         Returns (best_reward, best_idx, per-episode mean reward over the envs); gym's monitor
         (agent.py:357-359) is the emulator's business and not reproduced."""
         if test_ep is None:
@@ -312,7 +331,7 @@ class Agent(BaseModel):
             for _ in range(int(n_step)):
                 # 1. predict   2. act   3. observe
                 action = self.network.evaluate(test_history, step, self.seed + 1,
-                                               ep=test_ep if self.loss_mode == 'async_q' else None,
+                                               ep=test_ep if self.has_target else None,
                                                env_id_base=self.env_id_base)
                 screen, reward, terminal = self.env.act(action, is_training=False, fused=True)
                 test_history.add(screen)
@@ -352,6 +371,9 @@ class Agent(BaseModel):
             new_head = (hist.head + 1) % hist.ring_slots
             hist.head = new_head                                 # host state first: the launches read it
             refresh = self.network._fc_w_stale() if will_update else False
+            # nstep_q: rebuild the target's weight image in this update only after a target sync
+            target_refresh = (self.loss_mode == 'nstep_q' and will_update
+                              and self.network._target_fc_w_stale())
 
             # bench.py: an event pair around K1 -- launched eagerly between its events, or (when the
             # events can be graph nodes) captured with the rest of the step
@@ -367,10 +389,10 @@ class Agent(BaseModel):
                            _cabi.ptr(self.batch_reward[t]), _cabi.ptr(self.batch_terminal[t]),
                            self.num_envs, _cabi.ptr(self.step_dev), 1, _cabi.stream_ptr())
                 if will_update:
-                    self._update_launches(refresh)
+                    self._update_launches(refresh, target_refresh)
             self._run(('observe', t, new_head, screen.data_ptr(), reward.data_ptr(),
                        terminal.data_ptr(), tuple(screen.shape), will_update, refresh, k1_eager,
-                       hist.timer is not None),
+                       hist.timer is not None, target_refresh),
                       launches)
             self._step_dev_host = self.step + 1
             self.t += 1
@@ -379,21 +401,24 @@ class Agent(BaseModel):
                 self.update_count += 1
                 self.t = 0
         self.T += self.global_envs                               # agent.py:165 counts every worker
-        if self.loss_mode == 'async_q' and \
-                self.T - self._last_target_sync >= self.target_q_update_step:
+        if self.has_target and self.T - self._last_target_sync >= self.target_q_update_step:
             self.update_target_q_network()                       # agent.py:166-167
             self._last_target_sync = self.T
 
-    def _update_launches(self, refresh):
-        """Device work of ``batch_update`` in a3c mode with the learning rate taken from the device
-        step counter (already advanced past the last frame of the rollout: offset -t_max gives
-        the step of the rollout's first frame, SURVEY §8 step 9)."""
+    def _update_launches(self, refresh, target_refresh=False):
+        """Device work of ``batch_update`` in a3c / nstep_q mode with the learning rate taken from
+        the device step counter (already advanced past the last frame of the rollout: offset -t_max
+        gives the step of the rollout's first frame, SURVEY §8 step 9)."""
         net = self.network
         in_lib = self.world_size > 1 and self.collective == 'library'
-        v_boot = net.bootstrap_value(self.history, refresh=refresh)
         scale = 1.0 / self.global_envs if self.reduce_mean else 1.0
-        net.compute_gradients(self.history, self.batch_reward, self.batch_terminal, v_boot,
-                              grad_scale=scale, allreduce=in_lib, refresh=False)
+        if self.loss_mode == 'nstep_q':
+            net.compute_nstep_q_gradients(self.history, self.batch_reward, self.batch_terminal, scale,
+                                          allreduce=in_lib, target_refresh=target_refresh, refresh=refresh)
+        else:
+            v_boot = net.bootstrap_value(self.history, refresh=refresh)
+            net.compute_gradients(self.history, self.batch_reward, self.batch_terminal, v_boot,
+                                  grad_scale=scale, allreduce=in_lib, refresh=False)
         if self.world_size > 1 and self.collective == 'torch':
             dist.all_reduce(net.grads, op=dist.ReduceOp.SUM)
         net.apply_gradients_sched(self.step_dev, -self.t_max, self.learning_rate, self.max_step,
@@ -409,6 +434,11 @@ class Agent(BaseModel):
             scale = 1.0 / (self.t_max * self.global_envs) if self.reduce_mean else 1.0 / self.t_max
             net.compute_q_gradients(self.history, self.batch_reward, self.batch_terminal, scale,
                                     allreduce=in_lib)
+        elif self.loss_mode == 'nstep_q':
+            # sum over t, mean over (global) envs: the A3C reduction (the paper accumulates over the rollout)
+            scale = 1.0 / self.global_envs if self.reduce_mean else 1.0
+            net.compute_nstep_q_gradients(self.history, self.batch_reward, self.batch_terminal, scale,
+                                          allreduce=in_lib)
         else:
             v_boot = net.bootstrap_value(self.history)           # R = V(s_T), masked if terminal
             scale = 1.0 / self.global_envs if self.reduce_mean else 1.0
@@ -421,8 +451,10 @@ class Agent(BaseModel):
         self.t = 0
 
     def update_target_q_network(self):
-        """agent.py:342-344 (async_q mode; the A3C path has no target network)."""
-        if self.loss_mode == 'async_q':
+        """agent.py:342-344 (async_q / nstep_q mode; the A3C path has no target network).  A host
+        copy outside the captured graphs; in nstep_q mode the next update then rebuilds the
+        target's weight image (Network._target_fc_w_stale)."""
+        if self.has_target:
             self.network.update_target()
 
     @property

@@ -403,14 +403,21 @@ class Network(object):
         return self.grads
 
     # -- async-Q mode (agent.py:169-207, 298-314): the Q head lives in the p_w/p_b slot ---------
-    def make_target(self):
-        """agent.py:257-296: a second parameter set, the target network."""
+    def make_target(self, one_step=True):
+        """agent.py:257-296: a second parameter set, the target network.  ``one_step``: also the
+        [T*B] target buffers of the 1-step learner (async_q); the n-step learner (nstep_q) evaluates
+        the target network on the B states s_T only (``q_boot``)."""
         self.target_params = self.params.clone()
-        N, A = self.num_envs * self.t_max, self.action_size
+        B, A = self.num_envs, self.action_size
+        N = B * self.t_max
         f32 = dict(device=self.device, dtype=torch.float32)
-        self.target_q = torch.empty(N, A, **f32)              # agent.py:186 q_t_plus_1
-        self.target_q_t = torch.empty(N, **f32)               # agent.py:190
-        self._tq_scratch = (torch.empty(N, A, **f32), torch.empty(N, **f32))
+        if one_step:
+            self.target_q = torch.empty(N, A, **f32)          # agent.py:186 q_t_plus_1
+            self.target_q_t = torch.empty(N, **f32)           # agent.py:190
+            self._tq_scratch = (torch.empty(N, A, **f32), torch.empty(N, **f32))
+        else:
+            self.q_boot = torch.empty(B, A, **f32)            # Q(s_T; theta^-)
+            self._target_fc_w_key = None
         self.target_fc_w = torch.empty(_cabi.prepared_floats(), device=self.device)
         return self.target_params
 
@@ -448,6 +455,65 @@ class Network(object):
                    history.ring_slots, history.first_slot(T), T, P(self.l1), P(self.l2), P(self.l4),
                    P(self.d_logits), P(self.d_value), P(self.d_l4), P(self.d_l2),
                    P(self.d_l1), P(self.grads), P(self.workspace), S, 1 if allreduce else 0, st)
+        return self.grads
+
+    # -- n-step Q mode (Mnih et al. 2016, asynchronous n-step Q-learning): the Q head is the p_w/p_b
+    # slot as in async_q; the cycle is the A3C cycle with the bootstrap taken from the target network
+    def _target_fc_w_stale(self):
+        """True (once) when target_params has changed since target_fc_w was made from it (a target
+        sync, a checkpoint load): torch bumps ``_version`` on every in-place write."""
+        key = self.target_params._version
+        stale = key != self._target_fc_w_key
+        self._target_fc_w_key = key
+        return stale
+
+    def forward_egreedy(self, history, t, seed, env_id_base=0, step_dev=None, ep_sched=None, refresh=None,
+                        step=0, ep=0.0):
+        """``forward`` into rollout slot t + the epsilon-greedy draw of agent.py:141-151 on the Q values
+        as one composed call (arl_forward_egreedy: the draw runs inside the heads launch).  With the
+        int64 device counter ``step_dev`` the step is ``step`` + *step_dev and epsilon is agent.py:142-144
+        evaluated on the device from it with ``ep_sched`` = (ep_start, ep_end, ep_end_t, learn_start);
+        without it the step is ``step`` and epsilon is ``ep``."""
+        r = self._rows(t)
+        P, st = _cabi.ptr, _cabi.stream_ptr()
+        refresh = (1 if self._fc_w_stale() else 0) if refresh is None else int(bool(refresh))
+        if step_dev is not None and ep_sched is None:
+            raise ValueError("forward_egreedy: step_dev needs ep_sched = (ep_start, ep_end, ep_end_t, learn_start)")
+        e0, e1, et, ls = (float(x) for x in (ep_sched if ep_sched is not None else (0.0, 0.0, 1.0, 0.0)))
+        self._timed_call("arl_forward_egreedy", P(self.params), P(self.fc_w), refresh, self.action_size,
+                         P(history.ring), self.num_envs, history.ring_slots, history.first_slot(0), P(self.l1[r]),
+                         P(self.l2[r]), P(self.l4[r]), P(self.policy_logits[r]), P(self.policy[r]),
+                         P(self.value[r]), P(self.sampled_action[r]), int(env_id_base), int(step),
+                         P(step_dev) if step_dev is not None else None, int(seed), float(ep), e0, e1, et, ls, st)
+        return self.sampled_action[r]
+
+    def compute_nstep_q_gradients(self, history, rewards, terminals, grad_scale, allreduce=False,
+                                  target_refresh=None, refresh=None):
+        """The n-step Q learner's gradient over the rollout: target-network forward over the B
+        states s_T (into ``q_boot``, after rebuilding target_fc_w when ``target_refresh``; None =
+        decide from the target's version), R_T = max_a q_boot, the n-step returns and dQ of the acted
+        actions (arl_nstep_q_lossgrad), then the backward (agent.py:317).  ``history`` must have had
+        exactly t_max pushes since s_0."""
+        T, B, A = self.t_max, self.num_envs, self.action_size
+        P, st = _cabi.ptr, _cabi.stream_ptr()
+        b = self._b
+        if target_refresh is None:
+            target_refresh = self._target_fc_w_stale()
+        self._timed_call("arl_forward", P(self.target_params), P(self.target_fc_w), int(bool(target_refresh)), A,
+                         P(history.ring), B, history.ring_slots, history.first_slot(0), 1, P(b['l1']), P(b['l2']),
+                         P(b['l4']), P(self.q_boot), P(b['probs']), P(b['value']), st)
+        self.loss_sums.zero_()
+        self._timed_call("arl_nstep_q_lossgrad", P(rewards), P(terminals), P(self.sampled_action),
+                         P(self.policy_logits), P(self.q_boot), P(self.R), P(self.d_logits), P(self.loss_sums),
+                         T, B, A, self.gamma, self.min_reward, self.max_reward, float(grad_scale), st)
+        self.d_value.zero_()                                   # the value head is unused
+        if self._fc_w_stale() if refresh is None else refresh:   # (a forward normally did this already)
+            _cabi.call("arl_prepare_weights", P(self.params), P(self.fc_w), st)
+        S = self.tensor_scale = self.pick_tensor_scale(grad_scale)
+        self._timed_call("arl_backward", P(self.params), P(self.fc_w), A, P(history.ring), B,
+                         history.ring_slots, history.first_slot(T), T, P(self.l1), P(self.l2), P(self.l4),
+                         P(self.d_logits), P(self.d_value), P(self.d_l4), P(self.d_l2),
+                         P(self.d_l1), P(self.grads), P(self.workspace), S, 1 if allreduce else 0, st)
         return self.grads
 
     @property

@@ -188,9 +188,12 @@ class NatureNetwork(Network):
             _cabi.call("arl_allreduce_grads", P(self.grads), int(self.grads.numel()), st)
         return self.grads
 
-    def make_target(self):
+    def make_target(self, one_step=True):
         raise NotImplementedError("loss_mode='async_q' runs the reference's agent.py net, which is the "
-                                  "nips trunk (agent.py:226-252); the nature trunk is A3C-only")
+                                  "nips trunk (agent.py:226-252); the nature trunk is A3C-only"
+                                  if one_step else
+                                  "loss_mode='nstep_q' is built on the nips trunk (agent.py:226-252); "
+                                  "the nature trunk is A3C-only")
 
     def _update(self, lr, step_dev, step_offset, base_lr, max_step, exchange=False):
         _cabi.call("arl_exchange_clip_rmsprop" if exchange else "arl_clip_rmsprop_layout",

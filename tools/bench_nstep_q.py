@@ -1,0 +1,123 @@
+"""Cycle time of the three learners on one GPU: a3c and nstep_q replayed from CUDA graphs, async_q
+eager (its own path: host epsilon, a separate draw launch, a target forward over all T*B next states).
+
+    python tools/bench_nstep_q.py [--rounds R] [--cycles K] [--out profiles/r03_nstep_q_bench.json]
+
+For each shape (envs x t_max x actions: 4096 x 5 x 6 and 16384 x 20 x 18) one agent per mode is built
+and warmed up until a whole ring period has replayed without a new graph capture; then the modes take
+turns, R rounds of K whole cycles each (t_max x (predict, act, observe) + the update), with a CUDA
+event pair around every K-cycle block.  Reported per mode: ms per cycle (median, min, max over the
+rounds) and env frames/s (envs x t_max / median cycle time).  The card's name and power limit are
+read in the same run and written beside the numbers.  Synthetic frames, resident in HBM; the frame
+pool is larger than L2 at both shapes.
+"""
+import argparse
+import importlib
+import json
+import os
+import random
+import statistics
+import subprocess
+import sys
+
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
+
+MODES = ("a3c", "nstep_q", "async_q")
+
+
+def card():
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader",
+                            "-i", str(torch.cuda.current_device())], capture_output=True, text=True, timeout=60)
+        name, power, clock = [x.strip() for x in q.stdout.strip().splitlines()[0].split(",")]
+        return {"name": name, "power_limit": power, "max_sm_clock": clock}
+    except Exception as e:                                       # report, never guess
+        return {"name": torch.cuda.get_device_name(), "power_limit": "unknown (%s)" % str(e)[:80]}
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--rounds", type=int, default=5)
+    ap.add_argument("--cycles", type=int, default=20, help="cycles per timed block")
+    ap.add_argument("--shapes", default="4096x5x6,16384x20x18", help="envs x t_max x actions, comma separated")
+    ap.add_argument("--modes", default=",".join(MODES))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_nstep_q_bench.json"))
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        sys.exit("bench_nstep_q: needs a CUDA device")
+    pkg = importlib.import_module("async-rl-tensorflow_b200")
+    dev = torch.device("cuda", 0)
+    torch.cuda.set_device(dev)
+    modes = args.modes.split(",")
+    result = {"card": card(), "rounds": args.rounds, "cycles_per_block": args.cycles, "shapes": []}
+
+    for shape in args.shapes.split(","):
+        B, T, A = (int(x) for x in shape.split("x"))
+        pool = max(2, min(T, int(24e9 // (B * 100800) // len(modes))))   # frames kept per agent
+        agents = {}
+        for mode in modes:
+            cfg = pkg.config.get_config({"model": "m1", "num_envs": B, "t_max": T, "loss_mode": mode})
+            env = pkg.GymEnvironment(cfg, env=pkg.SyntheticAtari(B, A, seed=123, pool=pool, device=dev), device=dev)
+            agent = pkg.Agent(cfg, env, device=dev)
+            random.seed(cfg.seed)
+            agent.before_train()
+            agents[mode] = (agent, env)
+
+        def cycles(mode, k):
+            agent, env = agents[mode]
+            for _ in range(k):
+                for _ in range(T):
+                    a = agent.predict()
+                    scr, rew, term = env.act(a, is_training=True, fused=True)
+                    agent.observe(scr, rew, a, term)
+                    agent.step += 1
+
+        for mode in modes:                                       # warm-up: every graph captured
+            agent = agents[mode][0]
+            cycles(mode, 3)
+            seen, quiet = len(agent._graphs), 0
+            for _ in range(64):
+                if not agent.cuda_graphs or quiet >= 3:
+                    break
+                cycles(mode, 1)
+                quiet = quiet + 1 if len(agent._graphs) == seen else 0
+                seen = len(agent._graphs)
+        torch.cuda.synchronize()
+        ms = {m: [] for m in modes}
+        for _ in range(args.rounds):
+            for mode in modes:                                   # the modes alternate
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                cycles(mode, args.cycles)
+                e1.record()
+                torch.cuda.synchronize()
+                ms[mode].append(e0.elapsed_time(e1) / args.cycles)
+        entry = {"envs": B, "t_max": T, "actions": A, "frame_pool_steps": pool, "modes": {}}
+        for mode in modes:
+            med = statistics.median(ms[mode])
+            agent = agents[mode][0]
+            entry["modes"][mode] = {"ms_per_cycle": round(med, 4), "ms_min": round(min(ms[mode]), 4),
+                                    "ms_max": round(max(ms[mode]), 4), "frames_per_sec": round(B * T / med * 1e3),
+                                    "graph_replayed": bool(agent.graph_replays), "graphs": len(agent._graphs)}
+        if "a3c" in modes:
+            for mode in modes:
+                entry["modes"][mode]["vs_a3c"] = round(entry["modes"][mode]["ms_per_cycle"] /
+                                                       entry["modes"]["a3c"]["ms_per_cycle"], 4)
+        result["shapes"].append(entry)
+        print(json.dumps(entry), flush=True)
+        del agents
+        torch.cuda.empty_cache()
+
+    os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+    with open(args.out, "w") as f:
+        json.dump(result, f, indent=1)
+        f.write("\n")
+    print(json.dumps({"card": result["card"], "out": args.out}))
+
+
+if __name__ == "__main__":
+    main()
