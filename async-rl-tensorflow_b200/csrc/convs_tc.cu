@@ -20,8 +20,8 @@
 //   wgrads     : dW[(tap,ch), co] = sum_P X[P+shift][ch] * dyz[P][co] reduces over ROWS, so the
 //                same row-major images serve as MN-major operands (k = row index); tap b is a
 //                second copy of the image shifted by one row, tap a a descriptor row offset.
-//                Work is split over row ranges (conv1) or CTAs (conv2); partials are summed in a
-//                fixed order.
+//                Work is split over ranges of (env, step window, row tile) units (conv1) or CTAs
+//                (conv2); partials are summed in a fixed order.
 #include <stdlib.h>
 
 #include "gemm_tc.cuh"
@@ -151,58 +151,12 @@ __device__ __forceinline__ void copy_image(uint8_t* res, const uint8_t* __restri
 // ---- conv1 A operand: space-to-depth rows of the u8 ring ---------------------------------------
 // The ring stores every 84x84 plane in 4x4 blocks (K1 writes it that way): the 16 bytes at
 // plane + q*16 are block q = y'*21 + x' = frame rows 4y'..4y'+3, columns 4x'..4x'+3 = the 16
-// channels plane c contributes to X row (n, y', x') -> chunks kc = 2c (rows 0,1) and 2c+1 (rows
-// 2,3).  Work unit = (row, plane): ONE 16-byte load; lanes run along the rows of one plane, so a
-// warp instruction reads 512 contiguous bytes.  U units are in flight per lane.
-// SHIFTED: also store the copy shifted by one row into planes 8..15 (tap b = 1 of the wgrad).
+// channels plane c contributes to X row (n, y', x').  Sample n = t*num_envs + b stacks the planes
+// of env b in ring slots (first_slot + t + c) mod ring_slots, c = 0..3.
 struct RingGeo {
   const uint8_t* ring;
   int num_envs, ring_slots, first_slot;
 };
-// split in two so that the loads of the NEXT stage can be in flight while the producer waits for
-// its shared-memory slot (PolicyBase::PREFETCH): U * gsize >= ROWS * 4, one round
-template <int ROWS, int U>
-__device__ __forceinline__ void x1_request(uint4 (&w)[U], const RingGeo& g, int xr0, int num_samples,
-                                           int glane, int gsize) {
-  constexpr int GROWS = 441, TOTAL = ROWS * 4;
-  const int n0 = xr0 / GROWS, q0 = xr0 - n0 * GROWS;
-  const int tt0 = n0 / g.num_envs, b0 = n0 - tt0 * g.num_envs;
-#pragma unroll
-  for (int u = 0; u < U; ++u) {
-    const int un = glane + u * gsize;
-    const int c = un / ROWS, r = un - c * ROWS;
-    int q = q0 + r, n = n0, tt = tt0, b = b0;
-    if (q >= GROWS) {                                      // ROWS < GROWS: at most one wrap
-      q -= GROWS; ++n; ++b;
-      if (b == g.num_envs) { b = 0; ++tt; }
-    }
-    w[u] = make_uint4(0u, 0u, 0u, 0u);
-    if (un < TOTAL && n < num_samples) {
-      int slot = g.first_slot + tt + c;
-      slot -= slot >= g.ring_slots ? g.ring_slots : 0;
-      slot -= slot >= g.ring_slots ? g.ring_slots : 0;
-      w[u] = __ldg(reinterpret_cast<const uint4*>(g.ring + ((size_t)b * g.ring_slots + slot) * kPlane) + q);
-    }
-  }
-}
-template <int ROWS, int PL, int U, bool SHIFTED>
-__device__ __forceinline__ void x1_store(uint8_t* img, const uint4 (&w)[U], int glane, int gsize) {
-  constexpr int TOTAL = ROWS * 4;
-#pragma unroll
-  for (int u = 0; u < U; ++u) {
-    const int un = glane + u * gsize;
-    if (un >= TOTAL) break;
-    const int c = un / ROWS, r = un - c * ROWS;
-    const uint4 lo2 = tc::bytes8_to_f16(w[u].x, w[u].y), hi2 = tc::bytes8_to_f16(w[u].z, w[u].w);   // exact
-    uint8_t* d = img + (2 * c) * PL + r * 16;
-    *reinterpret_cast<uint4*>(d) = lo2;
-    *reinterpret_cast<uint4*>(d + PL) = hi2;
-    if (SHIFTED && r > 0) {
-      *reinterpret_cast<uint4*>(d + 8 * PL - 16) = lo2;
-      *reinterpret_cast<uint4*>(d + 9 * PL - 16) = hi2;
-    }
-  }
-}
 
 // ---- a1 in HBM: fp16, blocked ("a1s") -----------------------------------------------------------
 // conv1's output is only ever consumed as a tensor-core operand (conv2 forward / backward) and as
@@ -518,15 +472,6 @@ struct Conv2Fwd : tc::PolicyBase {
 // kept a bf16 hi + lo pair (28 224 B).
 constexpr int kDy1sRows = 441;
 
-// work item `item` (= its partial slice `ks`) covers the row range number `range`
-__device__ __forceinline__ TileCoord range_tile(int item, int64_t rows, int k_chunk, int range) {
-  TileCoord t;
-  t.mt = item; t.nt = 0; t.ks = item;
-  const int64_t b = (int64_t)range * k_chunk;
-  t.k_begin = (int)b;
-  t.k_end = (int)(b + k_chunk < rows ? b + k_chunk : rows);
-  return t;
-}
 // per-lane bias sums (4 floats of every CF4-th float4) -> per-warp partial row of CF4*4 floats
 template <int CF4>
 __device__ __forceinline__ void bias_partial_store(float* dst_row, float (&acc)[4], int lane) {
@@ -753,9 +698,9 @@ struct Conv1WgradArgs {
   RingGeo geo;
   const uint8_t* dy1s;   // fp16 on the X grid, written by conv2 backward (see dy1s above)
   float* partials;       // [items][4096]
-  int64_t rows;          // 441 * num_samples
-  int num_samples, k_chunk, items;
-  int reverse;           // item i takes row range items-1-i (see serpentine())
+  int64_t dy1s_rows;     // 441 * num_samples: rows of one dy1s co group
+  int steps, windows;    // windows = steps per env / Conv1Wgrad::S, rounded up
+  int units, k_chunk, items;
 };
 struct Conv1Wgrad : tc::PolicyBase {
   using Args = Conv1WgradArgs;
@@ -763,79 +708,140 @@ struct Conv1Wgrad : tc::PolicyBase {
   // Both operands fp16: the u8 pixels are exact, dy1 is one fp16 per value.  Tap b is folded into M
   // (a second copy of the X image shifted by one row), tap a into N (a second copy of the dy1 image
   // shifted BACK by 21 rows: sum_Q X[Q + b][ch] * dy1[Q - 21][co]), so one N = 32 MMA per 16 rows
-  // covers all four taps and the wide X tile is read from shared memory once.  The dy1 images
-  // arrive by cp.async.bulk from dy1s (4 copies of 2 KB per stage).
-  static constexpr int GW = 21, TROWS = 129;
-  static constexpr int PLA = (TROWS + 1) * 16, A_IMG = 16 * PLA;   // u8 -> fp16, exact
-  static constexpr int PLB = 128 * 16, B_IMG = 2 * PLB;            // dy1: 2 co groups
-  // stage = [A | dy | dy']  (dy' = shifted copy = tap a = 1); five stages of 41 KB
-  static constexpr int PROD_WARPS = 20, STAGES = 5, STAGE_BYTES = A_IMG + 2 * B_IMG, RES_BYTES = 0;
+  // covers all four taps and the wide X tile is read from shared memory once.
+  //
+  // Work unit (one pipeline stage) = env b, a window of up to S consecutive steps t0 .. t0+S-1 of
+  // that env, grid rows [q0, q0 + R) of each of their samples.  Sample t stacks ring planes
+  // t .. t+3, so the window's S samples share S + 3 planes: the producers load and convert each of
+  // them ONCE per unit (the t-major row walk of round 3 converted every plane up to 4 times).  A
+  // image, cin-major: per plane c of the window, 4 chunk planes [rows 0-1 | rows 2-3 | the same
+  // two shifted by one grid row]; the M = 128 rows of sample t are then the 16 chunk planes of
+  // planes t .. t+3 at one uniform stride, i.e. one descriptor based at plane t.  The dy1 images
+  // of each sample ([dy | dy'] x 2 co groups) arrive by cp.async.bulk from dy1s.
+  // Each work item = one CTA's contiguous range of units, so a CTA's accumulator sums its range.
+  // S = 5 = the flagship t_max (one window per env); R = 64 (7 row tiles, 448 rows for 441):
+  // R = 32 would double the bulk copies per sample row, R = 128 would pad 441 rows to 512.
+  static constexpr int GW = 21, GROWS = 441, S = 5, R = 64, TILES = (GROWS + R - 1) / R;
+  static constexpr int XROWS = R + 1;                               // + the row the shifted copy needs
+  static constexpr int PLA = XROWS * 16, A_IMG = (S + 3) * 4 * PLA; // u8 -> fp16, exact
+  static constexpr int PLB = R * 16, B_IMG = 4 * PLB;               // per sample: [dy | dy'] x 2 co groups
+  // stage = [A | B of sample 0 .. S-1]: four stages of 53 KB
+  static constexpr int PROD_WARPS = 16, STAGES = 4, STAGE_BYTES = A_IMG + S * B_IMG, RES_BYTES = 0;
   // accumulator columns: a*16 + co
   static constexpr int ACC_COLS = 32, OUT_COLS = 32, LO_DELTA = 0, SEG = 16;
+  struct Unit { int b, t0, ns, q0; };
+  static __device__ __forceinline__ Unit unit(const Args& g, int u) {
+    const int ew = u / TILES, w = ew % g.windows;
+    Unit x;
+    x.q0 = (u - ew * TILES) * R;
+    x.b = ew / g.windows;
+    x.t0 = w * S;
+    x.ns = min(S, g.steps - x.t0);
+    return x;
+  }
   static __device__ __forceinline__ int acc_col(int c) { return c; }
   static __device__ __forceinline__ int num_items(const Args& g) { return g.items; }
   static __device__ __forceinline__ TileCoord coord(const Args& g, int item) {
-    return range_tile(item, g.rows, g.k_chunk, g.reverse ? g.items - 1 - item : item);
+    TileCoord t;
+    t.mt = item; t.nt = 0; t.ks = item;
+    t.k_begin = item * g.k_chunk;
+    t.k_end = min(g.units, t.k_begin + g.k_chunk);
+    return t;
   }
   static __device__ __forceinline__ int num_stages(const Args&, const TileCoord& t) {
-    return (t.k_end - t.k_begin + 127) / 128;
+    return t.k_end - t.k_begin;
   }
   static __device__ __forceinline__ void load_resident(const Args&, uint8_t*, int, int) {}
   // the u8 ring rows of the NEXT stage are requested (5 x 16 B per lane, held in registers) before
   // the producer waits for its slot: the ncu capture of round 1 showed producers 24 % of their time
-  // waiting for a free stage and then another 13 % on the first use of these loads
+  // waiting for a free stage and then another 13 % on the first use of these loads.  Load = (plane,
+  // row): ONE 16-byte vector; lanes run along the rows of one plane, so a warp instruction reads
+  // 512 contiguous bytes.  Rows past the sample (last row tile) load as zeros.
   static constexpr bool PREFETCH = true;
-  static constexpr int XU = 5;                                      // 20 warps / 5 stages = 128 lanes x 5 >= 129 x 4
+  static constexpr int XU = 5;                                      // 16 warps / 4 stages = 128 lanes x 5 >= 8 x 65
+  static_assert(XU * 32 * (PROD_WARPS / STAGES) >= (S + 3) * XROWS, "one round of loads per stage");
   struct Prod { uint4 w[XU]; };
   static __device__ __forceinline__ void prefetch_stage(const Args& g, const TileCoord& t, int s, int glane,
                                                         int gsize, Prod& ps) {
-    x1_request<TROWS, XU>(ps.w, g.geo, t.k_begin + s * 128, g.num_samples, glane, gsize);
-  }
-  static __device__ __forceinline__ void load_stage(const Args& g, const TileCoord& t, int s,
-                                                    uint8_t* st, int glane, int gsize, Prod& ps) {
-    const int p0 = t.k_begin + s * 128;
-    // A: X rows p0 .. p0+128 (exact in bf16: one image); planes 8..15 = shifted copy (tap b = 1)
-    x1_store<TROWS, PLA, XU, true>(st, ps.w, glane, gsize);
-    // B: image row r of planes 0..3 = dy1 row p0 + r, of planes 4..7 = dy1 row p0 + r - 21; rows
-    // with p0 + r >= k_end (the next work item's) and rows before the first sample are zero
-    const int valid = t.k_end - p0, lead = p0 < GW ? GW - p0 : 0;
-    if (valid < 128 || lead > 0) {
-      for (int i = glane; i < 4 * 128; i += gsize) {
-        const int plane = i >> 7, r = i & 127;
-        if (r >= valid || (plane >= 2 && r < lead))
-          *reinterpret_cast<uint4*>(st + A_IMG + plane * PLB + r * 16) = make_uint4(0u, 0u, 0u, 0u);
+    const Unit x = unit(g, t.k_begin + s);
+    const uint8_t* env = g.geo.ring + (size_t)x.b * g.geo.ring_slots * kPlane;
+#pragma unroll
+    for (int u = 0; u < XU; ++u) {
+      const int un = glane + u * gsize, c = un / XROWS, q = x.q0 + un - c * XROWS;
+      ps.w[u] = make_uint4(0u, 0u, 0u, 0u);
+      if (c < x.ns + 3 && q < GROWS) {
+        int slot = g.geo.first_slot + x.t0 + c;                     // < 2 * ring_slots
+        slot -= slot >= g.geo.ring_slots ? g.geo.ring_slots : 0;
+        ps.w[u] = __ldg(reinterpret_cast<const uint4*>(env + (size_t)slot * kPlane) + q);
       }
     }
   }
-  // lanes 0..3 of the stage's group own one dy1 plane each: plane = copy*2 + co group
+  static __device__ __forceinline__ void load_stage(const Args& g, const TileCoord& t, int s,
+                                                    uint8_t* st, int glane, int gsize, Prod& ps) {
+    const Unit x = unit(g, t.k_begin + s);
+    // A: chunk planes 4c, 4c+1 = X rows q0 .. q0+R of plane c; 4c+2, 4c+3 = the copy shifted by one
+    // row (tap b = 1)
+#pragma unroll
+    for (int u = 0; u < XU; ++u) {
+      const int un = glane + u * gsize, c = un / XROWS, r = un - c * XROWS;
+      if (c >= x.ns + 3) break;
+      const uint4 lo2 = tc::bytes8_to_f16(ps.w[u].x, ps.w[u].y), hi2 = tc::bytes8_to_f16(ps.w[u].z, ps.w[u].w);
+      uint8_t* d = st + 4 * c * PLA + r * 16;
+      *reinterpret_cast<uint4*>(d) = lo2;
+      *reinterpret_cast<uint4*>(d + PLA) = hi2;
+      if (r > 0) {
+        *reinterpret_cast<uint4*>(d + 2 * PLA - 16) = lo2;
+        *reinterpret_cast<uint4*>(d + 3 * PLA - 16) = hi2;
+      }
+    }
+    // B of sample i, planes 4i + (0, 1) = dy1 rows q0 + r, 4i + (2, 3) = dy1 rows q0 + r - 21.  Rows
+    // past the sample (last row tile) and the 21 rows before it (first row tile) are zero here;
+    // bulk_stage copies the others.
+    const int valid = min(R, GROWS - x.q0), lead = x.q0 == 0 ? GW : 0;
+    if (valid < R || lead > 0) {
+      for (int i = glane; i < x.ns * 4 * R; i += gsize) {
+        const int sp = i / R, r = i - sp * R;
+        if ((sp & 2) ? r < lead : r >= valid)
+          *reinterpret_cast<uint4*>(st + A_IMG + sp * PLB + r * 16) = make_uint4(0u, 0u, 0u, 0u);
+      }
+    }
+  }
+  // lanes 0 .. 4*ns-1 of the stage's group own one dy1 plane each: sample i = lane / 4,
+  // plane = copy*2 + co group
   static __device__ __forceinline__ bool bulk_stage(const Args& g, const TileCoord& t, int s, uint8_t* st,
                                                     int glane, int, uint64_t* full) {
-    if (glane >= 4) return false;
-    const int p0 = t.k_begin + s * 128;
-    int cnt = t.k_end - p0 < 128 ? t.k_end - p0 : 128, src = p0, dst = 0;
-    if (glane >= 2) {
-      src = p0 - GW;
-      if (src < 0) { dst = -src; cnt -= dst; src = 0; }
+    const Unit x = unit(g, t.k_begin + s);
+    if (glane >= 4 * x.ns) return false;
+    const int n = (x.t0 + (glane >> 2)) * g.geo.num_envs + x.b;
+    int src = x.q0, dst = 0, cnt = min(R, GROWS - x.q0);
+    if (glane & 2) {
+      src = x.q0 - GW; cnt = R;
+      if (src < 0) { dst = -src; cnt += src; src = 0; }
     }
-    const uint32_t bytes = cnt > 0 ? (uint32_t)cnt * 16u : 0u;
-    mbar_expect_tx(full, bytes);
-    if (cnt > 0)
-      bulk_g2s(st + A_IMG + glane * PLB + dst * 16, g.dy1s + ((int64_t)(glane & 1) * g.rows + src) * 16, bytes, full);
+    mbar_expect_tx(full, (uint32_t)cnt * 16u);
+    bulk_g2s(st + A_IMG + glane * PLB + dst * 16,
+             g.dy1s + ((glane & 1) * g.dy1s_rows + (int64_t)n * GROWS + src) * 16, (uint32_t)cnt * 16u, full);
     return true;
   }
-  static __device__ __forceinline__ void issue(const Args&, const TileCoord&, int s, uint32_t st,
+  static __device__ __forceinline__ void issue(const Args& g, const TileCoord& t, int s, uint32_t st,
                                                uint32_t, uint32_t d) {
     constexpr uint32_t idesc = tc::make_idesc_h(32, true, true);   // [x ; x shifted] . [dy | dy']
-    // a_img = st, b_hi = st + A_IMG; one descriptor derivation per stage
+    const int ns = unit(g, t.k_begin + s).ns;
+    // one descriptor derivation per stage; sample i: A at plane i, B at its own image
     const uint64_t da0 = tc::make_sdesc(st, 128, PLA), db0 = tc::make_sdesc(st + A_IMG, 128, PLB);
 #pragma unroll
-    for (int k16 = 0; k16 < 8; ++k16)
-      tc::umma_f16(d, tc::sdesc_advance(da0, k16 * 256), tc::sdesc_advance(db0, k16 * 256), idesc,
-                   (s | k16) != 0 ? 1u : 0u);
+    for (int i = 0; i < S; ++i) {
+      if (i >= ns) break;
+#pragma unroll
+      for (int k16 = 0; k16 < R / 16; ++k16)
+        tc::umma_f16(d, tc::sdesc_advance(da0, i * 4 * PLA + k16 * 256),
+                     tc::sdesc_advance(db0, i * B_IMG + k16 * 256), idesc, (s | i | k16) != 0 ? 1u : 0u);
+    }
   }
-  // row = b*64 + ch, ch = (cin*4 + i)*4 + j ; segment a = 16 co of tap (kh = 4a+i, kw = 4b+j)
+  // row = cin*32 + b*16 + i*4 + j (chunk plane 4*cin + 2b + i/2); segment a = 16 co of tap
+  // (kh = 4a+i, kw = 4b+j)
   static __device__ __forceinline__ float* row_ptr(const Args& g, const TileCoord& t, int row) {
-    const int b = row >> 6, ch = row & 63, cin = ch >> 4, i = (ch >> 2) & 3, j = ch & 3;
+    const int cin = row >> 5, b = (row >> 4) & 1, i = (row >> 2) & 3, j = row & 3;
     const int kw = 4 * b + j;
     return g.partials + (size_t)t.ks * 4096 + ((i * 8 + kw) * 4 + cin) * 16;
   }
@@ -874,19 +880,12 @@ static_assert(Conv1Fwd::RES_BYTES <= kPrepW1Bytes && Conv2Fwd::RES_BYTES <= kPre
 // Serpentine sweep: consecutive kernels of a chain walk the samples in OPPOSITE directions, so a
 // kernel starts with the rows its predecessor touched last -- the ones still in the 126 MB L2 --
 // instead of the ones evicted longest ago.  forward: conv1 up, conv2 DOWN; backward: fc dgrad up,
-// conv2 backward DOWN, conv1 wgrad DOWN.  (conv1 wgrad gives each CTA one contiguous row range, so
-// its direction hardly changes which rows are read first: up measured the same, 244 us per cycle
-// at 4096 envs x t_max 5 on one B200.)  ARL_SERPENTINE=0 turns it off (A/B runs).
+// conv2 backward DOWN.  (conv1 wgrad walks envs, and the samples of one env lie at a stride of
+// num_envs samples across all of d_a1, so no direction starts with the rows conv2 backward wrote
+// last.)  ARL_SERPENTINE=0 turns it off (A/B runs).
 bool serpentine() {
   static const bool on = [] { const char* e = getenv("ARL_SERPENTINE"); return !(e && e[0] == '0'); }();
   return on;
-}
-
-int split_rows(int64_t rows, int want, int* k_chunk) {
-  int64_t per = (rows + want - 1) / want;
-  per = (per + 127) / 128 * 128;
-  *k_chunk = (int)per;
-  return (int)((rows + per - 1) / per);
 }
 
 }  // namespace
@@ -955,10 +954,13 @@ extern "C" int arl_conv1_backward(const uint8_t* ring, const float* d_a1, float*
   g.geo = {ring, num_envs, ring_slots, first_slot};
   g.dy1s = reinterpret_cast<const uint8_t*>(d_a1);
   g.partials = (float*)workspace;
-  g.rows = N * 441;
-  g.num_samples = (int)N;
-  g.items = split_rows(g.rows, num_sms(), &g.k_chunk);
-  g.reverse = serpentine() ? 1 : 0;
+  g.dy1s_rows = N * 441;
+  g.steps = steps;
+  g.windows = (steps + Conv1Wgrad::S - 1) / Conv1Wgrad::S;
+  g.units = num_envs * g.windows * Conv1Wgrad::TILES;              // <= 7 N: fits int
+  // one contiguous range of units per CTA: at most num_sms() partials
+  g.k_chunk = (g.units + num_sms() - 1) / num_sms();
+  g.items = (g.units + g.k_chunk - 1) / g.k_chunk;
   int rc = tc::launch<Conv1Wgrad>(g, g.items, st);
   if (rc) return rc;
   return reduce_partials_scaled(g.partials, grads, g.items, 4096, grad_unscale, st);   // l1_w
