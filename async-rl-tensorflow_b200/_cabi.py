@@ -1,4 +1,4 @@
-"""ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h, include/asyncrl_b200_nstep_q.h).
+"""ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h).
 
 The product path has no CPU fallback: if the shared library is missing or a call
 fails, this module raises.  PyTorch is only the carrier of device memory and
@@ -36,6 +36,9 @@ SIGNATURES = {
                              c_i64, c_vp],
     "arl_forward_sample": [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
                            c_vp, c_vp, c_i64, c_i64, c_vp, c_u64, c_vp],
+    "arl_forward_egreedy": [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
+                            c_vp, c_vp, c_i64, c_i64, c_vp, c_u64, c_f32, ctypes.c_double, ctypes.c_double,
+                            ctypes.c_double, ctypes.c_double, c_vp],
     "arl_debug_gemm": [c_int, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_vp],
     "arl_sample_actions": [c_vp, c_vp, c_int, c_int, c_i64, c_i64, c_u64, c_vp],
     "arl_greedy_actions": [c_vp, c_vp, c_int, c_int, c_vp],
@@ -44,6 +47,8 @@ SIGNATURES = {
     "arl_observe_store": [c_vp, c_vp, c_vp, c_vp, c_int, c_vp],
     "arl_q_lossgrad": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_f32, c_f32,
                        c_f32, c_f32, c_vp],
+    "arl_nstep_q_lossgrad": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_f32, c_f32,
+                             c_f32, c_f32, c_vp],
     "arl_returns_lossgrad": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int,
                              c_int, c_int, c_f32, c_f32, c_f32, c_f32, c_f32, c_vp],
     "arl_heads_backward": [c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_vp],
@@ -89,15 +94,6 @@ OTHER = {
 }
 EXPORTS = tuple(SIGNATURES) + tuple(OTHER)
 
-# the n-step Q-learning entries: their own header (include/asyncrl_b200_nstep_q.h), their own table
-NSTEP_Q_SIGNATURES = {
-    "arl_forward_egreedy": [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
-                            c_vp, c_vp, c_i64, c_i64, c_vp, c_u64, c_f32, ctypes.c_double, ctypes.c_double,
-                            ctypes.c_double, ctypes.c_double, c_vp],
-    "arl_nstep_q_lossgrad": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_f32, c_f32,
-                             c_f32, c_f32, c_vp],
-}
-
 
 class ArlError(RuntimeError):
     pass
@@ -116,7 +112,7 @@ def load():
         raise ArlError("%s is missing: build it with async-rl-tensorflow_b200/csrc/build.sh "
                        "(or __graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = ctypes.CDLL(LIB_PATH)
-    for name, argtypes in list(SIGNATURES.items()) + list(NSTEP_Q_SIGNATURES.items()):
+    for name, argtypes in SIGNATURES.items():
         fn = getattr(lib, name)
         fn.argtypes, fn.restype = argtypes, c_int
     for name, (argtypes, restype) in OTHER.items():

@@ -99,10 +99,20 @@ extern "C" int64_t arl_a2_block_rows(int num_envs) {
   return num_envs;
 }
 
+namespace arl {
+template <class Draw>
+int fc_heads_forward(const float* params, const float* prepared, int action_size, const float* a2, float* h,
+                     float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base, int64_t step,
+                     const int64_t* step_dev, uint64_t seed, int64_t num_samples, Draw draw, void* stream);
+}
+
+// One env step of the forward, env range by env range; `draw` is the action draw of the heads launch
+// (common.cuh: SampleDraw with actions == NULL draws nothing)
+template <class Draw>
 static int forward_step(const float* params, float* prepared, int action_size, const uint8_t* ring,
                         int num_envs, int ring_slots, int first_slot, float* a1, float* a2, float* h,
                         float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base,
-                        int64_t step, const int64_t* step_dev, uint64_t seed, void* stream) {
+                        int64_t step, const int64_t* step_dev, uint64_t seed, Draw draw, void* stream) {
   const int chunk = (int)arl_a2_block_rows(num_envs);
   for (int off = 0; off < num_envs; off += chunk) {
     const int n = num_envs - off < chunk ? num_envs - off : chunk;
@@ -115,10 +125,9 @@ static int forward_step(const float* params, float* prepared, int action_size, c
     rc = arl_conv2_forward(prepared, a1c, a2c, n, stream);
     if (rc) return rc;
     // fc256, then heads + softmax (+ the action draw) in one launch
-    rc = arl_fc_heads_forward(params, prepared, action_size, a2c, hc, logits + (size_t)off * action_size,
-                              probs + (size_t)off * action_size, value + off,
-                              actions ? actions + off : nullptr, env_id_base + off, step, step_dev, seed, n,
-                              stream);
+    rc = fc_heads_forward(params, prepared, action_size, a2c, hc, logits + (size_t)off * action_size,
+                          probs + (size_t)off * action_size, value + off, actions ? actions + off : nullptr,
+                          env_id_base + off, step, step_dev, seed, n, draw, stream);
     if (rc) return rc;
   }
   return ARL_OK;
@@ -134,7 +143,7 @@ extern "C" int arl_forward(const float* params, float* prepared, int refresh_pre
   if (rc) return rc;
   if (steps == 1)
     return forward_step(params, prepared, action_size, ring, num_envs, ring_slots, first_slot, a1, a2, h,
-                        logits, probs, value, nullptr, 0, 0, nullptr, 0, stream);
+                        logits, probs, value, nullptr, 0, 0, nullptr, 0, SampleDraw{}, stream);
   rc = arl_conv1_forward(prepared, ring, a1, num_envs, ring_slots, first_slot, steps, stream);
   if (rc) return rc;
   rc = arl_conv2_forward(prepared, a1, a2, N, stream);
@@ -153,7 +162,31 @@ extern "C" int arl_forward_sample(const float* params, float* prepared, int refr
   if (refresh_prepared) rc = arl_prepare_weights(params, prepared, stream);
   if (rc) return rc;
   return forward_step(params, prepared, action_size, ring, num_envs, ring_slots, first_slot, a1, a2, h,
-                      logits, probs, value, actions, env_id_base, step, step_dev, seed, stream);
+                      logits, probs, value, actions, env_id_base, step, step_dev, seed, SampleDraw{}, stream);
+}
+
+extern "C" int arl_forward_egreedy(const float* params, float* prepared, int refresh_prepared, int action_size,
+                                   const uint8_t* ring, int num_envs, int ring_slots, int first_slot,
+                                   float* a1, float* a2, float* h, float* logits, float* probs, float* value,
+                                   int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev,
+                                   uint64_t seed, float ep, double ep_start, double ep_end, double ep_end_t,
+                                   double learn_start, void* stream) {
+  ARL_REQUIRE(params && prepared && ring && a1 && a2 && h && logits && probs && value && actions,
+              "arl_forward_egreedy: null pointer");
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_forward_egreedy: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
+  ARL_REQUIRE(num_envs >= 0 && env_id_base >= 0 && step >= 0, "arl_forward_egreedy: negative argument");
+  ARL_REQUIRE(ep >= 0.f && ep <= 1.f, "arl_forward_egreedy: ep %f outside [0,1]", (double)ep);
+  ARL_REQUIRE(step_dev == nullptr || (ep_start >= 0.0 && ep_start <= 1.0 && ep_end >= 0.0 && ep_end <= 1.0),
+              "arl_forward_egreedy: ep_start %f / ep_end %f outside [0,1]", ep_start, ep_end);
+  ARL_REQUIRE(step_dev == nullptr || ep_end_t > 0.0, "arl_forward_egreedy: ep_end_t must be > 0");
+  if (num_envs == 0) return ARL_OK;
+  int rc = ARL_OK;
+  if (refresh_prepared) rc = arl_prepare_weights(params, prepared, stream);
+  if (rc) return rc;
+  return forward_step(params, prepared, action_size, ring, num_envs, ring_slots, first_slot, a1, a2, h,
+                      logits, probs, value, actions, env_id_base, step, step_dev, seed,
+                      EgreedyDraw{ep, ep_start, ep_end, ep_end_t, learn_start}, stream);
 }
 
 extern "C" int arl_backward(const float* params, const float* prepared, int action_size,

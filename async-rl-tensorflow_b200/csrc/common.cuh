@@ -52,6 +52,19 @@ inline ParamLayout param_layout(int A) {
 
 constexpr int kPlane = ARL_SCREEN * ARL_SCREEN;  // 7056 bytes, 441 x 16 B
 
+// The action draw of a heads launch (heads.cu heads_fwd_kernel's template argument): SampleDraw is
+// the policy sample of network.py:72, or no draw at all when `actions` is NULL; EgreedyDraw is
+// agent.py:141-151 on the logits (arl_forward_egreedy).  SampleDraw carries nothing and its branch
+// is the only one compiled in, so the A3C path pays nothing for the second kind.
+struct SampleDraw {
+  static constexpr bool kEgreedy = false;
+};
+struct EgreedyDraw {
+  static constexpr bool kEgreedy = true;
+  float ep;                                          // used when step_dev == nullptr
+  double ep_start, ep_end, ep_end_t, learn_start;    // used with step_dev (agent.py:142-144)
+};
+
 // "prepared" weights (arl_prepare_weights): the operand images the tensor-core kernels keep
 // resident, built once per parameter change instead of in every kernel prologue.  Byte offsets:
 constexpr int64_t kPrepFcW = 0;                                   // l4_w as a split block (fc.cu)

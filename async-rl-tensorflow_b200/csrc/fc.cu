@@ -18,10 +18,10 @@ int reduce_partials(const float* partials, float* out, int num_partials, int n,
                     cudaStream_t stream);
 int reduce_partials_scaled(const float* partials, float* out, int num_partials, int n, float alpha,
                            cudaStream_t stream);
-int heads_forward_sample(const float* params, int action_size, const float* h, float* logits, float* probs,
-                         float* value, int32_t* actions, int64_t env_id_base, int64_t step,
-                         const int64_t* step_dev, uint64_t seed, int64_t num_samples, cudaStream_t st,
-                         bool after_fc = false);
+template <class Draw>
+int heads_forward(const float* params, int action_size, const float* h, float* logits, float* probs, float* value,
+                  int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev, uint64_t seed,
+                  int64_t num_samples, int wait_first, Draw draw, cudaStream_t st);
 
 // X fp32 [rows][8*chunks] (row stride ld) -> one split block [part][chunk][row][8 bf16].
 // Thread = (row, chunk): reads 32 contiguous bytes, writes one hi and one lo vector.
@@ -316,11 +316,12 @@ extern "C" int arl_fc_forward(const float* params, const float* prepared, const 
   return fc_forward_impl(params, prepared, a2, h, num_samples, (cudaStream_t)stream);
 }
 
-extern "C" int arl_fc_heads_forward(const float* params, const float* prepared, int action_size,
-                                    const float* a2, float* h, float* logits, float* probs, float* value,
-                                    int32_t* actions, int64_t env_id_base, int64_t step,
-                                    const int64_t* step_dev, uint64_t seed, int64_t num_samples,
-                                    void* stream) {
+namespace arl {
+// arl_fc_heads_forward with the action draw `draw` (common.cuh): the forward entries of api.cu end here
+template <class Draw>
+int fc_heads_forward(const float* params, const float* prepared, int action_size, const float* a2, float* h,
+                     float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base, int64_t step,
+                     const int64_t* step_dev, uint64_t seed, int64_t num_samples, Draw draw, void* stream) {
   ARL_REQUIRE(params && prepared && a2 && h && logits && probs && value, "arl_fc_heads_forward: null pointer");
   ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
               "arl_fc_heads_forward: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
@@ -331,9 +332,23 @@ extern "C" int arl_fc_heads_forward(const float* params, const float* prepared, 
   if (num_samples == 0) return ARL_OK;
   int rc = fc_forward_impl(params, prepared, a2, h, num_samples, (cudaStream_t)stream);
   if (rc) return rc;
-  // heads + softmax + (optionally) the Philox draw: one warp-per-sample kernel
-  return heads_forward_sample(params, action_size, h, logits, probs, value, actions, env_id_base, step, step_dev,
-                              seed, num_samples, (cudaStream_t)stream, /*after_fc=*/true);
+  // heads + softmax + (optionally) the draw: one warp-per-sample kernel
+  return heads_forward(params, action_size, h, logits, probs, value, actions, env_id_base, step, step_dev, seed,
+                       num_samples, /*wait_first=*/0, draw, (cudaStream_t)stream);
+}
+template int fc_heads_forward(const float*, const float*, int, const float*, float*, float*, float*, float*,
+                              int32_t*, int64_t, int64_t, const int64_t*, uint64_t, int64_t, SampleDraw, void*);
+template int fc_heads_forward(const float*, const float*, int, const float*, float*, float*, float*, float*,
+                              int32_t*, int64_t, int64_t, const int64_t*, uint64_t, int64_t, EgreedyDraw, void*);
+}  // namespace arl
+
+extern "C" int arl_fc_heads_forward(const float* params, const float* prepared, int action_size,
+                                    const float* a2, float* h, float* logits, float* probs, float* value,
+                                    int32_t* actions, int64_t env_id_base, int64_t step,
+                                    const int64_t* step_dev, uint64_t seed, int64_t num_samples,
+                                    void* stream) {
+  return fc_heads_forward(params, prepared, action_size, a2, h, logits, probs, value, actions, env_id_base, step,
+                          step_dev, seed, num_samples, SampleDraw{}, stream);
 }
 
 extern "C" int arl_fc_backward(const float* prepared, const float* a2, int64_t a2_block_rows,

@@ -44,18 +44,8 @@ __device__ __forceinline__ void philox_two(uint32_t c0, uint32_t c1, uint32_t c2
 // across the lanes.  (First version: 16 samples per CTA staged in shared memory, one thread per
 // (sample, output) walking 256 k serially: 10 us per 4096 samples, latency-bound.)
 //
-// The action draw after the heads is chosen by the last argument's type: SampleDraw (network.py:72,
-// the A3C policy sample) or EgreedyDraw (agent.py:141-151 on the logits, the n-step Q learner of
-// arl_forward_egreedy).  SampleDraw carries nothing and its branch is the only one compiled in, so the
-// A3C path pays nothing for the second kind.
-struct SampleDraw {
-  static constexpr bool kEgreedy = false;
-};
-struct EgreedyDraw {
-  static constexpr bool kEgreedy = true;
-  float ep;                                          // used when step_dev == nullptr
-  double ep_start, ep_end, ep_end_t, learn_start;    // used with step_dev (agent.py:142-144)
-};
+// The action draw after the heads is chosen by the last argument's type (common.cuh: SampleDraw or
+// EgreedyDraw).
 
 // agent.py:142-144  ep_end + max(0., (ep_start - ep_end) * (ep_end_t - max(0., step - learn_start))
 // / ep_end_t), in double, one correctly rounded operation at a time in Python's order (the _rn
@@ -220,6 +210,48 @@ __global__ void egreedy_actions_kernel(const float* __restrict__ q, int32_t* __r
   actions[b] = a;
 }
 
+// ------------------------------- loss-kernel pieces ---------------------------------------
+// Shared by the three loss kernels below: the n-step return (A3C and n-step Q, so that their R is
+// bit-identical by construction), and the max over a Q row, the dQ row and the loss sums (async-Q
+// and n-step Q).
+
+// Algorithm 3 + agent.py:154,188-190: R_t of sample (t, b) from the bootstrap R_T, the recurrence
+// run from T-1 down to t -- the same operations in the same order as a walk over the whole rollout
+// (identical bits), T - t fused multiply-adds
+__device__ __forceinline__ float nstep_return(const float* rewards, const uint8_t* terminals, float R, int t,
+                                              int T, int B, int b, float gamma, float rmin, float rmax) {
+  for (int tt = T - 1; tt >= t; --tt) {
+    const size_t m = (size_t)tt * B + b;
+    const float r = fminf(fmaxf(rewards[m], rmin), rmax);               // agent.py:154
+    R = fmaf(gamma * (1.0f - (terminals[m] ? 1.0f : 0.0f)), R, r);      // agent.py:190
+  }
+  return R;
+}
+
+// max_a q[a], fmaxf in index order
+__device__ __forceinline__ float q_row_max(const float* q, int A) {
+  float mx = q[0];
+  for (int j = 1; j < A; ++j) mx = fmaxf(mx, q[j]);
+  return mx;
+}
+
+// the gradient of grad_scale * delta^2 w.r.t. the Q row: -2 * delta * grad_scale at the acted action
+__device__ __forceinline__ void acted_dq_row(float* dq, int A, int a, float delta, float grad_scale) {
+  for (int j = 0; j < A; ++j) dq[j] = j == a ? -2.0f * delta * grad_scale : 0.f;
+}
+
+// loss_sums (optional) += {sum delta^2, sum Q(s)[a]}: a warp sum, then one atomic per warp
+__device__ __forceinline__ void add_q_loss_sums(float* loss_sums, float s_loss, float s_q) {
+  if (loss_sums) {
+    s_loss = warp_sum(s_loss);
+    s_q = warp_sum(s_q);
+    if ((threadIdx.x & 31) == 0) {
+      atomicAdd(loss_sums + 0, s_loss);
+      atomicAdd(loss_sums + 1, s_q);
+    }
+  }
+}
+
 // ------------------------------- async-Q loss gradients -----------------------------------
 // agent.py:186-190, 310-314: target = clip(r) + (1 - terminal) * discount * max_a Q_target(s'),
 // delta = target - Q(s)[a], loss = mean(delta^2)  ->  dQ[a] = -2 * delta * grad_scale.
@@ -233,34 +265,24 @@ __global__ void q_lossgrad_kernel(const float* __restrict__ rewards,
   const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   float s_loss = 0.f, s_q = 0.f;
   if (n < num_samples) {
-    const float* qn = q_next + n * A;
-    float mx = qn[0];
-    for (int j = 1; j < A; ++j) mx = fmaxf(mx, qn[j]);
+    const float mx = q_row_max(q_next + n * A, A);
     const float r = fminf(fmaxf(rewards[n], rmin), rmax);                 // agent.py:154
     const float tgt = fmaf((1.0f - (terminals[n] ? 1.0f : 0.0f)) * discount, mx, r);   // agent.py:190
     const int a = actions[n];
     const float delta = tgt - q[n * A + a];
     target[n] = tgt;
-    for (int j = 0; j < A; ++j) dq[n * A + j] = j == a ? -2.0f * delta * grad_scale : 0.f;
+    acted_dq_row(dq + n * A, A, a, delta, grad_scale);
     s_loss = delta * delta;
     s_q = q[n * A + a];
   }
-  if (loss_sums) {
-    s_loss = warp_sum(s_loss);
-    s_q = warp_sum(s_q);
-    if ((threadIdx.x & 31) == 0) {
-      atomicAdd(loss_sums + 0, s_loss);
-      atomicAdd(loss_sums + 1, s_q);
-    }
-  }
+  add_q_loss_sums(loss_sums, s_loss, s_q);
 }
 
 // ------------------------------- returns + loss gradients ---------------------------------
 // One thread per SAMPLE (t, b): the return recurrence is the only serial part, and it is T - t
-// fused multiply-adds, so every thread just runs it from T-1 down to its own t (the same operations
-// in the same order as a walk over the whole rollout: identical bits) and then does the softmax /
-// gradient work of its one sample.  (One thread per env walking all T samples: 32 CTAs for 4096
-// envs, 14.4 us.)
+// fused multiply-adds, so every thread just runs it from T-1 down to its own t (nstep_return) and
+// then does the softmax / gradient work of its one sample.  (One thread per env walking all T
+// samples: 32 CTAs for 4096 envs, 14.4 us.)
 __global__ void returns_lossgrad_kernel(const float* __restrict__ rewards,
                                         const uint8_t* __restrict__ terminals,
                                         const int32_t* __restrict__ actions,
@@ -276,12 +298,7 @@ __global__ void returns_lossgrad_kernel(const float* __restrict__ rewards,
   pdl_wait();
   if (n < (int64_t)T * B) {
     const int t = (int)(n / B), b = (int)(n - (int64_t)t * B);
-    float R = v_boot[b];
-    for (int tt = T - 1; tt >= t; --tt) {
-      const size_t m = (size_t)tt * B + b;
-      const float r = fminf(fmaxf(rewards[m], rmin), rmax);               // agent.py:154
-      R = fmaf(gamma * (1.0f - (terminals[m] ? 1.0f : 0.0f)), R, r);      // agent.py:190
-    }
+    const float R = nstep_return(rewards, terminals, v_boot[b], t, T, B, b, gamma, rmin, rmax);
     returns[n] = R;
     const float* z = logits + n * A;
     float zz[ARL_MAX_ACTIONS];
@@ -318,6 +335,34 @@ __global__ void returns_lossgrad_kernel(const float* __restrict__ rewards,
       atomicAdd(loss_sums + 2, s_ent);
     }
   }
+}
+
+// ------------------------------- n-step Q loss gradients ----------------------------------
+// Asynchronous n-step Q-learning (Mnih et al. 2016): one thread per SAMPLE (t, b) as in
+// returns_lossgrad_kernel, the same return recurrence started from max_a Q(s_T; theta^-), then the
+// async-Q gradient of the acted action.
+__global__ void nstep_q_lossgrad_kernel(const float* __restrict__ rewards,
+                                        const uint8_t* __restrict__ terminals,
+                                        const int32_t* __restrict__ actions, const float* __restrict__ q,
+                                        const float* __restrict__ q_boot, float* __restrict__ returns,
+                                        float* __restrict__ dq, float* __restrict__ loss_sums, int T, int B,
+                                        int A, float gamma, float rmin, float rmax, float grad_scale) {
+  const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  float s_loss = 0.f, s_q = 0.f;
+  pdl_wait();
+  if (n < (int64_t)T * B) {
+    const int t = (int)(n / B), b = (int)(n - (int64_t)t * B);
+    const float R = nstep_return(rewards, terminals, q_row_max(q_boot + (size_t)b * A, A), t, T, B, b, gamma,
+                                 rmin, rmax);
+    returns[n] = R;
+    const int a = actions[n];
+    const float qa = q[n * A + a];
+    const float delta = R - qa;
+    acted_dq_row(dq + n * A, A, a, delta, grad_scale);
+    s_loss = delta * delta;
+    s_q = qa;
+  }
+  add_q_loss_sums(loss_sums, s_loss, s_q);
 }
 
 // ------------------------------- heads backward -------------------------------------------
@@ -472,41 +517,28 @@ using namespace arl;
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 namespace arl {
-int heads_forward_sample(const float* params, int action_size, const float* h, float* logits, float* probs,
-                         float* value, int32_t* actions, int64_t env_id_base, int64_t step,
-                         const int64_t* step_dev, uint64_t seed, int64_t num_samples, cudaStream_t st,
-                         bool after_fc) {
+// heads + softmax + the draw; wait_first = 0 behind the fc256 kernel (fc_heads_forward), 1 stand-alone
+template <class Draw>
+int heads_forward(const float* params, int action_size, const float* h, float* logits, float* probs, float* value,
+                  int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev, uint64_t seed,
+                  int64_t num_samples, int wait_first, Draw draw, cudaStream_t st) {
   const ParamLayout L = param_layout(action_size);
   const size_t smem = (size_t)(action_size + 1) * 256 * sizeof(float);
   const int64_t ctas = (num_samples + kHfThreads / 32 - 1) / (kHfThreads / 32);   // one warp per sample
   // up to 4 CTAs per SM: one env step of 4096 samples is ONE round of warps (two rounds cost a second
   // exposed load latency)
   const int grid = (int)(ctas < 4LL * num_sms() ? ctas : 4LL * num_sms());
-  ARL_CUDA(launch_pdl(heads_fwd_kernel<SampleDraw>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
+  ARL_CUDA(launch_pdl(heads_fwd_kernel<Draw>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
                       params + L.off[T_PB], params + L.off[T_QW], params + L.off[T_QB], h, logits, probs, value,
                       num_samples, action_size, actions, (uint64_t)env_id_base, (uint64_t)step, seed, step_dev,
-                      after_fc ? 0 : 1, SampleDraw{}));
+                      wait_first, draw));
   ARL_LAUNCH_CHECK("heads_fwd_kernel");
   return ARL_OK;
 }
-
-// heads + softmax + the epsilon-greedy draw, launched behind the fc256 kernel (arl_forward_egreedy)
-int heads_forward_egreedy(const float* params, int action_size, const float* h, float* logits, float* probs,
-                          float* value, int32_t* actions, int64_t env_id_base, int64_t step,
-                          const int64_t* step_dev, uint64_t seed, float ep, double ep_start, double ep_end,
-                          double ep_end_t, double learn_start, int64_t num_samples, cudaStream_t st) {
-  const ParamLayout L = param_layout(action_size);
-  const size_t smem = (size_t)(action_size + 1) * 256 * sizeof(float);
-  const int64_t ctas = (num_samples + kHfThreads / 32 - 1) / (kHfThreads / 32);
-  const int grid = (int)(ctas < 4LL * num_sms() ? ctas : 4LL * num_sms());
-  const EgreedyDraw draw = {ep, ep_start, ep_end, ep_end_t, learn_start};
-  ARL_CUDA(launch_pdl(heads_fwd_kernel<EgreedyDraw>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
-                      params + L.off[T_PB], params + L.off[T_QW], params + L.off[T_QB], h, logits, probs, value,
-                      num_samples, action_size, actions, (uint64_t)env_id_base, (uint64_t)step, seed, step_dev,
-                      0, draw));
-  ARL_LAUNCH_CHECK("heads_fwd_kernel");
-  return ARL_OK;
-}
+template int heads_forward(const float*, int, const float*, float*, float*, float*, int32_t*, int64_t, int64_t,
+                           const int64_t*, uint64_t, int64_t, int, SampleDraw, cudaStream_t);
+template int heads_forward(const float*, int, const float*, float*, float*, float*, int32_t*, int64_t, int64_t,
+                           const int64_t*, uint64_t, int64_t, int, EgreedyDraw, cudaStream_t);
 }  // namespace arl
 
 extern "C" int arl_heads_forward(const float* params, int action_size, const float* h,
@@ -518,8 +550,8 @@ extern "C" int arl_heads_forward(const float* params, int action_size, const flo
   ARL_REQUIRE(num_samples >= 0, "arl_heads_forward: negative size");
   ARL_REQUIRE(aligned16(h), "arl_heads_forward: h must be 16-byte aligned");
   if (num_samples == 0) return ARL_OK;
-  return heads_forward_sample(params, action_size, h, logits, probs, value, nullptr, 0, 0, nullptr, 0,
-                              num_samples, (cudaStream_t)stream, /*after_fc=*/false);
+  return heads_forward(params, action_size, h, logits, probs, value, nullptr, 0, 0, nullptr, 0, num_samples,
+                       /*wait_first=*/1, SampleDraw{}, (cudaStream_t)stream);
 }
 
 extern "C" int arl_sample_actions(const float* probs, int32_t* actions, int num_envs,
@@ -623,6 +655,24 @@ extern "C" int arl_returns_lossgrad(const float* rewards, const uint8_t* termina
                       dvalue, loss_sums, t_max, num_envs, action_size, gamma, beta, reward_min, reward_max,
                       grad_scale));
   ARL_LAUNCH_CHECK("returns_lossgrad_kernel");
+  return ARL_OK;
+}
+
+extern "C" int arl_nstep_q_lossgrad(const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                                    const float* q, const float* q_boot, float* returns, float* dq,
+                                    float* loss_sums, int t_max, int num_envs, int action_size, float gamma,
+                                    float reward_min, float reward_max, float grad_scale, void* stream) {
+  ARL_REQUIRE(rewards && terminals && actions && q && q_boot && returns && dq,
+              "arl_nstep_q_lossgrad: null pointer");
+  ARL_REQUIRE(t_max >= 0 && num_envs >= 0, "arl_nstep_q_lossgrad: negative size");
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_nstep_q_lossgrad: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
+  if (t_max == 0 || num_envs == 0) return ARL_OK;
+  const int64_t total = (int64_t)t_max * num_envs;
+  ARL_CUDA(launch_pdl(nstep_q_lossgrad_kernel, dim3((unsigned)((total + 127) / 128)), dim3(128), 0,
+                      (cudaStream_t)stream, rewards, terminals, actions, q, q_boot, returns, dq, loss_sums, t_max,
+                      num_envs, action_size, gamma, reward_min, reward_max, grad_scale));
+  ARL_LAUNCH_CHECK("nstep_q_lossgrad_kernel");
   return ARL_OK;
 }
 

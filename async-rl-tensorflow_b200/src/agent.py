@@ -405,48 +405,41 @@ class Agent(BaseModel):
             self.update_target_q_network()                       # agent.py:166-167
             self._last_target_sync = self.T
 
+    def _gradients(self, refresh=None, target_refresh=None):
+        """The learner's gradient of the rollout (agent.py:169-207) with its scale, summed over the
+        ranks when the exchange is the torch all-reduce.  ``refresh`` / ``target_refresh``: rebuild the
+        prepared weight images first (None = decide from the parameter versions)."""
+        net, hist = self.network, self.history
+        in_lib = self.world_size > 1 and self.collective == 'library'      # the one exchange per cycle
+        # a3c and nstep_q: sum over t, mean over (global) envs (nstep_q takes the A3C reduction: the
+        # paper accumulates over the rollout); async_q: agent.py:312-314's mean over the worker's batch
+        steps = self.t_max if self.loss_mode == 'async_q' else 1
+        scale = 1.0 / (steps * self.global_envs) if self.reduce_mean else 1.0 / steps
+        if self.loss_mode == 'async_q':
+            net.compute_q_gradients(hist, self.batch_reward, self.batch_terminal, scale, allreduce=in_lib)
+        elif self.loss_mode == 'nstep_q':
+            net.compute_nstep_q_gradients(hist, self.batch_reward, self.batch_terminal, scale, allreduce=in_lib,
+                                          target_refresh=target_refresh, refresh=refresh)
+        else:
+            v_boot = net.bootstrap_value(hist, refresh=refresh)          # R = V(s_T), masked if terminal
+            net.compute_gradients(hist, self.batch_reward, self.batch_terminal, v_boot, grad_scale=scale,
+                                  allreduce=in_lib, refresh=False)
+        if self.world_size > 1 and self.collective == 'torch':
+            dist.all_reduce(net.grads, op=dist.ReduceOp.SUM)
+
     def _update_launches(self, refresh, target_refresh=False):
         """Device work of ``batch_update`` in a3c / nstep_q mode with the learning rate taken from
         the device step counter (already advanced past the last frame of the rollout: offset -t_max
         gives the step of the rollout's first frame, SURVEY §8 step 9)."""
-        net = self.network
-        in_lib = self.world_size > 1 and self.collective == 'library'
-        scale = 1.0 / self.global_envs if self.reduce_mean else 1.0
-        if self.loss_mode == 'nstep_q':
-            net.compute_nstep_q_gradients(self.history, self.batch_reward, self.batch_terminal, scale,
-                                          allreduce=in_lib, target_refresh=target_refresh, refresh=refresh)
-        else:
-            v_boot = net.bootstrap_value(self.history, refresh=refresh)
-            net.compute_gradients(self.history, self.batch_reward, self.batch_terminal, v_boot,
-                                  grad_scale=scale, allreduce=in_lib, refresh=False)
-        if self.world_size > 1 and self.collective == 'torch':
-            dist.all_reduce(net.grads, op=dist.ReduceOp.SUM)
-        net.apply_gradients_sched(self.step_dev, -self.t_max, self.learning_rate, self.max_step,
-                                  count_write=False,
-                                  exchange=self.world_size > 1 and self.collective == 'p2p')
+        self._gradients(refresh, target_refresh)
+        self.network.apply_gradients_sched(self.step_dev, -self.t_max, self.learning_rate, self.max_step,
+                                           count_write=False,
+                                           exchange=self.world_size > 1 and self.collective == 'p2p')
 
     # -- agent.py:169-207 -------------------------------------------------------------------
     def batch_update(self, is_chief=False):
-        net = self.network
-        in_lib = self.world_size > 1 and self.collective == 'library'
-        if self.loss_mode == 'async_q':
-            # agent.py:312-314 mean over the worker's batch; mean over (global) envs as in a3c mode
-            scale = 1.0 / (self.t_max * self.global_envs) if self.reduce_mean else 1.0 / self.t_max
-            net.compute_q_gradients(self.history, self.batch_reward, self.batch_terminal, scale,
-                                    allreduce=in_lib)
-        elif self.loss_mode == 'nstep_q':
-            # sum over t, mean over (global) envs: the A3C reduction (the paper accumulates over the rollout)
-            scale = 1.0 / self.global_envs if self.reduce_mean else 1.0
-            net.compute_nstep_q_gradients(self.history, self.batch_reward, self.batch_terminal, scale,
-                                          allreduce=in_lib)
-        else:
-            v_boot = net.bootstrap_value(self.history)           # R = V(s_T), masked if terminal
-            scale = 1.0 / self.global_envs if self.reduce_mean else 1.0
-            net.compute_gradients(self.history, self.batch_reward, self.batch_terminal, v_boot,
-                                  grad_scale=scale, allreduce=in_lib)   # the one exchange per cycle
-        if self.world_size > 1 and self.collective == 'torch':
-            dist.all_reduce(net.grads, op=dist.ReduceOp.SUM)
-        net.apply_gradients(self.lr, exchange=self.world_size > 1 and self.collective == 'p2p')
+        self._gradients()
+        self.network.apply_gradients(self.lr, exchange=self.world_size > 1 and self.collective == 'p2p')
         self.update_count += 1
         self.t = 0
 

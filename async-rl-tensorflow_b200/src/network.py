@@ -199,12 +199,16 @@ class Network(object):
         self._fc_w_key = key
         return stale
 
+    def _refresh(self, refresh):
+        """A ``refresh`` argument as the C-ABI's int, None decided from the parameter version."""
+        return (1 if self._fc_w_stale() else 0) if refresh is None else int(bool(refresh))
+
     def _forward_into(self, history, l1, l2, l4, logits, probs, value, refresh=None):
         """``refresh``: rebuild the prepared weight images first; None = decide here from the
         parameter version (host state).  A captured region passes the decision in."""
         P, st = _cabi.ptr, _cabi.stream_ptr()
         B, A = self.num_envs, self.action_size
-        refresh = (1 if self._fc_w_stale() else 0) if refresh is None else int(bool(refresh))
+        refresh = self._refresh(refresh)
         if self.timed is None:
             _cabi.call("arl_forward", P(self.params), P(self.fc_w), refresh, A, P(history.ring), B,
                        history.ring_slots, history.first_slot(0), 1, P(l1), P(l2), P(l4),
@@ -246,7 +250,7 @@ class Network(object):
         r = self._rows(t)
         P, st = _cabi.ptr, _cabi.stream_ptr()
         B, A = self.num_envs, self.action_size
-        refresh = (1 if self._fc_w_stale() else 0) if refresh is None else int(bool(refresh))
+        refresh = self._refresh(refresh)
         sd = P(step_dev) if step_dev is not None else None
         if self.timed is None:
             _cabi.call("arl_forward_sample", P(self.params), P(self.fc_w), refresh, A, P(history.ring), B,
@@ -370,8 +374,16 @@ class Network(object):
                          _cabi.ptr(v_boot), _cabi.ptr(self.R), _cabi.ptr(self.d_logits),
                          _cabi.ptr(self.d_value), _cabi.ptr(self.loss_sums), T, B, A, self.gamma,
                          self.beta, self.min_reward, self.max_reward, float(grad_scale), st)
-        P = _cabi.ptr
-        if self._fc_w_stale() if refresh is None else refresh:   # (a forward normally did this already)
+        return self._backward(history, grad_scale, allreduce, refresh)
+
+    def _backward(self, history, grad_scale, allreduce, refresh):
+        """The backward (agent.py:317) of every learner from d_logits / d_value over the T*B samples
+        of the rollout, after rebuilding fc_w when ``refresh`` (None = decide from the parameter
+        version; a forward normally did this already).  Under ``timed`` it runs as its per-layer
+        entries."""
+        T, B, A = self.t_max, self.num_envs, self.action_size
+        P, st = _cabi.ptr, _cabi.stream_ptr()
+        if self._refresh(refresh):
             _cabi.call("arl_prepare_weights", P(self.params), P(self.fc_w), st)
         S = self.tensor_scale = self.pick_tensor_scale(grad_scale)
         if self.timed is None:
@@ -448,14 +460,7 @@ class Network(object):
                    P(self.loss_sums), T * B, A, self.gamma, self.min_reward, self.max_reward,
                    float(grad_scale), st)
         self.d_value.zero_()                                   # the value head is unused
-        if self._fc_w_stale():
-            _cabi.call("arl_prepare_weights", P(self.params), P(self.fc_w), st)
-        S = self.tensor_scale = self.pick_tensor_scale(grad_scale)
-        _cabi.call("arl_backward", P(self.params), P(self.fc_w), A, P(history.ring), B,
-                   history.ring_slots, history.first_slot(T), T, P(self.l1), P(self.l2), P(self.l4),
-                   P(self.d_logits), P(self.d_value), P(self.d_l4), P(self.d_l2),
-                   P(self.d_l1), P(self.grads), P(self.workspace), S, 1 if allreduce else 0, st)
-        return self.grads
+        return self._backward(history, grad_scale, allreduce, None)
 
     # -- n-step Q mode (Mnih et al. 2016, asynchronous n-step Q-learning): the Q head is the p_w/p_b
     # slot as in async_q; the cycle is the A3C cycle with the bootstrap taken from the target network
@@ -476,7 +481,7 @@ class Network(object):
         without it the step is ``step`` and epsilon is ``ep``."""
         r = self._rows(t)
         P, st = _cabi.ptr, _cabi.stream_ptr()
-        refresh = (1 if self._fc_w_stale() else 0) if refresh is None else int(bool(refresh))
+        refresh = self._refresh(refresh)
         if step_dev is not None and ep_sched is None:
             raise ValueError("forward_egreedy: step_dev needs ep_sched = (ep_start, ep_end, ep_end_t, learn_start)")
         e0, e1, et, ls = (float(x) for x in (ep_sched if ep_sched is not None else (0.0, 0.0, 1.0, 0.0)))
@@ -507,14 +512,7 @@ class Network(object):
                          P(self.policy_logits), P(self.q_boot), P(self.R), P(self.d_logits), P(self.loss_sums),
                          T, B, A, self.gamma, self.min_reward, self.max_reward, float(grad_scale), st)
         self.d_value.zero_()                                   # the value head is unused
-        if self._fc_w_stale() if refresh is None else refresh:   # (a forward normally did this already)
-            _cabi.call("arl_prepare_weights", P(self.params), P(self.fc_w), st)
-        S = self.tensor_scale = self.pick_tensor_scale(grad_scale)
-        self._timed_call("arl_backward", P(self.params), P(self.fc_w), A, P(history.ring), B,
-                         history.ring_slots, history.first_slot(T), T, P(self.l1), P(self.l2), P(self.l4),
-                         P(self.d_logits), P(self.d_value), P(self.d_l4), P(self.d_l2),
-                         P(self.d_l1), P(self.grads), P(self.workspace), S, 1 if allreduce else 0, st)
-        return self.grads
+        return self._backward(history, grad_scale, allreduce, refresh)
 
     @property
     def q(self):                                               # agent.py:252

@@ -17,11 +17,12 @@ def header_symbols():
 
 def test_header_declares_the_expected_surface():
     syms = header_symbols()
-    assert len(syms) == 57, syms
+    assert len(syms) == 59, syms
     for must in ("arl_preprocess_push", "arl_forward", "arl_backward", "arl_sample_actions",
                  "arl_returns_lossgrad", "arl_clip_rmsprop", "arl_param_layout", "arl_last_error",
                  "arl_comm_init", "arl_allreduce_grads"):      # SURVEY §8b minimum export set
         assert must in syms
+    assert "arl_forward_egreedy" in syms and "arl_nstep_q_lossgrad" in syms    # n-step Q: one header
 
 
 def test_library_exports_every_declared_symbol(pkg):

@@ -1,17 +1,9 @@
 """CPU: the n-step Q reference against the reference's executed 1-step formula and an explicit
-discounted sum, and the C-ABI surface of include/asyncrl_b200_nstep_q.h (ctypes table == header,
-every declared symbol exported)."""
-import ctypes
-import os
-import re
-
+discounted sum."""
 import numpy as np
 
 from oracle import a3c
 from nstep_q_oracle import nstep_q_gradients
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HEADER = os.path.join(ROOT, "include", "asyncrl_b200_nstep_q.h")
 
 
 def _inputs(T, B, A, seed):
@@ -61,41 +53,3 @@ def test_returns_are_the_masked_discounted_sum():
         ref[t] += disc * boot
     assert np.abs(aux["R"] - ref).max() <= 1e-12
     assert np.abs(aux["delta"] - (ref.reshape(-1) - aux["q"][np.arange(T * B), acts.reshape(-1)])).max() <= 1e-12
-
-
-def _decls():
-    src = re.sub(r"/\*.*?\*/", "", open(HEADER).read(), flags=re.S)
-    return dict((m.group(1), m.group(2)) for m in
-                re.finditer(r"ARL_API\s+int\s+(arl_\w+)\s*\(([^;]*?)\)\s*;", src, re.S))
-
-
-def test_ctypes_prototypes_match_the_companion_header(pkg):
-    """The check of test_ctypes_prototypes_match_the_header for the second table."""
-    decls = _decls()
-    table = pkg._cabi.NSTEP_Q_SIGNATURES
-    assert sorted(decls) == sorted(table) == ["arl_forward_egreedy", "arl_nstep_q_lossgrad"]
-    assert not set(table) & set(pkg._cabi.EXPORTS)                    # kept out of the main table
-    kind = {ctypes.c_void_p: "ptr", ctypes.c_int: "int", ctypes.c_int64: "i64",
-            ctypes.c_uint64: "u64", ctypes.c_float: "f32", ctypes.c_double: "f64"}
-
-    def ckind(param):
-        p = " ".join(param.split())
-        if "*" in p:
-            return "ptr"
-        for prefix, k in (("float", "f32"), ("double", "f64"), ("int64_t", "i64"), ("uint64_t", "u64")):
-            if p.startswith(prefix):
-                return k
-        assert p.startswith("int "), p
-        return "int"
-
-    for name, argtypes in table.items():
-        params = [p for p in decls[name].split(",") if p.strip() and p.strip() != "void"]
-        got = ["ptr" if isinstance(a, type) and issubclass(a, ctypes._Pointer) else kind[a] for a in argtypes]
-        assert got == [ckind(p) for p in params], (name, got, params)
-
-
-def test_library_exports_the_companion_header(pkg):
-    lib = pkg._cabi.load()
-    for name in _decls():
-        fn = getattr(lib, name)
-        assert fn.argtypes == pkg._cabi.NSTEP_Q_SIGNATURES[name]       # bound by load()
