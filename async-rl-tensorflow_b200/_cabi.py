@@ -1,4 +1,4 @@
-"""ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h).
+"""ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h, include/asyncrl_b200_sarsa.h).
 
 The product path has no CPU fallback: if the shared library is missing or a call
 fails, this module raises.  PyTorch is only the carrier of device memory and
@@ -94,6 +94,12 @@ OTHER = {
 }
 EXPORTS = tuple(SIGNATURES) + tuple(OTHER)
 
+# the one-step Sarsa entry: its own header (include/asyncrl_b200_sarsa.h), its own table
+SARSA_SIGNATURES = {
+    "arl_sarsa_lossgrad": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_f32, c_f32,
+                           c_f32, c_f32, c_vp],
+}
+
 
 class ArlError(RuntimeError):
     pass
@@ -112,7 +118,7 @@ def load():
         raise ArlError("%s is missing: build it with async-rl-tensorflow_b200/csrc/build.sh "
                        "(or __graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = ctypes.CDLL(LIB_PATH)
-    for name, argtypes in SIGNATURES.items():
+    for name, argtypes in list(SIGNATURES.items()) + list(SARSA_SIGNATURES.items()):
         fn = getattr(lib, name)
         fn.argtypes, fn.restype = argtypes, c_int
     for name, (argtypes, restype) in OTHER.items():

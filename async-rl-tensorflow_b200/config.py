@@ -45,8 +45,9 @@ class AgentConfig(object):
     clip_norm = 40.0                     # agent.py:319
     resize = 'cv2'                       # environment.py:5-12 executed branch
     loss_mode = 'a3c'                    # 'a3c' (network.py heads/loss) | 'async_q' (agent.py as run) |
-                                         # 'nstep_q' (the paper's asynchronous n-step Q-learning)
-    cuda_graphs = True                   # capture predict / observe(+update) as CUDA graphs (a3c, nstep_q)
+                                         # 'nstep_q' (the paper's asynchronous n-step Q-learning) |
+                                         # 'sarsa' (the paper's asynchronous one-step Sarsa)
+    cuda_graphs = True                   # capture predict / observe(+update) as CUDA graphs (a3c, nstep_q, sarsa)
     max_graphs = 1024                    # cap of the graph cache; beyond it the loop runs eagerly
     DQN_type = 'nips'                    # network.py:30-55 trunk: 'nips' (agent.py:226-252) | 'nature'
     collective = 'auto'                  # gradient exchange: 'p2p' (NVLink peer memory, fused into the update) |

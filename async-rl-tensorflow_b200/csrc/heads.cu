@@ -8,6 +8,7 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "../../include/asyncrl_b200_sarsa.h"
 
 namespace arl {
 
@@ -365,6 +366,34 @@ __global__ void nstep_q_lossgrad_kernel(const float* __restrict__ rewards,
   add_q_loss_sums(loss_sums, s_loss, s_q);
 }
 
+// ------------------------------- one-step Sarsa loss gradients ----------------------------
+// Asynchronous one-step Sarsa (Mnih et al. 2016): q_lossgrad_kernel's target expression with
+// Q(s', a'; theta^-) of the action a' taken in s' in place of max_a.  actions holds a_0 .. a_T, so
+// the next action of sample n is actions[n + B] for every t, the last step included.
+__global__ void sarsa_lossgrad_kernel(const float* __restrict__ rewards,
+                                      const uint8_t* __restrict__ terminals,
+                                      const int32_t* __restrict__ actions, const float* __restrict__ q,
+                                      const float* __restrict__ q_next, float* __restrict__ target,
+                                      float* __restrict__ dq, float* __restrict__ loss_sums, int T, int B,
+                                      int A, float gamma, float rmin, float rmax, float grad_scale) {
+  const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  float s_loss = 0.f, s_q = 0.f;
+  pdl_wait();
+  if (n < (int64_t)T * B) {
+    const float qn = q_next[n * A + actions[n + B]];
+    const float r = fminf(fmaxf(rewards[n], rmin), rmax);                 // agent.py:154
+    const float tgt = fmaf((1.0f - (terminals[n] ? 1.0f : 0.0f)) * gamma, qn, r);      // agent.py:190
+    const int a = actions[n];
+    const float qa = q[n * A + a];
+    const float delta = tgt - qa;
+    target[n] = tgt;
+    acted_dq_row(dq + n * A, A, a, delta, grad_scale);
+    s_loss = delta * delta;
+    s_q = qa;
+  }
+  add_q_loss_sums(loss_sums, s_loss, s_q);
+}
+
 // ------------------------------- heads backward -------------------------------------------
 // CTA = 256 threads (thread k owns hidden unit k).  Per sample: d_h[n][k] = (h>0) * sum_j
 // dz[n][j]*Wcat[k][j];  dWcat[k][j] += h[n][k]*dz[n][j];  dbcat[j] += dz[n][j].
@@ -673,6 +702,24 @@ extern "C" int arl_nstep_q_lossgrad(const float* rewards, const uint8_t* termina
                       (cudaStream_t)stream, rewards, terminals, actions, q, q_boot, returns, dq, loss_sums, t_max,
                       num_envs, action_size, gamma, reward_min, reward_max, grad_scale));
   ARL_LAUNCH_CHECK("nstep_q_lossgrad_kernel");
+  return ARL_OK;
+}
+
+extern "C" int arl_sarsa_lossgrad(const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                                  const float* q, const float* q_next, float* target, float* dq,
+                                  float* loss_sums, int t_max, int num_envs, int action_size, float gamma,
+                                  float reward_min, float reward_max, float grad_scale, void* stream) {
+  ARL_REQUIRE(rewards && terminals && actions && q && q_next && target && dq,
+              "arl_sarsa_lossgrad: null pointer");
+  ARL_REQUIRE(t_max >= 0 && num_envs >= 0, "arl_sarsa_lossgrad: negative size");
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_sarsa_lossgrad: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
+  if (t_max == 0 || num_envs == 0) return ARL_OK;
+  const int64_t total = (int64_t)t_max * num_envs;
+  ARL_CUDA(launch_pdl(sarsa_lossgrad_kernel, dim3((unsigned)((total + 127) / 128)), dim3(128), 0,
+                      (cudaStream_t)stream, rewards, terminals, actions, q, q_next, target, dq, loss_sums, t_max,
+                      num_envs, action_size, gamma, reward_min, reward_max, grad_scale));
+  ARL_LAUNCH_CHECK("sarsa_lossgrad_kernel");
   return ARL_OK;
 }
 

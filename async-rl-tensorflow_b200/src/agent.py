@@ -71,7 +71,6 @@ class Agent(BaseModel):
         T, B = self.t_max, self.num_envs
         self.batch_reward = torch.zeros(T, B, device=self.device)
         self.batch_terminal = torch.zeros(T, B, dtype=torch.uint8, device=self.device)
-        self.batch_action = self.network.sampled_action.view(T, B)
         self.t = 0                                               # position inside the rollout
         self.step = 0
         self.T = 0
@@ -81,19 +80,25 @@ class Agent(BaseModel):
         # loss_mode 'nstep_q' = the paper's asynchronous n-step Q-learning: the same Q head,
         # epsilon-greedy schedule and target network, n-step returns bootstrapped from
         # max_a Q(s_T; theta^-) -- the A3C cycle with another loss kernel, on the graph-replayed path
+        # loss_mode 'sarsa' = the paper's asynchronous one-step Sarsa: async_q's 1-step targets with
+        # Q(s', a'; theta^-) of the action a' actually taken in s'; on the graph-replayed path too
         self.loss_mode = getattr(config, 'loss_mode', 'a3c')
-        if self.loss_mode not in ('a3c', 'async_q', 'nstep_q'):
-            raise ValueError("loss_mode must be 'a3c', 'async_q' or 'nstep_q', got %r" % (self.loss_mode,))
-        self.has_target = self.loss_mode in ('async_q', 'nstep_q')
+        if self.loss_mode not in ('a3c', 'async_q', 'nstep_q', 'sarsa'):
+            raise ValueError("loss_mode must be 'a3c', 'async_q', 'nstep_q' or 'sarsa', got %r" % (self.loss_mode,))
+        self.has_target = self.loss_mode in ('async_q', 'nstep_q', 'sarsa')
         if self.has_target:
-            self.network.make_target(one_step=self.loss_mode == 'async_q')
+            self.network.make_target(one_step=self.loss_mode != 'nstep_q', next_actions=self.loss_mode == 'sarsa')
             self._last_target_sync = 0
+        # sarsa: the update drew a_T, the action the next rollout's step 0 takes (row T of
+        # network.sarsa_actions); False before the first update and after before_train
+        self.sarsa_pending = False
+        self.batch_action = self.network.sampled_action.view(T, B)
         # CUDA graphs of the loop (SURVEY a16): the device work of ``predict`` and of ``observe``
         # (+ the learner step at the end of a rollout) is captured once per distinct set of launch
         # arguments -- rollout slot, ring position, frame / reward buffers -- and replayed from then
         # on.  The two host values that change on every step, the Philox step and the step the
         # learning rate is annealed on, are read from ``step_dev`` (device memory) instead.
-        self.cuda_graphs = bool(getattr(config, 'cuda_graphs', True)) and self.loss_mode in ('a3c', 'nstep_q')
+        self.cuda_graphs = bool(getattr(config, 'cuda_graphs', True)) and self.loss_mode in ('a3c', 'nstep_q', 'sarsa')
         self.max_graphs = int(getattr(config, 'max_graphs', 1024))
         self.graph_warmup_updates = 2                            # eager cycles first (lazy init, autotune)
         self.step_dev = torch.zeros(1, dtype=torch.int64, device=self.device)
@@ -114,6 +119,7 @@ class Agent(BaseModel):
         self.update_target_q_network()                           # main.py:92
         if self.has_target:
             self._last_target_sync = self.T
+        self.sarsa_pending = False                               # the first step draws its action
         return self.env.frames, 0, 0, self.env.terminal, range(self.step, self.max_step)
 
     # -- agent.py:52-67 ---------------------------------------------------------------------
@@ -168,7 +174,7 @@ class Agent(BaseModel):
                 self.env.new_random_game(mask=terminal)
             if self.update_count != before:                      # agent.py:199-201
                 sums = self.network.loss_sums
-                if self.has_target:                              # async_q, nstep_q: {sum delta^2, sum Q}
+                if self.has_target:                              # async_q, nstep_q, sarsa: {sum delta^2, sum Q}
                     n = float(self.t_max * B)
                     acc['loss'] += sums[0] / n
                     acc['q'] += sums[1] / n
@@ -228,6 +234,12 @@ class Agent(BaseModel):
         elif self.loss_mode == 'nstep_q':                         # + where the sync schedule stands
             torch.save({"target": self.network.target_params.cpu(), "last_target_sync": self._last_target_sync},
                        os.path.join(d, "target-%d.pt" % self.step_op))
+        elif self.loss_mode == 'sarsa':                           # + the action a_T the next step takes
+            net = self.network
+            torch.save({"target": net.target_params.cpu(), "last_target_sync": self._last_target_sync,
+                        "pending_action": net.sarsa_actions[net.t_max * net.num_envs:].cpu(),
+                        "pending": self.sarsa_pending},
+                       os.path.join(d, "target-%d.pt" % self.step_op))
         return path
 
     def load_checkpoint(self, checkpoint_dir=None):
@@ -240,8 +252,12 @@ class Agent(BaseModel):
             p = os.path.join(d, "target-%d.pt" % self.step_op)
             if os.path.exists(p):
                 saved = torch.load(p)
-                if isinstance(saved, dict):                      # nstep_q
+                if isinstance(saved, dict):                      # nstep_q, sarsa
                     self._last_target_sync = int(saved["last_target_sync"])
+                    if "pending" in saved:                       # sarsa
+                        net = self.network
+                        net.sarsa_actions[net.t_max * net.num_envs:].copy_(saved["pending_action"].to(self.device))
+                        self.sarsa_pending = bool(saved["pending"])
                     saved = saved["target"]
                 self.network.target_params.copy_(saved.to(self.device))
             else:
@@ -292,21 +308,31 @@ class Agent(BaseModel):
             net.forward(self.history, t)
             ep = self.ep if test_ep is None else test_ep
             return net.egreedy(t, self.step, self.seed, ep, self.env_id_base)
-        if self.loss_mode == 'nstep_q' and test_ep is not None:   # a fixed epsilon: eager
+        if self.loss_mode in ('nstep_q', 'sarsa') and test_ep is not None:   # a fixed epsilon: eager
             return net.forward_egreedy(self.history, t, self.seed, self.env_id_base, step=self.step, ep=test_ep)
         self._sync_step_dev()
         refresh = net._fc_w_stale()
+        # sarsa: step 0 after an update takes the action a_T that update drew (Mnih et al. 2016:
+        # choose a', accumulate, update, take a'); the forward still runs, its activations are s_0's
+        take_pending = self.loss_mode == 'sarsa' and t == 0 and self.sarsa_pending
 
         def launches():                                        # forward + heads + Philox draw
-            if self.loss_mode == 'nstep_q':                    # agent.py:142-149, epsilon from step_dev
+            if take_pending:
+                r = net._rows(0)
+                net.forward(self.history, 0, refresh=refresh)
+                net.sampled_action[r].copy_(net.sarsa_actions[self.t_max * self.num_envs:])   # cudaMemcpyAsync
+            elif self.loss_mode in ('nstep_q', 'sarsa'):       # agent.py:142-149, epsilon from step_dev
                 net.forward_egreedy(self.history, t, self.seed, self.env_id_base, step_dev=self.step_dev,
-                                    ep_sched=(self.ep_start, self.ep_end, self.ep_end_t, self.learn_start),
-                                    refresh=refresh)
+                                    ep_sched=self._ep_sched(), refresh=refresh)
             else:
                 net.forward_sample(self.history, t, 0, self.seed, self.env_id_base, step_dev=self.step_dev,
                                    refresh=refresh)
-        self._run(('predict', t, self.history.head, refresh), launches)
+        self._run(('predict', t, self.history.head, refresh, take_pending), launches)
         return net.sampled_action[net._rows(t)]
+
+    def _ep_sched(self):
+        """agent.py:142-144's constants, for the epsilon the kernels evaluate from ``step_dev``."""
+        return (self.ep_start, self.ep_end, self.ep_end_t, self.learn_start)
 
     # -- agent.py:351-391 -------------------------------------------------------------------
     def play(self, sv=None, is_chief=True, n_step=10000, n_episode=100, test_ep=None, render=False):
@@ -314,8 +340,8 @@ class Agent(BaseModel):
         History seeded with 4 copies of the first screen (agent.py:365-366), then predict / act
         (is_training=False: no life-loss terminal) / add until every env has finished its episode
         or ``n_step`` steps have passed.  Action selection: epsilon-greedy with ``test_ep``
-        (default ep_end, agent.py:352-353) in async_q / nstep_q mode, a sample from the policy in
-        a3c mode.
+        (default ep_end, agent.py:352-353) in async_q / nstep_q / sarsa mode, a sample from the policy
+        in a3c mode.
         Returns (best_reward, best_idx, per-episode mean reward over the envs); gym's monitor
         (agent.py:357-359) is the emulator's business and not reproduced."""
         if test_ep is None:
@@ -371,8 +397,8 @@ class Agent(BaseModel):
             new_head = (hist.head + 1) % hist.ring_slots
             hist.head = new_head                                 # host state first: the launches read it
             refresh = self.network._fc_w_stale() if will_update else False
-            # nstep_q: rebuild the target's weight image in this update only after a target sync
-            target_refresh = (self.loss_mode == 'nstep_q' and will_update
+            # nstep_q, sarsa: rebuild the target's weight image in this update only after a target sync
+            target_refresh = (self.loss_mode in ('nstep_q', 'sarsa') and will_update
                               and self.network._target_fc_w_stale())
 
             # bench.py: an event pair around K1 -- launched eagerly between its events, or (when the
@@ -399,6 +425,7 @@ class Agent(BaseModel):
             if will_update:
                 self.network._param_writes += 1                  # the update wrote the parameters
                 self.update_count += 1
+                self.sarsa_pending = self.loss_mode == 'sarsa'
                 self.t = 0
         self.T += self.global_envs                               # agent.py:165 counts every worker
         if self.has_target and self.T - self._last_target_sync >= self.target_q_update_step:
@@ -411,8 +438,9 @@ class Agent(BaseModel):
         prepared weight images first (None = decide from the parameter versions)."""
         net, hist = self.network, self.history
         in_lib = self.world_size > 1 and self.collective == 'library'      # the one exchange per cycle
-        # a3c and nstep_q: sum over t, mean over (global) envs (nstep_q takes the A3C reduction: the
-        # paper accumulates over the rollout); async_q: agent.py:312-314's mean over the worker's batch
+        # a3c, nstep_q and sarsa: sum over t, mean over (global) envs (the Q learners take the A3C
+        # reduction: the paper accumulates over the rollout); async_q: agent.py:312-314's mean over the
+        # worker's batch
         steps = self.t_max if self.loss_mode == 'async_q' else 1
         scale = 1.0 / (steps * self.global_envs) if self.reduce_mean else 1.0 / steps
         if self.loss_mode == 'async_q':
@@ -420,6 +448,10 @@ class Agent(BaseModel):
         elif self.loss_mode == 'nstep_q':
             net.compute_nstep_q_gradients(hist, self.batch_reward, self.batch_terminal, scale, allreduce=in_lib,
                                           target_refresh=target_refresh, refresh=refresh)
+        elif self.loss_mode == 'sarsa':                                  # a_T: step and epsilon of step_dev
+            net.compute_sarsa_gradients(hist, self.batch_reward, self.batch_terminal, scale, self.step_dev,
+                                        self.seed, self._ep_sched(), self.env_id_base, allreduce=in_lib,
+                                        target_refresh=target_refresh, refresh=refresh)
         else:
             v_boot = net.bootstrap_value(hist, refresh=refresh)          # R = V(s_T), masked if terminal
             net.compute_gradients(hist, self.batch_reward, self.batch_terminal, v_boot, grad_scale=scale,
@@ -428,7 +460,7 @@ class Agent(BaseModel):
             dist.all_reduce(net.grads, op=dist.ReduceOp.SUM)
 
     def _update_launches(self, refresh, target_refresh=False):
-        """Device work of ``batch_update`` in a3c / nstep_q mode with the learning rate taken from
+        """Device work of ``batch_update`` in a3c / nstep_q / sarsa mode with the learning rate taken from
         the device step counter (already advanced past the last frame of the rollout: offset -t_max
         gives the step of the rollout's first frame, SURVEY §8 step 9)."""
         self._gradients(refresh, target_refresh)
@@ -438,15 +470,21 @@ class Agent(BaseModel):
 
     # -- agent.py:169-207 -------------------------------------------------------------------
     def batch_update(self, is_chief=False):
+        if self.loss_mode == 'sarsa':
+            # a_T is drawn with the step of the next rollout's first frame, as on the replayed path
+            # (observe has advanced step_dev past this rollout's last frame there)
+            self.step_dev.fill_(int(self.step) + 1)
+            self._step_dev_host = self.step + 1
         self._gradients()
         self.network.apply_gradients(self.lr, exchange=self.world_size > 1 and self.collective == 'p2p')
         self.update_count += 1
+        self.sarsa_pending = self.loss_mode == 'sarsa'
         self.t = 0
 
     def update_target_q_network(self):
-        """agent.py:342-344 (async_q / nstep_q mode; the A3C path has no target network).  A host
-        copy outside the captured graphs; in nstep_q mode the next update then rebuilds the
-        target's weight image (Network._target_fc_w_stale)."""
+        """agent.py:342-344 (async_q / nstep_q / sarsa mode; the A3C path has no target network).  A
+        host copy outside the captured graphs; in nstep_q and sarsa mode the next update then rebuilds
+        the target's weight image (Network._target_fc_w_stale)."""
         if self.has_target:
             self.network.update_target()
 

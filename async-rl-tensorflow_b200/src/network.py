@@ -415,10 +415,12 @@ class Network(object):
         return self.grads
 
     # -- async-Q mode (agent.py:169-207, 298-314): the Q head lives in the p_w/p_b slot ---------
-    def make_target(self, one_step=True):
+    def make_target(self, one_step=True, next_actions=False):
         """agent.py:257-296: a second parameter set, the target network.  ``one_step``: also the
-        [T*B] target buffers of the 1-step learner (async_q); the n-step learner (nstep_q) evaluates
-        the target network on the B states s_T only (``q_boot``)."""
+        [T*B] target buffers of the 1-step learners (async_q, sarsa); the n-step learner (nstep_q)
+        evaluates the target network on the B states s_T only (``q_boot``).  ``next_actions``
+        (sarsa): the rollout's actions get one more row, a_T, the action taken in s_T
+        (``sarsa_actions`` [(T+1)*B]; ``sampled_action`` becomes a view of its first T rows)."""
         self.target_params = self.params.clone()
         B, A = self.num_envs, self.action_size
         N = B * self.t_max
@@ -427,6 +429,10 @@ class Network(object):
             self.target_q = torch.empty(N, A, **f32)          # agent.py:186 q_t_plus_1
             self.target_q_t = torch.empty(N, **f32)           # agent.py:190
             self._tq_scratch = (torch.empty(N, A, **f32), torch.empty(N, **f32))
+            if next_actions:
+                self.sarsa_actions = torch.zeros(N + B, dtype=torch.int32, device=self.device)
+                self.sampled_action = self.sarsa_actions[:N]
+                self._target_fc_w_key = None
         else:
             self.q_boot = torch.empty(B, A, **f32)            # Q(s_T; theta^-)
             self._target_fc_w_key = None
@@ -513,6 +519,43 @@ class Network(object):
                          T, B, A, self.gamma, self.min_reward, self.max_reward, float(grad_scale), st)
         self.d_value.zero_()                                   # the value head is unused
         return self._backward(history, grad_scale, allreduce, refresh)
+
+    # -- one-step Sarsa mode (Mnih et al. 2016, asynchronous one-step Sarsa): async_q's Q head,
+    # target forward and 1-step targets, bootstrapped from the action taken in s' instead of max_a
+    def compute_sarsa_gradients(self, history, rewards, terminals, grad_scale, step_dev, seed, ep_sched,
+                                env_id_base=0, allreduce=False, target_refresh=None, refresh=None):
+        """The one-step Sarsa learner's gradient over the rollout:
+          1. target-network forward over s_1..s_T into ``target_q`` (async_q's call; target_fc_w is
+             rebuilt only when ``target_refresh``, None = decide from the target's version);
+          2. the action a_T taken in s_T, drawn now: the epsilon-greedy draw of ``forward_egreedy`` on
+             Q(s_T; theta) under the parameters before this update, with the step and epsilon of the
+             int64 device counter ``step_dev`` (the next rollout's first step), into row T of
+             ``sarsa_actions`` -- the next rollout's step 0 takes it;
+          3. targets y = clip(r) + gamma (1 - term) Q(s', a'; theta^-) and dQ of the acted actions
+             (arl_sarsa_lossgrad);
+          4. the backward (agent.py:317).
+        ``history`` must have had exactly t_max pushes since s_0."""
+        T, B, A = self.t_max, self.num_envs, self.action_size
+        P, st = _cabi.ptr, _cabi.stream_ptr()
+        b = self._b
+        probs, value = self._tq_scratch
+        if target_refresh is None:
+            target_refresh = self._target_fc_w_stale()
+        self._timed_call("arl_forward", P(self.target_params), P(self.target_fc_w), int(bool(target_refresh)), A,
+                         P(history.ring), B, history.ring_slots, history.first_slot(T - 1), T, P(self.d_l1),
+                         P(self.d_l2), P(self.d_l4), P(self.target_q), P(probs), P(value), st)
+        e0, e1, et, ls = (float(x) for x in ep_sched)
+        self._timed_call("arl_forward_egreedy", P(self.params), P(self.fc_w), self._refresh(refresh), A,
+                         P(history.ring), B, history.ring_slots, history.first_slot(0), P(b['l1']), P(b['l2']),
+                         P(b['l4']), P(b['logits']), P(b['probs']), P(b['value']), P(self.sarsa_actions[T * B:]),
+                         int(env_id_base), 0, P(step_dev), int(seed), 0.0, e0, e1, et, ls, st)
+        self.loss_sums.zero_()
+        self._timed_call("arl_sarsa_lossgrad", P(rewards), P(terminals), P(self.sarsa_actions),
+                         P(self.policy_logits), P(self.target_q), P(self.target_q_t), P(self.d_logits),
+                         P(self.loss_sums), T, B, A, self.gamma, self.min_reward, self.max_reward,
+                         float(grad_scale), st)
+        self.d_value.zero_()                                   # the value head is unused
+        return self._backward(history, grad_scale, allreduce, False)   # fc_w: refreshed by step 2
 
     @property
     def q(self):                                               # agent.py:252

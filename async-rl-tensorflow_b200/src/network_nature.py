@@ -188,7 +188,10 @@ class NatureNetwork(Network):
             _cabi.call("arl_allreduce_grads", P(self.grads), int(self.grads.numel()), st)
         return self.grads
 
-    def make_target(self, one_step=True):
+    def make_target(self, one_step=True, next_actions=False):
+        if next_actions:
+            raise NotImplementedError("loss_mode='sarsa' is built on the nips trunk (agent.py:226-252); "
+                                      "the nature trunk is A3C-only")
         raise NotImplementedError("loss_mode='async_q' runs the reference's agent.py net, which is the "
                                   "nips trunk (agent.py:226-252); the nature trunk is A3C-only"
                                   if one_step else

@@ -1,7 +1,8 @@
-"""Cycle time of the three learners on one GPU: a3c and nstep_q replayed from CUDA graphs, async_q
-eager (its own path: host epsilon, a separate draw launch, a target forward over all T*B next states).
+"""Cycle time of the four learners on one GPU: a3c, nstep_q and sarsa replayed from CUDA graphs,
+async_q eager (its own path: host epsilon, a separate draw launch, a target forward over all T*B next
+states; sarsa runs that target forward too, inside its graph).
 
-    python tools/bench_nstep_q.py [--rounds R] [--cycles K] [--out profiles/r03_nstep_q_bench.json]
+    python tools/bench_nstep_q.py [--rounds R] [--cycles K] [--modes a3c,nstep_q,...] [--out FILE]
 
 For each shape (envs x t_max x actions: 4096 x 5 x 6 and 16384 x 20 x 18) one agent per mode is built
 and warmed up until a whole ring period has replayed without a new graph capture; then the modes take
@@ -26,7 +27,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-MODES = ("a3c", "nstep_q", "async_q")
+MODES = ("a3c", "nstep_q", "sarsa", "async_q")
 
 
 def card():
@@ -45,7 +46,7 @@ def main():
     ap.add_argument("--cycles", type=int, default=20, help="cycles per timed block")
     ap.add_argument("--shapes", default="4096x5x6,16384x20x18", help="envs x t_max x actions, comma separated")
     ap.add_argument("--modes", default=",".join(MODES))
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_nstep_q_bench.json"))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r05_sarsa_bench.json"))
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("bench_nstep_q: needs a CUDA device")
