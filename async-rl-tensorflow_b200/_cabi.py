@@ -1,4 +1,5 @@
-"""ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h, include/asyncrl_b200_sarsa.h).
+"""ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h, include/asyncrl_b200_sarsa.h,
+include/asyncrl_b200_dueling.h).
 
 The product path has no CPU fallback: if the shared library is missing or a call
 fails, this module raises.  PyTorch is only the carrier of device memory and
@@ -100,6 +101,19 @@ SARSA_SIGNATURES = {
                            c_f32, c_f32, c_vp],
 }
 
+# the dueling Q heads: their own header (include/asyncrl_b200_dueling.h), their own table
+DUELING_SIGNATURES = {
+    "arl_forward_dueling": [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp,
+                            c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_u64, c_f32, ctypes.c_double, ctypes.c_double,
+                            ctypes.c_double, ctypes.c_double, c_vp],
+    "arl_q_lossgrad_dueling": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_f32, c_f32,
+                               c_f32, c_f32, c_vp],
+    "arl_nstep_q_lossgrad_dueling": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int,
+                                     c_f32, c_f32, c_f32, c_f32, c_vp],
+    "arl_sarsa_lossgrad_dueling": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int,
+                                   c_f32, c_f32, c_f32, c_f32, c_vp],
+}
+
 
 class ArlError(RuntimeError):
     pass
@@ -118,7 +132,7 @@ def load():
         raise ArlError("%s is missing: build it with async-rl-tensorflow_b200/csrc/build.sh "
                        "(or __graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = ctypes.CDLL(LIB_PATH)
-    for name, argtypes in list(SIGNATURES.items()) + list(SARSA_SIGNATURES.items()):
+    for name, argtypes in list(SIGNATURES.items()) + list(SARSA_SIGNATURES.items()) + list(DUELING_SIGNATURES.items()):
         fn = getattr(lib, name)
         fn.argtypes, fn.restype = argtypes, c_int
     for name, (argtypes, restype) in OTHER.items():

@@ -33,7 +33,10 @@ class AgentConfig(object):
     max_delta = 1
 
     double_q = False
-    dueling = False
+    dueling = False                      # dueling Q heads (Wang et al. 2016, "average" aggregator) for the
+                                         # Q learners (async_q, nstep_q, sarsa) on the nips trunk: p_w/p_b is the
+                                         # advantage stream, q_w/q_b the value stream, both on fc256's output
+                                         # (no hidden layer per stream); a3c refuses it
 
     _test_step = 0.5 * scale
 

@@ -4,6 +4,7 @@
 #include <string.h>
 
 #include "common.cuh"
+#include "../../include/asyncrl_b200_dueling.h"
 
 namespace arl {
 
@@ -100,15 +101,15 @@ extern "C" int64_t arl_a2_block_rows(int num_envs) {
 }
 
 namespace arl {
-template <class Draw>
+template <class Draw, bool Dueling>
 int fc_heads_forward(const float* params, const float* prepared, int action_size, const float* a2, float* h,
                      float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base, int64_t step,
                      const int64_t* step_dev, uint64_t seed, int64_t num_samples, Draw draw, void* stream);
 }
 
 // One env step of the forward, env range by env range; `draw` is the action draw of the heads launch
-// (common.cuh: SampleDraw with actions == NULL draws nothing)
-template <class Draw>
+// (common.cuh: SampleDraw with actions == NULL draws nothing), Dueling the head kind (heads.cu)
+template <bool Dueling = false, class Draw>
 static int forward_step(const float* params, float* prepared, int action_size, const uint8_t* ring,
                         int num_envs, int ring_slots, int first_slot, float* a1, float* a2, float* h,
                         float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base,
@@ -125,9 +126,10 @@ static int forward_step(const float* params, float* prepared, int action_size, c
     rc = arl_conv2_forward(prepared, a1c, a2c, n, stream);
     if (rc) return rc;
     // fc256, then heads + softmax (+ the action draw) in one launch
-    rc = fc_heads_forward(params, prepared, action_size, a2c, hc, logits + (size_t)off * action_size,
-                          probs + (size_t)off * action_size, value + off, actions ? actions + off : nullptr,
-                          env_id_base + off, step, step_dev, seed, n, draw, stream);
+    rc = fc_heads_forward<Draw, Dueling>(params, prepared, action_size, a2c, hc, logits + (size_t)off * action_size,
+                                         probs + (size_t)off * action_size, value + off,
+                                         actions ? actions + off : nullptr, env_id_base + off, step, step_dev, seed,
+                                         n, draw, stream);
     if (rc) return rc;
   }
   return ARL_OK;
@@ -165,28 +167,76 @@ extern "C" int arl_forward_sample(const float* params, float* prepared, int refr
                       logits, probs, value, actions, env_id_base, step, step_dev, seed, SampleDraw{}, stream);
 }
 
+// the argument checks of the epsilon-greedy forward (fn = the C entry's name, for errors)
+static int egreedy_args(const char* fn, const float* params, const float* prepared, int action_size,
+                        const uint8_t* ring, const float* a1, const float* a2, const float* h, const float* logits,
+                        const float* probs, const float* value, const int32_t* actions, int num_envs,
+                        int64_t env_id_base, int64_t step, const int64_t* step_dev, float ep, double ep_start,
+                        double ep_end, double ep_end_t) {
+  ARL_REQUIRE(params && prepared && ring && a1 && a2 && h && logits && probs && value && actions,
+              "%s: null pointer", fn);
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "%s: action_size %d outside [1,%d]", fn, action_size, ARL_MAX_ACTIONS);
+  ARL_REQUIRE(num_envs >= 0 && env_id_base >= 0 && step >= 0, "%s: negative argument", fn);
+  ARL_REQUIRE(ep >= 0.f && ep <= 1.f, "%s: ep %f outside [0,1]", fn, (double)ep);
+  ARL_REQUIRE(step_dev == nullptr || (ep_start >= 0.0 && ep_start <= 1.0 && ep_end >= 0.0 && ep_end <= 1.0),
+              "%s: ep_start %f / ep_end %f outside [0,1]", fn, ep_start, ep_end);
+  ARL_REQUIRE(step_dev == nullptr || ep_end_t > 0.0, "%s: ep_end_t must be > 0", fn);
+  return ARL_OK;
+}
+
 extern "C" int arl_forward_egreedy(const float* params, float* prepared, int refresh_prepared, int action_size,
                                    const uint8_t* ring, int num_envs, int ring_slots, int first_slot,
                                    float* a1, float* a2, float* h, float* logits, float* probs, float* value,
                                    int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev,
                                    uint64_t seed, float ep, double ep_start, double ep_end, double ep_end_t,
                                    double learn_start, void* stream) {
-  ARL_REQUIRE(params && prepared && ring && a1 && a2 && h && logits && probs && value && actions,
-              "arl_forward_egreedy: null pointer");
-  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
-              "arl_forward_egreedy: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
-  ARL_REQUIRE(num_envs >= 0 && env_id_base >= 0 && step >= 0, "arl_forward_egreedy: negative argument");
-  ARL_REQUIRE(ep >= 0.f && ep <= 1.f, "arl_forward_egreedy: ep %f outside [0,1]", (double)ep);
-  ARL_REQUIRE(step_dev == nullptr || (ep_start >= 0.0 && ep_start <= 1.0 && ep_end >= 0.0 && ep_end <= 1.0),
-              "arl_forward_egreedy: ep_start %f / ep_end %f outside [0,1]", ep_start, ep_end);
-  ARL_REQUIRE(step_dev == nullptr || ep_end_t > 0.0, "arl_forward_egreedy: ep_end_t must be > 0");
-  if (num_envs == 0) return ARL_OK;
-  int rc = ARL_OK;
+  int rc = egreedy_args("arl_forward_egreedy", params, prepared, action_size, ring, a1, a2, h, logits, probs, value,
+                         actions, num_envs, env_id_base, step, step_dev, ep, ep_start, ep_end, ep_end_t);
+  if (rc || num_envs == 0) return rc;
   if (refresh_prepared) rc = arl_prepare_weights(params, prepared, stream);
   if (rc) return rc;
   return forward_step(params, prepared, action_size, ring, num_envs, ring_slots, first_slot, a1, a2, h,
                       logits, probs, value, actions, env_id_base, step, step_dev, seed,
                       EgreedyDraw{ep, ep_start, ep_end, ep_end_t, learn_start}, stream);
+}
+
+extern "C" int arl_forward_dueling(const float* params, float* prepared, int refresh_prepared, int action_size,
+                                   const uint8_t* ring, int num_envs, int ring_slots, int first_slot, int steps,
+                                   float* a1, float* a2, float* h, float* logits, float* probs, float* value,
+                                   int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev,
+                                   uint64_t seed, float ep, double ep_start, double ep_end, double ep_end_t,
+                                   double learn_start, void* stream) {
+  int rc = ARL_OK;
+  if (actions != nullptr) {                       // one env step + the draw of arl_forward_egreedy
+    ARL_REQUIRE(steps == 1, "arl_forward_dueling: the action draw needs steps == 1, got %d", steps);
+    rc = egreedy_args("arl_forward_dueling", params, prepared, action_size, ring, a1, a2, h, logits, probs, value,
+                      actions, num_envs, env_id_base, step, step_dev, ep, ep_start, ep_end, ep_end_t);
+    if (rc || num_envs == 0) return rc;
+    if (refresh_prepared) rc = arl_prepare_weights(params, prepared, stream);
+    if (rc) return rc;
+    return forward_step<true>(params, prepared, action_size, ring, num_envs, ring_slots, first_slot, a1, a2, h,
+                              logits, probs, value, actions, env_id_base, step, step_dev, seed,
+                              EgreedyDraw{ep, ep_start, ep_end, ep_end_t, learn_start}, stream);
+  }
+  ARL_REQUIRE(params && prepared && ring && a1 && a2 && h && logits && probs && value,
+              "arl_forward_dueling: null pointer");
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_forward_dueling: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
+  ARL_REQUIRE(num_envs >= 0 && steps >= 0, "arl_forward_dueling: negative size");
+  if (num_envs == 0 || steps == 0) return ARL_OK;
+  if (refresh_prepared) rc = arl_prepare_weights(params, prepared, stream);
+  if (rc) return rc;
+  if (steps == 1)                                 // arl_forward's paths, no draw
+    return forward_step<true>(params, prepared, action_size, ring, num_envs, ring_slots, first_slot, a1, a2, h,
+                              logits, probs, value, nullptr, 0, 0, nullptr, 0, SampleDraw{}, stream);
+  const int64_t N = (int64_t)num_envs * steps;
+  rc = arl_conv1_forward(prepared, ring, a1, num_envs, ring_slots, first_slot, steps, stream);
+  if (rc) return rc;
+  rc = arl_conv2_forward(prepared, a1, a2, N, stream);
+  if (rc) return rc;
+  return fc_heads_forward<SampleDraw, true>(params, prepared, action_size, a2, h, logits, probs, value, nullptr, 0,
+                                            0, nullptr, 0, N, SampleDraw{}, stream);
 }
 
 extern "C" int arl_backward(const float* params, const float* prepared, int action_size,

@@ -18,7 +18,7 @@ int reduce_partials(const float* partials, float* out, int num_partials, int n,
                     cudaStream_t stream);
 int reduce_partials_scaled(const float* partials, float* out, int num_partials, int n, float alpha,
                            cudaStream_t stream);
-template <class Draw>
+template <class Draw, bool Dueling>
 int heads_forward(const float* params, int action_size, const float* h, float* logits, float* probs, float* value,
                   int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev, uint64_t seed,
                   int64_t num_samples, int wait_first, Draw draw, cudaStream_t st);
@@ -317,8 +317,9 @@ extern "C" int arl_fc_forward(const float* params, const float* prepared, const 
 }
 
 namespace arl {
-// arl_fc_heads_forward with the action draw `draw` (common.cuh): the forward entries of api.cu end here
-template <class Draw>
+// arl_fc_heads_forward with the action draw `draw` (common.cuh) and the head kind Dueling (heads.cu):
+// the forward entries of api.cu end here
+template <class Draw, bool Dueling>
 int fc_heads_forward(const float* params, const float* prepared, int action_size, const float* a2, float* h,
                      float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base, int64_t step,
                      const int64_t* step_dev, uint64_t seed, int64_t num_samples, Draw draw, void* stream) {
@@ -333,13 +334,21 @@ int fc_heads_forward(const float* params, const float* prepared, int action_size
   int rc = fc_forward_impl(params, prepared, a2, h, num_samples, (cudaStream_t)stream);
   if (rc) return rc;
   // heads + softmax + (optionally) the draw: one warp-per-sample kernel
-  return heads_forward(params, action_size, h, logits, probs, value, actions, env_id_base, step, step_dev, seed,
-                       num_samples, /*wait_first=*/0, draw, (cudaStream_t)stream);
+  return heads_forward<Draw, Dueling>(params, action_size, h, logits, probs, value, actions, env_id_base, step,
+                                      step_dev, seed, num_samples, /*wait_first=*/0, draw, (cudaStream_t)stream);
 }
-template int fc_heads_forward(const float*, const float*, int, const float*, float*, float*, float*, float*,
-                              int32_t*, int64_t, int64_t, const int64_t*, uint64_t, int64_t, SampleDraw, void*);
-template int fc_heads_forward(const float*, const float*, int, const float*, float*, float*, float*, float*,
-                              int32_t*, int64_t, int64_t, const int64_t*, uint64_t, int64_t, EgreedyDraw, void*);
+template int fc_heads_forward<SampleDraw, false>(const float*, const float*, int, const float*, float*, float*,
+                                                 float*, float*, int32_t*, int64_t, int64_t, const int64_t*,
+                                                 uint64_t, int64_t, SampleDraw, void*);
+template int fc_heads_forward<EgreedyDraw, false>(const float*, const float*, int, const float*, float*, float*,
+                                                  float*, float*, int32_t*, int64_t, int64_t, const int64_t*,
+                                                  uint64_t, int64_t, EgreedyDraw, void*);
+template int fc_heads_forward<SampleDraw, true>(const float*, const float*, int, const float*, float*, float*,
+                                                float*, float*, int32_t*, int64_t, int64_t, const int64_t*,
+                                                uint64_t, int64_t, SampleDraw, void*);
+template int fc_heads_forward<EgreedyDraw, true>(const float*, const float*, int, const float*, float*, float*,
+                                                 float*, float*, int32_t*, int64_t, int64_t, const int64_t*,
+                                                 uint64_t, int64_t, EgreedyDraw, void*);
 }  // namespace arl
 
 extern "C" int arl_fc_heads_forward(const float* params, const float* prepared, int action_size,
@@ -347,8 +356,8 @@ extern "C" int arl_fc_heads_forward(const float* params, const float* prepared, 
                                     int32_t* actions, int64_t env_id_base, int64_t step,
                                     const int64_t* step_dev, uint64_t seed, int64_t num_samples,
                                     void* stream) {
-  return fc_heads_forward(params, prepared, action_size, a2, h, logits, probs, value, actions, env_id_base, step,
-                          step_dev, seed, num_samples, SampleDraw{}, stream);
+  return fc_heads_forward<SampleDraw, false>(params, prepared, action_size, a2, h, logits, probs, value, actions,
+                                             env_id_base, step, step_dev, seed, num_samples, SampleDraw{}, stream);
 }
 
 extern "C" int arl_fc_backward(const float* prepared, const float* a2, int64_t a2_block_rows,

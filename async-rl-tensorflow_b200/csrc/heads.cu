@@ -9,6 +9,7 @@
 
 #include "common.cuh"
 #include "../../include/asyncrl_b200_sarsa.h"
+#include "../../include/asyncrl_b200_dueling.h"
 
 namespace arl {
 
@@ -46,7 +47,9 @@ __device__ __forceinline__ void philox_two(uint32_t c0, uint32_t c1, uint32_t c2
 // (sample, output) walking 256 k serially: 10 us per 4096 samples, latency-bound.)
 //
 // The action draw after the heads is chosen by the last argument's type (common.cuh: SampleDraw or
-// EgreedyDraw).
+// EgreedyDraw).  Dueling (Wang et al. 2016, "average" aggregator) makes the A-wide head the advantage
+// stream and the 1-wide head the value stream: the row written to `logits` (and softmaxed into
+// `probs`, and drawn from) is then Q_j = v + (adv_j - mean_k adv_k); `value` is v either way.
 
 // agent.py:142-144  ep_end + max(0., (ep_start - ep_end) * (ep_end_t - max(0., step - learn_start))
 // / ep_end_t), in double, one correctly rounded operation at a time in Python's order (the _rn
@@ -60,7 +63,7 @@ __device__ __forceinline__ float egreedy_epsilon(const EgreedyDraw& d, int64_t s
 }
 
 constexpr int kHfThreads = 256;
-template <class Draw>
+template <class Draw, bool Dueling>
 __global__ void __launch_bounds__(kHfThreads)
 heads_fwd_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
                  const float* __restrict__ qw, const float* __restrict__ qb,
@@ -104,6 +107,11 @@ heads_fwd_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
       if (j == A) zv = t;
     }
     z += bias;
+    if constexpr (Dueling) {
+      // lane A holds the value head's sum: the mean runs over the lanes < A, one division by A
+      const float m = warp_sum(lane < A ? z : 0.f) / (float)A;
+      z = (zv + qb0) + (z - m);                       // TF: value + (advantage - reduce_mean(advantage))
+    }
     float mx = lane < A ? z : -INFINITY;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
@@ -241,6 +249,22 @@ __device__ __forceinline__ void acted_dq_row(float* dq, int A, int a, float delt
   for (int j = 0; j < A; ++j) dq[j] = j == a ? -2.0f * delta * grad_scale : 0.f;
 }
 
+// the same gradient through the dueling combine Q_j = v + adv_j - mean_k adv_k (heads_fwd_kernel):
+// g = -2 * delta * grad_scale, d adv_j = g * ([j == a] - 1/A), d v = g
+__device__ __forceinline__ void acted_dq_row(float* dadv, float* dv, int A, int a, float delta, float grad_scale) {
+  const float g = -2.0f * delta * grad_scale;
+  for (int j = 0; j < A; ++j) dadv[j] = g * ((j == a ? 1.f : 0.f) - 1.f / A);
+  *dv = g;
+}
+
+// the loss kernels' gradient store: the dQ row, or with Dueling the advantage row and d value
+template <bool Dueling>
+__device__ __forceinline__ void store_dq(float* dq, float* dvalue, int64_t n, int A, int a, float delta,
+                                         float grad_scale) {
+  if constexpr (Dueling) acted_dq_row(dq + n * A, dvalue + n, A, a, delta, grad_scale);
+  else acted_dq_row(dq + n * A, A, a, delta, grad_scale);
+}
+
 // loss_sums (optional) += {sum delta^2, sum Q(s)[a]}: a warp sum, then one atomic per warp
 __device__ __forceinline__ void add_q_loss_sums(float* loss_sums, float s_loss, float s_q) {
   if (loss_sums) {
@@ -256,13 +280,15 @@ __device__ __forceinline__ void add_q_loss_sums(float* loss_sums, float s_loss, 
 // ------------------------------- async-Q loss gradients -----------------------------------
 // agent.py:186-190, 310-314: target = clip(r) + (1 - terminal) * discount * max_a Q_target(s'),
 // delta = target - Q(s)[a], loss = mean(delta^2)  ->  dQ[a] = -2 * delta * grad_scale.
+// The three Q loss kernels take the head kind as a template argument and dvalue (Dueling only) last.
+template <bool Dueling>
 __global__ void q_lossgrad_kernel(const float* __restrict__ rewards,
                                   const uint8_t* __restrict__ terminals,
                                   const int32_t* __restrict__ actions, const float* __restrict__ q,
                                   const float* __restrict__ q_next, float* __restrict__ target,
                                   float* __restrict__ dq, float* __restrict__ loss_sums,
                                   int64_t num_samples, int A, float discount, float rmin, float rmax,
-                                  float grad_scale) {
+                                  float grad_scale, float* __restrict__ dvalue) {
   const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   float s_loss = 0.f, s_q = 0.f;
   if (n < num_samples) {
@@ -272,7 +298,7 @@ __global__ void q_lossgrad_kernel(const float* __restrict__ rewards,
     const int a = actions[n];
     const float delta = tgt - q[n * A + a];
     target[n] = tgt;
-    acted_dq_row(dq + n * A, A, a, delta, grad_scale);
+    store_dq<Dueling>(dq, dvalue, n, A, a, delta, grad_scale);
     s_loss = delta * delta;
     s_q = q[n * A + a];
   }
@@ -342,12 +368,14 @@ __global__ void returns_lossgrad_kernel(const float* __restrict__ rewards,
 // Asynchronous n-step Q-learning (Mnih et al. 2016): one thread per SAMPLE (t, b) as in
 // returns_lossgrad_kernel, the same return recurrence started from max_a Q(s_T; theta^-), then the
 // async-Q gradient of the acted action.
+template <bool Dueling>
 __global__ void nstep_q_lossgrad_kernel(const float* __restrict__ rewards,
                                         const uint8_t* __restrict__ terminals,
                                         const int32_t* __restrict__ actions, const float* __restrict__ q,
                                         const float* __restrict__ q_boot, float* __restrict__ returns,
                                         float* __restrict__ dq, float* __restrict__ loss_sums, int T, int B,
-                                        int A, float gamma, float rmin, float rmax, float grad_scale) {
+                                        int A, float gamma, float rmin, float rmax, float grad_scale,
+                                        float* __restrict__ dvalue) {
   const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   float s_loss = 0.f, s_q = 0.f;
   pdl_wait();
@@ -359,7 +387,7 @@ __global__ void nstep_q_lossgrad_kernel(const float* __restrict__ rewards,
     const int a = actions[n];
     const float qa = q[n * A + a];
     const float delta = R - qa;
-    acted_dq_row(dq + n * A, A, a, delta, grad_scale);
+    store_dq<Dueling>(dq, dvalue, n, A, a, delta, grad_scale);
     s_loss = delta * delta;
     s_q = qa;
   }
@@ -370,12 +398,14 @@ __global__ void nstep_q_lossgrad_kernel(const float* __restrict__ rewards,
 // Asynchronous one-step Sarsa (Mnih et al. 2016): q_lossgrad_kernel's target expression with
 // Q(s', a'; theta^-) of the action a' taken in s' in place of max_a.  actions holds a_0 .. a_T, so
 // the next action of sample n is actions[n + B] for every t, the last step included.
+template <bool Dueling>
 __global__ void sarsa_lossgrad_kernel(const float* __restrict__ rewards,
                                       const uint8_t* __restrict__ terminals,
                                       const int32_t* __restrict__ actions, const float* __restrict__ q,
                                       const float* __restrict__ q_next, float* __restrict__ target,
                                       float* __restrict__ dq, float* __restrict__ loss_sums, int T, int B,
-                                      int A, float gamma, float rmin, float rmax, float grad_scale) {
+                                      int A, float gamma, float rmin, float rmax, float grad_scale,
+                                      float* __restrict__ dvalue) {
   const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   float s_loss = 0.f, s_q = 0.f;
   pdl_wait();
@@ -387,7 +417,7 @@ __global__ void sarsa_lossgrad_kernel(const float* __restrict__ rewards,
     const float qa = q[n * A + a];
     const float delta = tgt - qa;
     target[n] = tgt;
-    acted_dq_row(dq + n * A, A, a, delta, grad_scale);
+    store_dq<Dueling>(dq, dvalue, n, A, a, delta, grad_scale);
     s_loss = delta * delta;
     s_q = qa;
   }
@@ -532,10 +562,11 @@ __global__ void observe_store_kernel(const float* __restrict__ reward, const uin
 }
 
 int heads_init() {
-  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<SampleDraw>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)((ARL_MAX_ACTIONS + 1) * 256 * sizeof(float))));
-  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<EgreedyDraw>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)((ARL_MAX_ACTIONS + 1) * 256 * sizeof(float))));
+  const int smem = (int)((ARL_MAX_ACTIONS + 1) * 256 * sizeof(float));
+  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<SampleDraw, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<EgreedyDraw, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<SampleDraw, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<EgreedyDraw, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   return ARL_OK;
 }
 
@@ -546,8 +577,9 @@ using namespace arl;
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 namespace arl {
-// heads + softmax + the draw; wait_first = 0 behind the fc256 kernel (fc_heads_forward), 1 stand-alone
-template <class Draw>
+// heads + softmax + the draw; wait_first = 0 behind the fc256 kernel (fc_heads_forward), 1 stand-alone;
+// Dueling: the Q row of the dueling combine (heads_fwd_kernel)
+template <class Draw, bool Dueling>
 int heads_forward(const float* params, int action_size, const float* h, float* logits, float* probs, float* value,
                   int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev, uint64_t seed,
                   int64_t num_samples, int wait_first, Draw draw, cudaStream_t st) {
@@ -557,17 +589,25 @@ int heads_forward(const float* params, int action_size, const float* h, float* l
   // up to 4 CTAs per SM: one env step of 4096 samples is ONE round of warps (two rounds cost a second
   // exposed load latency)
   const int grid = (int)(ctas < 4LL * num_sms() ? ctas : 4LL * num_sms());
-  ARL_CUDA(launch_pdl(heads_fwd_kernel<Draw>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
+  ARL_CUDA(launch_pdl(heads_fwd_kernel<Draw, Dueling>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
                       params + L.off[T_PB], params + L.off[T_QW], params + L.off[T_QB], h, logits, probs, value,
                       num_samples, action_size, actions, (uint64_t)env_id_base, (uint64_t)step, seed, step_dev,
                       wait_first, draw));
   ARL_LAUNCH_CHECK("heads_fwd_kernel");
   return ARL_OK;
 }
-template int heads_forward(const float*, int, const float*, float*, float*, float*, int32_t*, int64_t, int64_t,
-                           const int64_t*, uint64_t, int64_t, int, SampleDraw, cudaStream_t);
-template int heads_forward(const float*, int, const float*, float*, float*, float*, int32_t*, int64_t, int64_t,
-                           const int64_t*, uint64_t, int64_t, int, EgreedyDraw, cudaStream_t);
+template int heads_forward<SampleDraw, false>(const float*, int, const float*, float*, float*, float*, int32_t*,
+                                             int64_t, int64_t, const int64_t*, uint64_t, int64_t, int, SampleDraw,
+                                             cudaStream_t);
+template int heads_forward<EgreedyDraw, false>(const float*, int, const float*, float*, float*, float*, int32_t*,
+                                              int64_t, int64_t, const int64_t*, uint64_t, int64_t, int, EgreedyDraw,
+                                              cudaStream_t);
+template int heads_forward<SampleDraw, true>(const float*, int, const float*, float*, float*, float*, int32_t*,
+                                            int64_t, int64_t, const int64_t*, uint64_t, int64_t, int, SampleDraw,
+                                            cudaStream_t);
+template int heads_forward<EgreedyDraw, true>(const float*, int, const float*, float*, float*, float*, int32_t*,
+                                             int64_t, int64_t, const int64_t*, uint64_t, int64_t, int, EgreedyDraw,
+                                             cudaStream_t);
 }  // namespace arl
 
 extern "C" int arl_heads_forward(const float* params, int action_size, const float* h,
@@ -579,8 +619,8 @@ extern "C" int arl_heads_forward(const float* params, int action_size, const flo
   ARL_REQUIRE(num_samples >= 0, "arl_heads_forward: negative size");
   ARL_REQUIRE(aligned16(h), "arl_heads_forward: h must be 16-byte aligned");
   if (num_samples == 0) return ARL_OK;
-  return heads_forward(params, action_size, h, logits, probs, value, nullptr, 0, 0, nullptr, 0, num_samples,
-                       /*wait_first=*/1, SampleDraw{}, (cudaStream_t)stream);
+  return heads_forward<SampleDraw, false>(params, action_size, h, logits, probs, value, nullptr, 0, 0, nullptr, 0,
+                                          num_samples, /*wait_first=*/1, SampleDraw{}, (cudaStream_t)stream);
 }
 
 extern "C" int arl_sample_actions(const float* probs, int32_t* actions, int num_envs,
@@ -648,21 +688,42 @@ extern "C" int arl_egreedy_actions(const float* q, int32_t* actions, int num_env
   return ARL_OK;
 }
 
+// The Q loss entries: one launcher per learner for both head kinds (fn = the C entry's name, for errors)
+template <bool Dueling>
+static int q_lossgrad(const char* fn, const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                      const float* q, const float* q_next, float* target, float* dq, float* dvalue,
+                      float* loss_sums, int64_t num_samples, int action_size, float discount, float reward_min,
+                      float reward_max, float grad_scale, void* stream) {
+  ARL_REQUIRE(rewards && terminals && actions && q && q_next && target && dq && (dvalue || !Dueling),
+              "%s: null pointer", fn);
+  ARL_REQUIRE(num_samples >= 0, "%s: negative size", fn);
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "%s: action_size %d outside [1,%d]", fn, action_size, ARL_MAX_ACTIONS);
+  if (num_samples == 0) return ARL_OK;
+  q_lossgrad_kernel<Dueling><<<(unsigned)((num_samples + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+      rewards, terminals, actions, q, q_next, target, dq, loss_sums, num_samples, action_size,
+      discount, reward_min, reward_max, grad_scale, dvalue);
+  ARL_LAUNCH_CHECK("q_lossgrad_kernel");
+  return ARL_OK;
+}
+
 extern "C" int arl_q_lossgrad(const float* rewards, const uint8_t* terminals, const int32_t* actions,
                               const float* q, const float* q_next, float* target, float* dq,
                               float* loss_sums, int64_t num_samples, int action_size, float discount,
                               float reward_min, float reward_max, float grad_scale, void* stream) {
-  ARL_REQUIRE(rewards && terminals && actions && q && q_next && target && dq,
-              "arl_q_lossgrad: null pointer");
-  ARL_REQUIRE(num_samples >= 0, "arl_q_lossgrad: negative size");
-  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
-              "arl_q_lossgrad: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
-  if (num_samples == 0) return ARL_OK;
-  q_lossgrad_kernel<<<(unsigned)((num_samples + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
-      rewards, terminals, actions, q, q_next, target, dq, loss_sums, num_samples, action_size,
-      discount, reward_min, reward_max, grad_scale);
-  ARL_LAUNCH_CHECK("q_lossgrad_kernel");
-  return ARL_OK;
+  return q_lossgrad<false>("arl_q_lossgrad", rewards, terminals, actions, q, q_next, target, dq, nullptr,
+                           loss_sums, num_samples, action_size, discount, reward_min, reward_max, grad_scale,
+                           stream);
+}
+
+extern "C" int arl_q_lossgrad_dueling(const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                                      const float* q, const float* q_next, float* target, float* dq,
+                                      float* dvalue, float* loss_sums, int64_t num_samples, int action_size,
+                                      float discount, float reward_min, float reward_max, float grad_scale,
+                                      void* stream) {
+  return q_lossgrad<true>("arl_q_lossgrad_dueling", rewards, terminals, actions, q, q_next, target, dq, dvalue,
+                          loss_sums, num_samples, action_size, discount, reward_min, reward_max, grad_scale,
+                          stream);
 }
 
 extern "C" int arl_returns_lossgrad(const float* rewards, const uint8_t* terminals,
@@ -687,21 +748,60 @@ extern "C" int arl_returns_lossgrad(const float* rewards, const uint8_t* termina
   return ARL_OK;
 }
 
+template <bool Dueling>
+static int nstep_q_lossgrad(const char* fn, const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                            const float* q, const float* q_boot, float* returns, float* dq, float* dvalue,
+                            float* loss_sums, int t_max, int num_envs, int action_size, float gamma,
+                            float reward_min, float reward_max, float grad_scale, void* stream) {
+  ARL_REQUIRE(rewards && terminals && actions && q && q_boot && returns && dq && (dvalue || !Dueling),
+              "%s: null pointer", fn);
+  ARL_REQUIRE(t_max >= 0 && num_envs >= 0, "%s: negative size", fn);
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "%s: action_size %d outside [1,%d]", fn, action_size, ARL_MAX_ACTIONS);
+  if (t_max == 0 || num_envs == 0) return ARL_OK;
+  const int64_t total = (int64_t)t_max * num_envs;
+  ARL_CUDA(launch_pdl(nstep_q_lossgrad_kernel<Dueling>, dim3((unsigned)((total + 127) / 128)), dim3(128), 0,
+                      (cudaStream_t)stream, rewards, terminals, actions, q, q_boot, returns, dq, loss_sums, t_max,
+                      num_envs, action_size, gamma, reward_min, reward_max, grad_scale, dvalue));
+  ARL_LAUNCH_CHECK("nstep_q_lossgrad_kernel");
+  return ARL_OK;
+}
+
 extern "C" int arl_nstep_q_lossgrad(const float* rewards, const uint8_t* terminals, const int32_t* actions,
                                     const float* q, const float* q_boot, float* returns, float* dq,
                                     float* loss_sums, int t_max, int num_envs, int action_size, float gamma,
                                     float reward_min, float reward_max, float grad_scale, void* stream) {
-  ARL_REQUIRE(rewards && terminals && actions && q && q_boot && returns && dq,
-              "arl_nstep_q_lossgrad: null pointer");
-  ARL_REQUIRE(t_max >= 0 && num_envs >= 0, "arl_nstep_q_lossgrad: negative size");
+  return nstep_q_lossgrad<false>("arl_nstep_q_lossgrad", rewards, terminals, actions, q, q_boot, returns, dq,
+                                 nullptr, loss_sums, t_max, num_envs, action_size, gamma, reward_min, reward_max,
+                                 grad_scale, stream);
+}
+
+extern "C" int arl_nstep_q_lossgrad_dueling(const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                                            const float* q, const float* q_boot, float* returns, float* dq,
+                                            float* dvalue, float* loss_sums, int t_max, int num_envs,
+                                            int action_size, float gamma, float reward_min, float reward_max,
+                                            float grad_scale, void* stream) {
+  return nstep_q_lossgrad<true>("arl_nstep_q_lossgrad_dueling", rewards, terminals, actions, q, q_boot, returns,
+                                dq, dvalue, loss_sums, t_max, num_envs, action_size, gamma, reward_min,
+                                reward_max, grad_scale, stream);
+}
+
+template <bool Dueling>
+static int sarsa_lossgrad(const char* fn, const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                          const float* q, const float* q_next, float* target, float* dq, float* dvalue,
+                          float* loss_sums, int t_max, int num_envs, int action_size, float gamma,
+                          float reward_min, float reward_max, float grad_scale, void* stream) {
+  ARL_REQUIRE(rewards && terminals && actions && q && q_next && target && dq && (dvalue || !Dueling),
+              "%s: null pointer", fn);
+  ARL_REQUIRE(t_max >= 0 && num_envs >= 0, "%s: negative size", fn);
   ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
-              "arl_nstep_q_lossgrad: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
+              "%s: action_size %d outside [1,%d]", fn, action_size, ARL_MAX_ACTIONS);
   if (t_max == 0 || num_envs == 0) return ARL_OK;
   const int64_t total = (int64_t)t_max * num_envs;
-  ARL_CUDA(launch_pdl(nstep_q_lossgrad_kernel, dim3((unsigned)((total + 127) / 128)), dim3(128), 0,
-                      (cudaStream_t)stream, rewards, terminals, actions, q, q_boot, returns, dq, loss_sums, t_max,
-                      num_envs, action_size, gamma, reward_min, reward_max, grad_scale));
-  ARL_LAUNCH_CHECK("nstep_q_lossgrad_kernel");
+  ARL_CUDA(launch_pdl(sarsa_lossgrad_kernel<Dueling>, dim3((unsigned)((total + 127) / 128)), dim3(128), 0,
+                      (cudaStream_t)stream, rewards, terminals, actions, q, q_next, target, dq, loss_sums, t_max,
+                      num_envs, action_size, gamma, reward_min, reward_max, grad_scale, dvalue));
+  ARL_LAUNCH_CHECK("sarsa_lossgrad_kernel");
   return ARL_OK;
 }
 
@@ -709,18 +809,19 @@ extern "C" int arl_sarsa_lossgrad(const float* rewards, const uint8_t* terminals
                                   const float* q, const float* q_next, float* target, float* dq,
                                   float* loss_sums, int t_max, int num_envs, int action_size, float gamma,
                                   float reward_min, float reward_max, float grad_scale, void* stream) {
-  ARL_REQUIRE(rewards && terminals && actions && q && q_next && target && dq,
-              "arl_sarsa_lossgrad: null pointer");
-  ARL_REQUIRE(t_max >= 0 && num_envs >= 0, "arl_sarsa_lossgrad: negative size");
-  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
-              "arl_sarsa_lossgrad: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
-  if (t_max == 0 || num_envs == 0) return ARL_OK;
-  const int64_t total = (int64_t)t_max * num_envs;
-  ARL_CUDA(launch_pdl(sarsa_lossgrad_kernel, dim3((unsigned)((total + 127) / 128)), dim3(128), 0,
-                      (cudaStream_t)stream, rewards, terminals, actions, q, q_next, target, dq, loss_sums, t_max,
-                      num_envs, action_size, gamma, reward_min, reward_max, grad_scale));
-  ARL_LAUNCH_CHECK("sarsa_lossgrad_kernel");
-  return ARL_OK;
+  return sarsa_lossgrad<false>("arl_sarsa_lossgrad", rewards, terminals, actions, q, q_next, target, dq, nullptr,
+                               loss_sums, t_max, num_envs, action_size, gamma, reward_min, reward_max, grad_scale,
+                               stream);
+}
+
+extern "C" int arl_sarsa_lossgrad_dueling(const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                                          const float* q, const float* q_next, float* target, float* dq,
+                                          float* dvalue, float* loss_sums, int t_max, int num_envs,
+                                          int action_size, float gamma, float reward_min, float reward_max,
+                                          float grad_scale, void* stream) {
+  return sarsa_lossgrad<true>("arl_sarsa_lossgrad_dueling", rewards, terminals, actions, q, q_next, target, dq,
+                              dvalue, loss_sums, t_max, num_envs, action_size, gamma, reward_min, reward_max,
+                              grad_scale, stream);
 }
 
 extern "C" int arl_act_update(const float* step_reward, const uint8_t* step_terminal,

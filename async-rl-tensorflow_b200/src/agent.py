@@ -40,6 +40,12 @@ class Agent(BaseModel):
         self.global_envs = self.world_size * self.num_envs
 
         self.step_op = 0                                         # agent.py:25 global step (host int)
+        # config.py:36 dueling: Wang et al. 2016's dueling Q heads for the Q learners (Network.dueling);
+        # a policy/value network has no dueling form
+        self.dueling = bool(getattr(config, 'dueling', False))
+        if self.dueling and getattr(config, 'loss_mode', 'a3c') == 'a3c':
+            raise ValueError("dueling=True needs a Q learner (loss_mode 'async_q', 'nstep_q' or 'sarsa'); "
+                             "loss_mode 'a3c' trains a policy/value network, which has no dueling form")
         # network.py:30-55: 'nips' (what agent.py:226-252 wires, the default) or 'nature'
         self.network = make_network(
             DQN_type=getattr(config, 'DQN_type', 'nips'), action_size=self.env.action_size, data_format=self.cnn_format,
@@ -47,7 +53,7 @@ class Agent(BaseModel):
             screen_width=self.screen_width, gamma=self.discount, beta=self.beta,
             num_envs=self.num_envs, t_max=self.t_max, device=self.device, seed=self.seed,
             decay=self.decay, epsilon=self.epsilon, clip_norm=self.clip_norm,
-            min_reward=self.min_reward, max_reward=self.max_reward)
+            min_reward=self.min_reward, max_reward=self.max_reward, dueling=self.dueling)
         self.w = self.network.w
         # the per-cycle exchange runs inside the library (arl_comm_init / arl_backward(allreduce=1):
         # NCCL, bucketed so that the fc256 gradient travels while the conv backward kernels run);

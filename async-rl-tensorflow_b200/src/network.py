@@ -86,11 +86,16 @@ def initial_weights(action_size, seed=123, stddev=0.02):
 
 
 class Network(object):
+    # dueling Q heads (Wang et al. 2016, include/asyncrl_b200_dueling.h): the Q row every Q forward
+    # writes to ``policy_logits`` is v + (adv - mean adv), with p_w/p_b the advantage stream and q_w/q_b
+    # the value stream; the Q losses then train both heads.  Fixed for the network's life.
+    dueling = False
+
     def __init__(self, sess=None, data_format='NHWC', history_length=4, screen_height=84,
                  screen_width=84, action_size=6, activation_fn='relu', initializer=None,
                  gamma=0.99, beta=0.01, global_network=None, global_optim=None, DQN_type='nips',
                  num_envs=256, t_max=5, device='cuda', seed=123, decay=0.99, epsilon=0.1,
-                 clip_norm=40.0, min_reward=-1.0, max_reward=1.0):
+                 clip_norm=40.0, min_reward=-1.0, max_reward=1.0, dueling=False):
         if DQN_type.lower() != 'nips':
             raise ValueError("Network is the 'nips' trunk (network.py:43-52); DQN_type='nature' "
                              "(network.py:30-42) is network_nature.NatureNetwork -- use "
@@ -109,6 +114,7 @@ class Network(object):
         self.decay, self.epsilon, self.clip_norm = float(decay), float(epsilon), float(clip_norm)
         self.min_reward, self.max_reward = float(min_reward), float(max_reward)
         self.global_network = global_network
+        self.dueling = bool(dueling)
 
         A, B, T = self.action_size, self.num_envs, self.t_max
         self.offsets = _cabi.param_layout(A)
@@ -209,6 +215,10 @@ class Network(object):
         P, st = _cabi.ptr, _cabi.stream_ptr()
         B, A = self.num_envs, self.action_size
         refresh = self._refresh(refresh)
+        if self.dueling:
+            self._forward_dueling(self.params, self.fc_w, refresh, history, history.first_slot(0), 1, l1, l2, l4,
+                                  logits, probs, value)
+            return
         if self.timed is None:
             _cabi.call("arl_forward", P(self.params), P(self.fc_w), refresh, A, P(history.ring), B,
                        history.ring_slots, history.first_slot(0), 1, P(l1), P(l2), P(l4),
@@ -217,6 +227,18 @@ class Network(object):
         if refresh:
             _cabi.call("arl_prepare_weights", P(self.params), P(self.fc_w), st)
         self._timed_layers(history, l1, l2, l4, logits, probs, value, None, 0, 0, None, 0)
+
+    def _forward_dueling(self, params, fc_w, refresh, history, first_slot, steps, l1, l2, l4, logits, probs, value,
+                         actions=None, env_id_base=0, step=0, step_dev=None, seed=0, ep=0.0, ep_sched=None):
+        """arl_forward_dueling: ``steps`` env steps from ``first_slot`` under ``params`` with the dueling Q
+        row into ``logits``; with ``actions`` (one step) also the epsilon-greedy draw of
+        ``forward_egreedy``.  One entry under ``timed``."""
+        P = _cabi.ptr
+        e0, e1, et, ls = (float(x) for x in (ep_sched if ep_sched is not None else (0.0, 0.0, 1.0, 0.0)))
+        self._timed_call("arl_forward_dueling", P(params), P(fc_w), int(bool(refresh)), self.action_size,
+                         P(history.ring), self.num_envs, history.ring_slots, first_slot, steps, P(l1), P(l2), P(l4),
+                         P(logits), P(probs), P(value), P(actions), int(env_id_base), int(step), P(step_dev),
+                         int(seed), float(ep), e0, e1, et, ls, _cabi.stream_ptr())
 
     def _timed_layers(self, history, l1, l2, l4, logits, probs, value, actions, env_id_base, step, sd, seed):
         """The per-layer entries arl_forward / arl_forward_sample are made of, one event pair each
@@ -247,6 +269,7 @@ class Network(object):
         """``forward`` into rollout slot t + ``sample`` (network.py:72) as one composed call: the
         heads and the Philox draw run inside the fc256 kernel (arl_forward_sample).  The Philox step
         is ``step`` (+ the int64 device counter ``step_dev`` when given)."""
+        self._policy_value_only("forward_sample")
         r = self._rows(t)
         P, st = _cabi.ptr, _cabi.stream_ptr()
         B, A = self.num_envs, self.action_size
@@ -314,6 +337,7 @@ class Network(object):
 
     def bootstrap_value(self, history, refresh=None):
         """V(s_T) under the same theta (Algorithm 3: R = V(s_t, theta'_v))."""
+        self._policy_value_only("bootstrap_value")
         b = self._b
         self._forward_into(history, b['l1'], b['l2'], b['l4'], b['logits'], b['probs'], b['value'],
                            refresh)
@@ -365,6 +389,7 @@ class Network(object):
                           grad_scale=1.0, allreduce=False, refresh=None):
         """Returns + loss grads (K4) then the full backward (agent.py:317) over the T*B samples
         of the rollout.  ``history`` must have had exactly t_max pushes since s_0."""
+        self._policy_value_only("compute_gradients")
         T, B, A = self.t_max, self.num_envs, self.action_size
         acts = self.sampled_action if actions is None else actions
         self.loss_sums.zero_()
@@ -375,6 +400,13 @@ class Network(object):
                          _cabi.ptr(self.d_value), _cabi.ptr(self.loss_sums), T, B, A, self.gamma,
                          self.beta, self.min_reward, self.max_reward, float(grad_scale), st)
         return self._backward(history, grad_scale, allreduce, refresh)
+
+    def _policy_value_only(self, entry):
+        """The A3C entry points (policy sample, V(s_T) bootstrap, policy/value loss) have no dueling
+        form: with dueling heads the A-wide head is an advantage stream, not policy logits."""
+        if self.dueling:
+            raise ValueError("Network.%s is the A3C policy/value path; a dueling network (dueling=True) "
+                             "serves the Q learners only" % entry)
 
     def _backward(self, history, grad_scale, allreduce, refresh):
         """The backward (agent.py:317) of every learner from d_logits / d_value over the T*B samples
@@ -457,16 +489,31 @@ class Network(object):
         T, B, A = self.t_max, self.num_envs, self.action_size
         P, st = _cabi.ptr, _cabi.stream_ptr()
         probs, value = self._tq_scratch
-        _cabi.call("arl_forward", P(self.target_params), P(self.target_fc_w), 1, A, P(history.ring),
-                   B, history.ring_slots, history.first_slot(T - 1), T, P(self.d_l1), P(self.d_l2),
-                   P(self.d_l4), P(self.target_q), P(probs), P(value), st)
+        if self.dueling:
+            self._forward_dueling(self.target_params, self.target_fc_w, 1, history, history.first_slot(T - 1), T,
+                                  self.d_l1, self.d_l2, self.d_l4, self.target_q, probs, value)
+        else:
+            _cabi.call("arl_forward", P(self.target_params), P(self.target_fc_w), 1, A, P(history.ring),
+                       B, history.ring_slots, history.first_slot(T - 1), T, P(self.d_l1), P(self.d_l2),
+                       P(self.d_l4), P(self.target_q), P(probs), P(value), st)
         self.loss_sums.zero_()
-        _cabi.call("arl_q_lossgrad", P(rewards), P(terminals), P(self.sampled_action),
-                   P(self.policy_logits), P(self.target_q), P(self.target_q_t), P(self.d_logits),
-                   P(self.loss_sums), T * B, A, self.gamma, self.min_reward, self.max_reward,
-                   float(grad_scale), st)
-        self.d_value.zero_()                                   # the value head is unused
+        self._q_lossgrad("arl_q_lossgrad", (P(rewards), P(terminals), P(self.sampled_action), P(self.policy_logits),
+                                            P(self.target_q), P(self.target_q_t)),
+                         (P(self.loss_sums), T * B, A, self.gamma, self.min_reward, self.max_reward,
+                          float(grad_scale), st), timed=False)
         return self._backward(history, grad_scale, allreduce, None)
+
+    def _q_lossgrad(self, name, head, tail, timed=True):
+        """A Q learner's loss entry ``name``: its arguments are ``head``, the dQ row (d_logits), ``tail``.
+        Dueling: the entry's dueling form, which also writes d_value (dL/dv); else the value head is
+        unused and d_value is zeroed.  ``timed``: an event pair around it under ``timed``."""
+        P = _cabi.ptr
+        call = self._timed_call if timed else _cabi.call
+        if self.dueling:
+            call(name + "_dueling", *head, P(self.d_logits), P(self.d_value), *tail)
+        else:
+            call(name, *head, P(self.d_logits), *tail)
+            self.d_value.zero_()                               # the value head is unused
 
     # -- n-step Q mode (Mnih et al. 2016, asynchronous n-step Q-learning): the Q head is the p_w/p_b
     # slot as in async_q; the cycle is the A3C cycle with the bootstrap taken from the target network
@@ -490,6 +537,11 @@ class Network(object):
         refresh = self._refresh(refresh)
         if step_dev is not None and ep_sched is None:
             raise ValueError("forward_egreedy: step_dev needs ep_sched = (ep_start, ep_end, ep_end_t, learn_start)")
+        if self.dueling:
+            self._forward_dueling(self.params, self.fc_w, refresh, history, history.first_slot(0), 1, self.l1[r],
+                                  self.l2[r], self.l4[r], self.policy_logits[r], self.policy[r], self.value[r],
+                                  self.sampled_action[r], env_id_base, step, step_dev, seed, ep, ep_sched)
+            return self.sampled_action[r]
         e0, e1, et, ls = (float(x) for x in (ep_sched if ep_sched is not None else (0.0, 0.0, 1.0, 0.0)))
         self._timed_call("arl_forward_egreedy", P(self.params), P(self.fc_w), refresh, self.action_size,
                          P(history.ring), self.num_envs, history.ring_slots, history.first_slot(0), P(self.l1[r]),
@@ -510,14 +562,19 @@ class Network(object):
         b = self._b
         if target_refresh is None:
             target_refresh = self._target_fc_w_stale()
-        self._timed_call("arl_forward", P(self.target_params), P(self.target_fc_w), int(bool(target_refresh)), A,
-                         P(history.ring), B, history.ring_slots, history.first_slot(0), 1, P(b['l1']), P(b['l2']),
-                         P(b['l4']), P(self.q_boot), P(b['probs']), P(b['value']), st)
+        if self.dueling:
+            self._forward_dueling(self.target_params, self.target_fc_w, target_refresh, history,
+                                  history.first_slot(0), 1, b['l1'], b['l2'], b['l4'], self.q_boot, b['probs'],
+                                  b['value'])
+        else:
+            self._timed_call("arl_forward", P(self.target_params), P(self.target_fc_w), int(bool(target_refresh)),
+                             A, P(history.ring), B, history.ring_slots, history.first_slot(0), 1, P(b['l1']),
+                             P(b['l2']), P(b['l4']), P(self.q_boot), P(b['probs']), P(b['value']), st)
         self.loss_sums.zero_()
-        self._timed_call("arl_nstep_q_lossgrad", P(rewards), P(terminals), P(self.sampled_action),
-                         P(self.policy_logits), P(self.q_boot), P(self.R), P(self.d_logits), P(self.loss_sums),
-                         T, B, A, self.gamma, self.min_reward, self.max_reward, float(grad_scale), st)
-        self.d_value.zero_()                                   # the value head is unused
+        self._q_lossgrad("arl_nstep_q_lossgrad", (P(rewards), P(terminals), P(self.sampled_action),
+                                                  P(self.policy_logits), P(self.q_boot), P(self.R)),
+                         (P(self.loss_sums), T, B, A, self.gamma, self.min_reward, self.max_reward,
+                          float(grad_scale), st))
         return self._backward(history, grad_scale, allreduce, refresh)
 
     # -- one-step Sarsa mode (Mnih et al. 2016, asynchronous one-step Sarsa): async_q's Q head,
@@ -541,20 +598,28 @@ class Network(object):
         probs, value = self._tq_scratch
         if target_refresh is None:
             target_refresh = self._target_fc_w_stale()
-        self._timed_call("arl_forward", P(self.target_params), P(self.target_fc_w), int(bool(target_refresh)), A,
-                         P(history.ring), B, history.ring_slots, history.first_slot(T - 1), T, P(self.d_l1),
-                         P(self.d_l2), P(self.d_l4), P(self.target_q), P(probs), P(value), st)
-        e0, e1, et, ls = (float(x) for x in ep_sched)
-        self._timed_call("arl_forward_egreedy", P(self.params), P(self.fc_w), self._refresh(refresh), A,
-                         P(history.ring), B, history.ring_slots, history.first_slot(0), P(b['l1']), P(b['l2']),
-                         P(b['l4']), P(b['logits']), P(b['probs']), P(b['value']), P(self.sarsa_actions[T * B:]),
-                         int(env_id_base), 0, P(step_dev), int(seed), 0.0, e0, e1, et, ls, st)
+        if self.dueling:
+            self._forward_dueling(self.target_params, self.target_fc_w, target_refresh, history,
+                                  history.first_slot(T - 1), T, self.d_l1, self.d_l2, self.d_l4, self.target_q, probs,
+                                  value)
+            self._forward_dueling(self.params, self.fc_w, self._refresh(refresh), history, history.first_slot(0), 1,
+                                  b['l1'], b['l2'], b['l4'], b['logits'], b['probs'], b['value'],
+                                  self.sarsa_actions[T * B:], env_id_base, 0, step_dev, seed, 0.0, ep_sched)
+        else:
+            self._timed_call("arl_forward", P(self.target_params), P(self.target_fc_w), int(bool(target_refresh)),
+                             A, P(history.ring), B, history.ring_slots, history.first_slot(T - 1), T, P(self.d_l1),
+                             P(self.d_l2), P(self.d_l4), P(self.target_q), P(probs), P(value), st)
+            e0, e1, et, ls = (float(x) for x in ep_sched)
+            self._timed_call("arl_forward_egreedy", P(self.params), P(self.fc_w), self._refresh(refresh), A,
+                             P(history.ring), B, history.ring_slots, history.first_slot(0), P(b['l1']), P(b['l2']),
+                             P(b['l4']), P(b['logits']), P(b['probs']), P(b['value']),
+                             P(self.sarsa_actions[T * B:]), int(env_id_base), 0, P(step_dev), int(seed), 0.0, e0, e1,
+                             et, ls, st)
         self.loss_sums.zero_()
-        self._timed_call("arl_sarsa_lossgrad", P(rewards), P(terminals), P(self.sarsa_actions),
-                         P(self.policy_logits), P(self.target_q), P(self.target_q_t), P(self.d_logits),
-                         P(self.loss_sums), T, B, A, self.gamma, self.min_reward, self.max_reward,
-                         float(grad_scale), st)
-        self.d_value.zero_()                                   # the value head is unused
+        self._q_lossgrad("arl_sarsa_lossgrad", (P(rewards), P(terminals), P(self.sarsa_actions),
+                                                P(self.policy_logits), P(self.target_q), P(self.target_q_t)),
+                         (P(self.loss_sums), T, B, A, self.gamma, self.min_reward, self.max_reward,
+                          float(grad_scale), st))
         return self._backward(history, grad_scale, allreduce, False)   # fc_w: refreshed by step 2
 
     @property
@@ -606,6 +671,8 @@ class Network(object):
         blobs = {k: v.detach().cpu().numpy() for k, v in self.w.items()}
         blobs["rms"] = self.rms.detach().cpu().numpy()
         blobs["step"] = np.int64(step if step is not None else 0)
+        if self.dueling:                                       # absent = not dueling: older files load as such
+            blobs["dueling"] = np.bool_(True)
         np.savez(path, **blobs)
         return path
 
@@ -617,6 +684,11 @@ class Network(object):
         if not files:
             return False
         z = np.load(os.path.join(checkpoint_dir, files[-1]))
+        saved = bool(z["dueling"]) if "dueling" in z.files else False
+        if saved != self.dueling:                              # same weights, another function: refuse
+            raise ValueError("checkpoint %s was written by a %s network; this network is %s"
+                             % (files[-1], "dueling" if saved else "non-dueling",
+                                "dueling" if self.dueling else "non-dueling"))
         self.set_weights({k: z[k] for k in PARAM_NAMES})
         self.rms.copy_(torch.as_tensor(z["rms"]))
         self.loaded_step = int(z["step"])
@@ -630,6 +702,9 @@ def make_network(DQN_type='nips', **kw):
     if kind == 'nips':
         return Network(DQN_type='nips', **kw)
     if kind == 'nature':
+        if kw.pop('dueling', False):
+            raise NotImplementedError("dueling Q heads are built on the nips trunk (agent.py:226-252); the "
+                                      "nature trunk is A3C-only")
         from .network_nature import NatureNetwork
         return NatureNetwork(DQN_type='nature', **kw)
     raise ValueError('Wrong DQN type: %s' % DQN_type)

@@ -6,7 +6,8 @@
  * arl_status, message in arl_last_error()), device pointers owned by the caller, samples indexed
  * n = t * num_envs + b, launches asynchronous on `stream` (last argument).  The Q values are the
  * p_w/p_b head ("logits"), as in the async-Q and n-step Q entries of asyncrl_b200.h; the value head
- * q_w/q_b is computed but unused by this learner.  The rest of the Sarsa cycle runs on entries of
+ * q_w/q_b is computed but unused by this learner (asyncrl_b200_dueling.h: with dueling heads it is
+ * the value stream).  The rest of the Sarsa cycle runs on entries of
  * asyncrl_b200.h: arl_forward on the target parameters over s_1..s_T (q_next), arl_forward_egreedy
  * on s_T for the action a_T the next rollout starts with, arl_backward.
  */

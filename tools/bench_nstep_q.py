@@ -2,7 +2,8 @@
 async_q eager (its own path: host epsilon, a separate draw launch, a target forward over all T*B next
 states; sarsa runs that target forward too, inside its graph).
 
-    python tools/bench_nstep_q.py [--rounds R] [--cycles K] [--modes a3c,nstep_q,...] [--out FILE]
+    python tools/bench_nstep_q.py [--rounds R] [--cycles K] [--modes a3c,nstep_q,...] [--dueling off|on|both]
+                                  [--out FILE]
 
 For each shape (envs x t_max x actions: 4096 x 5 x 6 and 16384 x 20 x 18) one agent per mode is built
 and warmed up until a whole ring period has replayed without a new graph capture; then the modes take
@@ -11,6 +12,9 @@ event pair around every K-cycle block.  Reported per mode: ms per cycle (median,
 rounds) and env frames/s (envs x t_max / median cycle time).  The card's name and power limit are
 read in the same run and written beside the numbers.  Synthetic frames, resident in HBM; the frame
 pool is larger than L2 at both shapes.
+
+--dueling on runs the Q learners with dueling Q heads (dueling=True; reported as "<mode>+dueling"),
+--dueling both runs every Q learner both ways, all of them alternating.
 """
 import argparse
 import importlib
@@ -46,14 +50,25 @@ def main():
     ap.add_argument("--cycles", type=int, default=20, help="cycles per timed block")
     ap.add_argument("--shapes", default="4096x5x6,16384x20x18", help="envs x t_max x actions, comma separated")
     ap.add_argument("--modes", default=",".join(MODES))
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r05_sarsa_bench.json"))
+    ap.add_argument("--dueling", default="off", choices=("off", "on", "both"),
+                    help="dueling Q heads for the Q learners: off, on, or both (each Q learner twice)")
+    ap.add_argument("--out", default=None, help="default: profiles/r05_sarsa_bench.json, or "
+                                                "profiles/r06_dueling_bench.json with --dueling on|both")
     args = ap.parse_args()
+    if args.out is None:
+        args.out = os.path.join(ROOT, "profiles", "r05_sarsa_bench.json" if args.dueling == "off"
+                                else "r06_dueling_bench.json")
     if not torch.cuda.is_available():
         sys.exit("bench_nstep_q: needs a CUDA device")
     pkg = importlib.import_module("async-rl-tensorflow_b200")
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
-    modes = args.modes.split(",")
+    modes = []
+    for m in args.modes.split(","):
+        if args.dueling != "on" or m == "a3c":
+            modes.append(m)
+        if args.dueling != "off" and m != "a3c":
+            modes.append(m + "+dueling")
     result = {"card": card(), "rounds": args.rounds, "cycles_per_block": args.cycles, "shapes": []}
 
     for shape in args.shapes.split(","):
@@ -61,7 +76,8 @@ def main():
         pool = max(2, min(T, int(24e9 // (B * 100800) // len(modes))))   # frames kept per agent
         agents = {}
         for mode in modes:
-            cfg = pkg.config.get_config({"model": "m1", "num_envs": B, "t_max": T, "loss_mode": mode})
+            cfg = pkg.config.get_config({"model": "m1", "num_envs": B, "t_max": T, "loss_mode": mode.split("+")[0],
+                                         "dueling": mode.endswith("+dueling")})
             env = pkg.GymEnvironment(cfg, env=pkg.SyntheticAtari(B, A, seed=123, pool=pool, device=dev), device=dev)
             agent = pkg.Agent(cfg, env, device=dev)
             random.seed(cfg.seed)
