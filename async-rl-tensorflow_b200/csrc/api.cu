@@ -139,6 +139,9 @@ extern "C" int arl_forward(const float* params, float* prepared, int refresh_pre
                            const uint8_t* ring, int num_envs, int ring_slots, int first_slot, int steps,
                            float* a1, float* a2, float* h, float* logits, float* probs, float* value,
                            void* stream) {
+  // refused before the first launch: a bad action count must leave a1, a2 and `prepared` as they were
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_forward: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
   const int64_t N = (int64_t)num_envs * steps;
   int rc = ARL_OK;
   if (refresh_prepared) rc = arl_prepare_weights(params, prepared, stream);
@@ -160,6 +163,8 @@ extern "C" int arl_forward_sample(const float* params, float* prepared, int refr
                                   int32_t* actions, int64_t env_id_base, int64_t step,
                                   const int64_t* step_dev, uint64_t seed, void* stream) {
   ARL_REQUIRE(actions, "arl_forward_sample: null pointer");
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_forward_sample: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
   int rc = ARL_OK;
   if (refresh_prepared) rc = arl_prepare_weights(params, prepared, stream);
   if (rc) return rc;
