@@ -1,5 +1,5 @@
 """ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h, include/asyncrl_b200_sarsa.h,
-include/asyncrl_b200_dueling.h).
+include/asyncrl_b200_dueling.h, include/asyncrl_b200_double.h).
 
 The product path has no CPU fallback: if the shared library is missing or a call
 fails, this module raises.  PyTorch is only the carrier of device memory and
@@ -114,6 +114,18 @@ DUELING_SIGNATURES = {
                                    c_f32, c_f32, c_f32, c_f32, c_vp],
 }
 
+# the double Q-learning targets: their own header (include/asyncrl_b200_double.h), their own table
+DOUBLE_SIGNATURES = {
+    "arl_double_q_lossgrad": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_f32,
+                              c_f32, c_f32, c_f32, c_vp],
+    "arl_double_q_lossgrad_dueling": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int,
+                                      c_int, c_f32, c_f32, c_f32, c_f32, c_vp],
+    "arl_double_nstep_q_lossgrad": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int,
+                                    c_f32, c_f32, c_f32, c_f32, c_vp],
+    "arl_double_nstep_q_lossgrad_dueling": [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int,
+                                            c_int, c_int, c_f32, c_f32, c_f32, c_f32, c_vp],
+}
+
 
 class ArlError(RuntimeError):
     pass
@@ -132,7 +144,8 @@ def load():
         raise ArlError("%s is missing: build it with async-rl-tensorflow_b200/csrc/build.sh "
                        "(or __graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = ctypes.CDLL(LIB_PATH)
-    for name, argtypes in list(SIGNATURES.items()) + list(SARSA_SIGNATURES.items()) + list(DUELING_SIGNATURES.items()):
+    for name, argtypes in (list(SIGNATURES.items()) + list(SARSA_SIGNATURES.items())
+                           + list(DUELING_SIGNATURES.items()) + list(DOUBLE_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes, fn.restype = argtypes, c_int
     for name, (argtypes, restype) in OTHER.items():

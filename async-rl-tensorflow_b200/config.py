@@ -32,7 +32,10 @@ class AgentConfig(object):
     min_delta = -1
     max_delta = 1
 
-    double_q = False
+    double_q = False                     # double Q-learning targets (van Hasselt et al. 2016, Double DQN) for the
+                                         # learners that bootstrap from a max (async_q, nstep_q): the online network
+                                         # picks a* = argmax_a Q(s'; theta), the target network evaluates
+                                         # Q(s', a*; theta^-); a3c and sarsa refuse it, as does the nature trunk
     dueling = False                      # dueling Q heads (Wang et al. 2016, "average" aggregator) for the
                                          # Q learners (async_q, nstep_q, sarsa) on the nips trunk: p_w/p_b is the
                                          # advantage stream, q_w/q_b the value stream, both on fc256's output

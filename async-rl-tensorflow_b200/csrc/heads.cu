@@ -10,6 +10,7 @@
 #include "common.cuh"
 #include "../../include/asyncrl_b200_sarsa.h"
 #include "../../include/asyncrl_b200_dueling.h"
+#include "../../include/asyncrl_b200_double.h"
 
 namespace arl {
 
@@ -244,6 +245,15 @@ __device__ __forceinline__ float q_row_max(const float* q, int A) {
   return mx;
 }
 
+// argmax_a q[a], ties -> lowest index (greedy_actions_kernel's rule, tf.argmax)
+__device__ __forceinline__ int q_row_argmax(const float* q, int A) {
+  int a = 0;
+  float best = q[0];
+  for (int j = 1; j < A; ++j)
+    if (q[j] > best) { best = q[j]; a = j; }
+  return a;
+}
+
 // the gradient of grad_scale * delta^2 w.r.t. the Q row: -2 * delta * grad_scale at the acted action
 __device__ __forceinline__ void acted_dq_row(float* dq, int A, int a, float delta, float grad_scale) {
   for (int j = 0; j < A; ++j) dq[j] = j == a ? -2.0f * delta * grad_scale : 0.f;
@@ -281,18 +291,30 @@ __device__ __forceinline__ void add_q_loss_sums(float* loss_sums, float s_loss, 
 // agent.py:186-190, 310-314: target = clip(r) + (1 - terminal) * discount * max_a Q_target(s'),
 // delta = target - Q(s)[a], loss = mean(delta^2)  ->  dQ[a] = -2 * delta * grad_scale.
 // The three Q loss kernels take the head kind as a template argument and dvalue (Dueling only) last.
-template <bool Dueling>
+// Double (van Hasselt et al. 2016, Double DQN): the bootstrap is Q(s', a*; theta^-) with
+// a* = argmax_a Q(s', a; theta) in place of max_a Q(s'; theta^-).  The online rows of s' are the
+// rollout's own Q rows (q row n + B) for t < T-1 and q_online_T (row b) for t = T-1; these
+// arguments come after dvalue, so the plain instantiations keep their parameter offsets.
+template <bool Dueling, bool Double>
 __global__ void q_lossgrad_kernel(const float* __restrict__ rewards,
                                   const uint8_t* __restrict__ terminals,
                                   const int32_t* __restrict__ actions, const float* __restrict__ q,
                                   const float* __restrict__ q_next, float* __restrict__ target,
                                   float* __restrict__ dq, float* __restrict__ loss_sums,
                                   int64_t num_samples, int A, float discount, float rmin, float rmax,
-                                  float grad_scale, float* __restrict__ dvalue) {
+                                  float grad_scale, float* __restrict__ dvalue,
+                                  const float* __restrict__ q_online_T, int B) {
   const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   float s_loss = 0.f, s_q = 0.f;
   if (n < num_samples) {
-    const float mx = q_row_max(q_next + n * A, A);
+    float mx;
+    if constexpr (Double) {
+      const int64_t m = n + B;                                           // sample (t + 1, b)
+      const float* online = m < num_samples ? q + m * A : q_online_T + (m - num_samples) * A;
+      mx = q_next[n * A + q_row_argmax(online, A)];
+    } else {
+      mx = q_row_max(q_next + n * A, A);
+    }
     const float r = fminf(fmaxf(rewards[n], rmin), rmax);                 // agent.py:154
     const float tgt = fmaf((1.0f - (terminals[n] ? 1.0f : 0.0f)) * discount, mx, r);   // agent.py:190
     const int a = actions[n];
@@ -367,22 +389,26 @@ __global__ void returns_lossgrad_kernel(const float* __restrict__ rewards,
 // ------------------------------- n-step Q loss gradients ----------------------------------
 // Asynchronous n-step Q-learning (Mnih et al. 2016): one thread per SAMPLE (t, b) as in
 // returns_lossgrad_kernel, the same return recurrence started from max_a Q(s_T; theta^-), then the
-// async-Q gradient of the acted action.
-template <bool Dueling>
+// async-Q gradient of the acted action.  Double: started from Q(s_T, a*; theta^-) with
+// a* = argmax_a Q(s_T, a; theta), the online row b of q_online_T (an argument after dvalue, as in
+// q_lossgrad_kernel).
+template <bool Dueling, bool Double>
 __global__ void nstep_q_lossgrad_kernel(const float* __restrict__ rewards,
                                         const uint8_t* __restrict__ terminals,
                                         const int32_t* __restrict__ actions, const float* __restrict__ q,
                                         const float* __restrict__ q_boot, float* __restrict__ returns,
                                         float* __restrict__ dq, float* __restrict__ loss_sums, int T, int B,
                                         int A, float gamma, float rmin, float rmax, float grad_scale,
-                                        float* __restrict__ dvalue) {
+                                        float* __restrict__ dvalue, const float* __restrict__ q_online_T) {
   const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   float s_loss = 0.f, s_q = 0.f;
   pdl_wait();
   if (n < (int64_t)T * B) {
     const int t = (int)(n / B), b = (int)(n - (int64_t)t * B);
-    const float R = nstep_return(rewards, terminals, q_row_max(q_boot + (size_t)b * A, A), t, T, B, b, gamma,
-                                 rmin, rmax);
+    float boot;
+    if constexpr (Double) boot = q_boot[(size_t)b * A + q_row_argmax(q_online_T + (size_t)b * A, A)];
+    else boot = q_row_max(q_boot + (size_t)b * A, A);
+    const float R = nstep_return(rewards, terminals, boot, t, T, B, b, gamma, rmin, rmax);
     returns[n] = R;
     const int a = actions[n];
     const float qa = q[n * A + a];
@@ -688,21 +714,24 @@ extern "C" int arl_egreedy_actions(const float* q, int32_t* actions, int num_env
   return ARL_OK;
 }
 
-// The Q loss entries: one launcher per learner for both head kinds (fn = the C entry's name, for errors)
-template <bool Dueling>
+// The Q loss entries: one launcher per learner for both head kinds and both targets (fn = the C
+// entry's name, for errors; q_online_T and num_envs: Double only)
+template <bool Dueling, bool Double = false>
 static int q_lossgrad(const char* fn, const float* rewards, const uint8_t* terminals, const int32_t* actions,
                       const float* q, const float* q_next, float* target, float* dq, float* dvalue,
                       float* loss_sums, int64_t num_samples, int action_size, float discount, float reward_min,
-                      float reward_max, float grad_scale, void* stream) {
-  ARL_REQUIRE(rewards && terminals && actions && q && q_next && target && dq && (dvalue || !Dueling),
+                      float reward_max, float grad_scale, void* stream, const float* q_online_T = nullptr,
+                      int num_envs = 0) {
+  ARL_REQUIRE(rewards && terminals && actions && q && q_next && target && dq && (dvalue || !Dueling) &&
+                  (q_online_T || !Double),
               "%s: null pointer", fn);
   ARL_REQUIRE(num_samples >= 0, "%s: negative size", fn);
   ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
               "%s: action_size %d outside [1,%d]", fn, action_size, ARL_MAX_ACTIONS);
   if (num_samples == 0) return ARL_OK;
-  q_lossgrad_kernel<Dueling><<<(unsigned)((num_samples + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+  q_lossgrad_kernel<Dueling, Double><<<(unsigned)((num_samples + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
       rewards, terminals, actions, q, q_next, target, dq, loss_sums, num_samples, action_size,
-      discount, reward_min, reward_max, grad_scale, dvalue);
+      discount, reward_min, reward_max, grad_scale, dvalue, q_online_T, num_envs);
   ARL_LAUNCH_CHECK("q_lossgrad_kernel");
   return ARL_OK;
 }
@@ -724,6 +753,40 @@ extern "C" int arl_q_lossgrad_dueling(const float* rewards, const uint8_t* termi
   return q_lossgrad<true>("arl_q_lossgrad_dueling", rewards, terminals, actions, q, q_next, target, dq, dvalue,
                           loss_sums, num_samples, action_size, discount, reward_min, reward_max, grad_scale,
                           stream);
+}
+
+// Double DQN targets (include/asyncrl_b200_double.h): t_max x num_envs samples, so that the kernel
+// knows which rows are the last step
+template <bool Dueling>
+static int double_q_lossgrad(const char* fn, const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                             const float* q, const float* q_next, const float* q_online_T, float* target, float* dq,
+                             float* dvalue, float* loss_sums, int t_max, int num_envs, int action_size,
+                             float discount, float reward_min, float reward_max, float grad_scale, void* stream) {
+  ARL_REQUIRE(t_max >= 0 && num_envs >= 0, "%s: negative size", fn);
+  return q_lossgrad<Dueling, true>(fn, rewards, terminals, actions, q, q_next, target, dq, dvalue, loss_sums,
+                                   (int64_t)t_max * num_envs, action_size, discount, reward_min, reward_max,
+                                   grad_scale, stream, q_online_T, num_envs);
+}
+
+extern "C" int arl_double_q_lossgrad(const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                                     const float* q, const float* q_next, const float* q_online_T, float* target,
+                                     float* dq, float* loss_sums, int t_max, int num_envs, int action_size,
+                                     float discount, float reward_min, float reward_max, float grad_scale,
+                                     void* stream) {
+  return double_q_lossgrad<false>("arl_double_q_lossgrad", rewards, terminals, actions, q, q_next, q_online_T,
+                                  target, dq, nullptr, loss_sums, t_max, num_envs, action_size, discount,
+                                  reward_min, reward_max, grad_scale, stream);
+}
+
+extern "C" int arl_double_q_lossgrad_dueling(const float* rewards, const uint8_t* terminals,
+                                             const int32_t* actions, const float* q, const float* q_next,
+                                             const float* q_online_T, float* target, float* dq, float* dvalue,
+                                             float* loss_sums, int t_max, int num_envs, int action_size,
+                                             float discount, float reward_min, float reward_max, float grad_scale,
+                                             void* stream) {
+  return double_q_lossgrad<true>("arl_double_q_lossgrad_dueling", rewards, terminals, actions, q, q_next,
+                                 q_online_T, target, dq, dvalue, loss_sums, t_max, num_envs, action_size, discount,
+                                 reward_min, reward_max, grad_scale, stream);
 }
 
 extern "C" int arl_returns_lossgrad(const float* rewards, const uint8_t* terminals,
@@ -748,21 +811,23 @@ extern "C" int arl_returns_lossgrad(const float* rewards, const uint8_t* termina
   return ARL_OK;
 }
 
-template <bool Dueling>
+template <bool Dueling, bool Double = false>
 static int nstep_q_lossgrad(const char* fn, const float* rewards, const uint8_t* terminals, const int32_t* actions,
                             const float* q, const float* q_boot, float* returns, float* dq, float* dvalue,
                             float* loss_sums, int t_max, int num_envs, int action_size, float gamma,
-                            float reward_min, float reward_max, float grad_scale, void* stream) {
-  ARL_REQUIRE(rewards && terminals && actions && q && q_boot && returns && dq && (dvalue || !Dueling),
+                            float reward_min, float reward_max, float grad_scale, void* stream,
+                            const float* q_online_T = nullptr) {
+  ARL_REQUIRE(rewards && terminals && actions && q && q_boot && returns && dq && (dvalue || !Dueling) &&
+                  (q_online_T || !Double),
               "%s: null pointer", fn);
   ARL_REQUIRE(t_max >= 0 && num_envs >= 0, "%s: negative size", fn);
   ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
               "%s: action_size %d outside [1,%d]", fn, action_size, ARL_MAX_ACTIONS);
   if (t_max == 0 || num_envs == 0) return ARL_OK;
   const int64_t total = (int64_t)t_max * num_envs;
-  ARL_CUDA(launch_pdl(nstep_q_lossgrad_kernel<Dueling>, dim3((unsigned)((total + 127) / 128)), dim3(128), 0,
-                      (cudaStream_t)stream, rewards, terminals, actions, q, q_boot, returns, dq, loss_sums, t_max,
-                      num_envs, action_size, gamma, reward_min, reward_max, grad_scale, dvalue));
+  ARL_CUDA(launch_pdl(nstep_q_lossgrad_kernel<Dueling, Double>, dim3((unsigned)((total + 127) / 128)), dim3(128),
+                      0, (cudaStream_t)stream, rewards, terminals, actions, q, q_boot, returns, dq, loss_sums, t_max,
+                      num_envs, action_size, gamma, reward_min, reward_max, grad_scale, dvalue, q_online_T));
   ARL_LAUNCH_CHECK("nstep_q_lossgrad_kernel");
   return ARL_OK;
 }
@@ -784,6 +849,27 @@ extern "C" int arl_nstep_q_lossgrad_dueling(const float* rewards, const uint8_t*
   return nstep_q_lossgrad<true>("arl_nstep_q_lossgrad_dueling", rewards, terminals, actions, q, q_boot, returns,
                                 dq, dvalue, loss_sums, t_max, num_envs, action_size, gamma, reward_min,
                                 reward_max, grad_scale, stream);
+}
+
+extern "C" int arl_double_nstep_q_lossgrad(const float* rewards, const uint8_t* terminals, const int32_t* actions,
+                                           const float* q, const float* q_boot, const float* q_online_T,
+                                           float* returns, float* dq, float* loss_sums, int t_max, int num_envs,
+                                           int action_size, float gamma, float reward_min, float reward_max,
+                                           float grad_scale, void* stream) {
+  return nstep_q_lossgrad<false, true>("arl_double_nstep_q_lossgrad", rewards, terminals, actions, q, q_boot,
+                                       returns, dq, nullptr, loss_sums, t_max, num_envs, action_size, gamma,
+                                       reward_min, reward_max, grad_scale, stream, q_online_T);
+}
+
+extern "C" int arl_double_nstep_q_lossgrad_dueling(const float* rewards, const uint8_t* terminals,
+                                                   const int32_t* actions, const float* q, const float* q_boot,
+                                                   const float* q_online_T, float* returns, float* dq,
+                                                   float* dvalue, float* loss_sums, int t_max, int num_envs,
+                                                   int action_size, float gamma, float reward_min, float reward_max,
+                                                   float grad_scale, void* stream) {
+  return nstep_q_lossgrad<true, true>("arl_double_nstep_q_lossgrad_dueling", rewards, terminals, actions, q,
+                                      q_boot, returns, dq, dvalue, loss_sums, t_max, num_envs, action_size, gamma,
+                                      reward_min, reward_max, grad_scale, stream, q_online_T);
 }
 
 template <bool Dueling>

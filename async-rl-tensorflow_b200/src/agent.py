@@ -46,6 +46,13 @@ class Agent(BaseModel):
         if self.dueling and getattr(config, 'loss_mode', 'a3c') == 'a3c':
             raise ValueError("dueling=True needs a Q learner (loss_mode 'async_q', 'nstep_q' or 'sarsa'); "
                              "loss_mode 'a3c' trains a policy/value network, which has no dueling form")
+        # config.py:35 double_q: Double DQN targets (van Hasselt et al. 2016) for the learners that
+        # bootstrap from a max; a3c has no max to decouple, sarsa bootstraps from the action taken in s'
+        self.double_q = bool(getattr(config, 'double_q', False))
+        if self.double_q and getattr(config, 'loss_mode', 'a3c') not in ('async_q', 'nstep_q'):
+            raise ValueError("double_q=True needs a learner that bootstraps from max_a Q (loss_mode 'async_q' or "
+                             "'nstep_q'); loss_mode %r has no max to decouple"
+                             % (getattr(config, 'loss_mode', 'a3c'),))
         # network.py:30-55: 'nips' (what agent.py:226-252 wires, the default) or 'nature'
         self.network = make_network(
             DQN_type=getattr(config, 'DQN_type', 'nips'), action_size=self.env.action_size, data_format=self.cnn_format,
@@ -53,7 +60,7 @@ class Agent(BaseModel):
             screen_width=self.screen_width, gamma=self.discount, beta=self.beta,
             num_envs=self.num_envs, t_max=self.t_max, device=self.device, seed=self.seed,
             decay=self.decay, epsilon=self.epsilon, clip_norm=self.clip_norm,
-            min_reward=self.min_reward, max_reward=self.max_reward, dueling=self.dueling)
+            min_reward=self.min_reward, max_reward=self.max_reward, dueling=self.dueling, double_q=self.double_q)
         self.w = self.network.w
         # the per-cycle exchange runs inside the library (arl_comm_init / arl_backward(allreduce=1):
         # NCCL, bucketed so that the fc256 gradient travels while the conv backward kernels run);

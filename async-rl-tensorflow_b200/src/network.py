@@ -90,12 +90,16 @@ class Network(object):
     # writes to ``policy_logits`` is v + (adv - mean adv), with p_w/p_b the advantage stream and q_w/q_b
     # the value stream; the Q losses then train both heads.  Fixed for the network's life.
     dueling = False
+    # double Q-learning targets (van Hasselt et al. 2016, include/asyncrl_b200_double.h): the async_q and
+    # nstep_q losses bootstrap from Q(s', a*; theta^-), a* = argmax_a Q(s'; theta); one more forward per
+    # update gives Q(s_T; theta) (``q_online_T``).  No parameter or stored state: fixed for the network's life.
+    double_q = False
 
     def __init__(self, sess=None, data_format='NHWC', history_length=4, screen_height=84,
                  screen_width=84, action_size=6, activation_fn='relu', initializer=None,
                  gamma=0.99, beta=0.01, global_network=None, global_optim=None, DQN_type='nips',
                  num_envs=256, t_max=5, device='cuda', seed=123, decay=0.99, epsilon=0.1,
-                 clip_norm=40.0, min_reward=-1.0, max_reward=1.0, dueling=False):
+                 clip_norm=40.0, min_reward=-1.0, max_reward=1.0, dueling=False, double_q=False):
         if DQN_type.lower() != 'nips':
             raise ValueError("Network is the 'nips' trunk (network.py:43-52); DQN_type='nature' "
                              "(network.py:30-42) is network_nature.NatureNetwork -- use "
@@ -115,6 +119,7 @@ class Network(object):
         self.min_reward, self.max_reward = float(min_reward), float(max_reward)
         self.global_network = global_network
         self.dueling = bool(dueling)
+        self.double_q = bool(double_q)
 
         A, B, T = self.action_size, self.num_envs, self.t_max
         self.offsets = _cabi.param_layout(A)
@@ -468,6 +473,9 @@ class Network(object):
         else:
             self.q_boot = torch.empty(B, A, **f32)            # Q(s_T; theta^-)
             self._target_fc_w_key = None
+        if self.double_q:                                     # Q(s_T; theta) + its probs / value scratch
+            self.q_online_T = torch.empty(B, A, **f32)
+            self._online_scratch = (torch.empty(B, A, **f32), torch.empty(B, **f32))
         self.target_fc_w = torch.empty(_cabi.prepared_floats(), device=self.device)
         return self.target_params
 
@@ -483,9 +491,26 @@ class Network(object):
                    int(env_id_base), int(step), int(seed), _cabi.stream_ptr())
         return self.sampled_action[r]
 
+    def _forward_online_T(self, history, refresh):
+        """Double Q: Q(s_T; theta) of the B current stacks into ``q_online_T`` under ``params`` / ``fc_w``
+        (rebuilt first when ``refresh``; None = decide from the parameter version), through the forward
+        every Q learner uses."""
+        P, b = _cabi.ptr, self._b
+        probs, value = self._online_scratch
+        refresh = self._refresh(refresh)
+        if self.dueling:
+            self._forward_dueling(self.params, self.fc_w, refresh, history, history.first_slot(0), 1, b['l1'],
+                                  b['l2'], b['l4'], self.q_online_T, probs, value)
+        else:
+            self._timed_call("arl_forward", P(self.params), P(self.fc_w), refresh, self.action_size,
+                             P(history.ring), self.num_envs, history.ring_slots, history.first_slot(0), 1,
+                             P(b['l1']), P(b['l2']), P(b['l4']), P(self.q_online_T), P(probs), P(value),
+                             _cabi.stream_ptr())
+
     def compute_q_gradients(self, history, rewards, terminals, grad_scale, allreduce=False):
         """agent.py:186-197: target-network forward over s_1..s_T, 1-step targets, MSE gradient,
-        backward.  The backward scratch buffers hold the target activations meanwhile."""
+        backward.  The backward scratch buffers hold the target activations meanwhile.  Double Q: the
+        online rows of s_1..s_{T-1} are the rollout's own Q rows, Q(s_T; theta) one more forward."""
         T, B, A = self.t_max, self.num_envs, self.action_size
         P, st = _cabi.ptr, _cabi.stream_ptr()
         probs, value = self._tq_scratch
@@ -496,12 +521,23 @@ class Network(object):
             _cabi.call("arl_forward", P(self.target_params), P(self.target_fc_w), 1, A, P(history.ring),
                        B, history.ring_slots, history.first_slot(T - 1), T, P(self.d_l1), P(self.d_l2),
                        P(self.d_l4), P(self.target_q), P(probs), P(value), st)
+        refresh = None
+        if self.double_q:
+            self._forward_online_T(history, None)
+            refresh = False                                    # fc_w: refreshed by the online forward
         self.loss_sums.zero_()
-        self._q_lossgrad("arl_q_lossgrad", (P(rewards), P(terminals), P(self.sampled_action), P(self.policy_logits),
-                                            P(self.target_q), P(self.target_q_t)),
-                         (P(self.loss_sums), T * B, A, self.gamma, self.min_reward, self.max_reward,
-                          float(grad_scale), st), timed=False)
-        return self._backward(history, grad_scale, allreduce, None)
+        if self.double_q:
+            self._q_lossgrad("arl_double_q_lossgrad", (P(rewards), P(terminals), P(self.sampled_action),
+                                                       P(self.policy_logits), P(self.target_q), P(self.q_online_T),
+                                                       P(self.target_q_t)),
+                             (P(self.loss_sums), T, B, A, self.gamma, self.min_reward, self.max_reward,
+                              float(grad_scale), st), timed=False)
+        else:
+            self._q_lossgrad("arl_q_lossgrad", (P(rewards), P(terminals), P(self.sampled_action),
+                                                P(self.policy_logits), P(self.target_q), P(self.target_q_t)),
+                             (P(self.loss_sums), T * B, A, self.gamma, self.min_reward, self.max_reward,
+                              float(grad_scale), st), timed=False)
+        return self._backward(history, grad_scale, allreduce, refresh)
 
     def _q_lossgrad(self, name, head, tail, timed=True):
         """A Q learner's loss entry ``name``: its arguments are ``head``, the dQ row (d_logits), ``tail``.
@@ -556,12 +592,16 @@ class Network(object):
         states s_T (into ``q_boot``, after rebuilding target_fc_w when ``target_refresh``; None =
         decide from the target's version), R_T = max_a q_boot, the n-step returns and dQ of the acted
         actions (arl_nstep_q_lossgrad), then the backward (agent.py:317).  ``history`` must have had
-        exactly t_max pushes since s_0."""
+        exactly t_max pushes since s_0.  Double Q: first the online forward of s_T (``q_online_T``,
+        with ``refresh``), and R_T = q_boot[a*], a* = argmax_a q_online_T (arl_double_nstep_q_lossgrad)."""
         T, B, A = self.t_max, self.num_envs, self.action_size
         P, st = _cabi.ptr, _cabi.stream_ptr()
         b = self._b
         if target_refresh is None:
             target_refresh = self._target_fc_w_stale()
+        if self.double_q:
+            self._forward_online_T(history, refresh)
+            refresh = False                                    # fc_w: refreshed by the online forward
         if self.dueling:
             self._forward_dueling(self.target_params, self.target_fc_w, target_refresh, history,
                                   history.first_slot(0), 1, b['l1'], b['l2'], b['l4'], self.q_boot, b['probs'],
@@ -571,6 +611,13 @@ class Network(object):
                              A, P(history.ring), B, history.ring_slots, history.first_slot(0), 1, P(b['l1']),
                              P(b['l2']), P(b['l4']), P(self.q_boot), P(b['probs']), P(b['value']), st)
         self.loss_sums.zero_()
+        if self.double_q:
+            self._q_lossgrad("arl_double_nstep_q_lossgrad", (P(rewards), P(terminals), P(self.sampled_action),
+                                                         P(self.policy_logits), P(self.q_boot), P(self.q_online_T),
+                                                         P(self.R)),
+                             (P(self.loss_sums), T, B, A, self.gamma, self.min_reward, self.max_reward,
+                              float(grad_scale), st))
+            return self._backward(history, grad_scale, allreduce, refresh)
         self._q_lossgrad("arl_nstep_q_lossgrad", (P(rewards), P(terminals), P(self.sampled_action),
                                                   P(self.policy_logits), P(self.q_boot), P(self.R)),
                          (P(self.loss_sums), T, B, A, self.gamma, self.min_reward, self.max_reward,
@@ -705,6 +752,9 @@ def make_network(DQN_type='nips', **kw):
         if kw.pop('dueling', False):
             raise NotImplementedError("dueling Q heads are built on the nips trunk (agent.py:226-252); the "
                                       "nature trunk is A3C-only")
+        if kw.pop('double_q', False):
+            raise NotImplementedError("double Q-learning targets are built on the nips trunk (agent.py:226-252); "
+                                      "the nature trunk is A3C-only")
         from .network_nature import NatureNetwork
         return NatureNetwork(DQN_type='nature', **kw)
     raise ValueError('Wrong DQN type: %s' % DQN_type)

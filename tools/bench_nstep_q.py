@@ -3,7 +3,7 @@ async_q eager (its own path: host epsilon, a separate draw launch, a target forw
 states; sarsa runs that target forward too, inside its graph).
 
     python tools/bench_nstep_q.py [--rounds R] [--cycles K] [--modes a3c,nstep_q,...] [--dueling off|on|both]
-                                  [--out FILE]
+                                  [--double off|on|both] [--out FILE]
 
 For each shape (envs x t_max x actions: 4096 x 5 x 6 and 16384 x 20 x 18) one agent per mode is built
 and warmed up until a whole ring period has replayed without a new graph capture; then the modes take
@@ -15,6 +15,8 @@ pool is larger than L2 at both shapes.
 
 --dueling on runs the Q learners with dueling Q heads (dueling=True; reported as "<mode>+dueling"),
 --dueling both runs every Q learner both ways, all of them alternating.
+--double on|both does the same with double Q-learning targets (double_q=True) for async_q and nstep_q,
+reported as "<mode>+double" or "<mode>+dueling+double".
 """
 import argparse
 import importlib
@@ -52,12 +54,15 @@ def main():
     ap.add_argument("--modes", default=",".join(MODES))
     ap.add_argument("--dueling", default="off", choices=("off", "on", "both"),
                     help="dueling Q heads for the Q learners: off, on, or both (each Q learner twice)")
-    ap.add_argument("--out", default=None, help="default: profiles/r05_sarsa_bench.json, or "
-                                                "profiles/r06_dueling_bench.json with --dueling on|both")
+    ap.add_argument("--double", default="off", choices=("off", "on", "both"),
+                    help="double Q-learning targets for async_q and nstep_q: off, on, or both")
+    ap.add_argument("--out", default=None, help="default: profiles/r05_sarsa_bench.json, "
+                                                "profiles/r06_dueling_bench.json with --dueling on|both, or "
+                                                "profiles/r08_double_q_bench.json with --double on|both")
     args = ap.parse_args()
     if args.out is None:
-        args.out = os.path.join(ROOT, "profiles", "r05_sarsa_bench.json" if args.dueling == "off"
-                                else "r06_dueling_bench.json")
+        args.out = os.path.join(ROOT, "profiles", "r08_double_q_bench.json" if args.double != "off"
+                                else "r05_sarsa_bench.json" if args.dueling == "off" else "r06_dueling_bench.json")
     if not torch.cuda.is_available():
         sys.exit("bench_nstep_q: needs a CUDA device")
     pkg = importlib.import_module("async-rl-tensorflow_b200")
@@ -65,10 +70,10 @@ def main():
     torch.cuda.set_device(dev)
     modes = []
     for m in args.modes.split(","):
-        if args.dueling != "on" or m == "a3c":
-            modes.append(m)
-        if args.dueling != "off" and m != "a3c":
-            modes.append(m + "+dueling")
+        heads = [""] if m == "a3c" else {"off": [""], "on": ["+dueling"], "both": ["", "+dueling"]}[args.dueling]
+        targets = ([""] if m not in ("async_q", "nstep_q")
+                   else {"off": [""], "on": ["+double"], "both": ["", "+double"]}[args.double])
+        modes += [m + h + d for h in heads for d in targets]
     result = {"card": card(), "rounds": args.rounds, "cycles_per_block": args.cycles, "shapes": []}
 
     for shape in args.shapes.split(","):
@@ -77,7 +82,7 @@ def main():
         agents = {}
         for mode in modes:
             cfg = pkg.config.get_config({"model": "m1", "num_envs": B, "t_max": T, "loss_mode": mode.split("+")[0],
-                                         "dueling": mode.endswith("+dueling")})
+                                         "dueling": "+dueling" in mode, "double_q": mode.endswith("+double")})
             env = pkg.GymEnvironment(cfg, env=pkg.SyntheticAtari(B, A, seed=123, pool=pool, device=dev), device=dev)
             agent = pkg.Agent(cfg, env, device=dev)
             random.seed(cfg.seed)
