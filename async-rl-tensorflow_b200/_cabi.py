@@ -1,5 +1,5 @@
 """ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h, include/asyncrl_b200_sarsa.h,
-include/asyncrl_b200_dueling.h, include/asyncrl_b200_double.h).
+include/asyncrl_b200_dueling.h, include/asyncrl_b200_double.h, include/asyncrl_b200_dueling_streams.h).
 
 The product path has no CPU fallback: if the shared library is missing or a call
 fails, this module raises.  PyTorch is only the carrier of device memory and
@@ -126,6 +126,25 @@ DOUBLE_SIGNATURES = {
                                             c_int, c_int, c_f32, c_f32, c_f32, c_f32, c_vp],
 }
 
+# the dueling streams (a hidden layer per stream): their own header (include/asyncrl_b200_dueling_streams.h),
+# their own tables
+STREAMS_SIGNATURES = {
+    "arl_streams_param_layout": [c_int, ctypes.POINTER(c_i64)],
+    "arl_prepare_weights_streams": [c_vp, c_vp, c_int, c_vp],
+    "arl_fc_forward_streams": [c_vp, c_vp, c_vp, c_i64, c_vp],
+    "arl_forward_streams": [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp,
+                            c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_u64, c_f32, ctypes.c_double, ctypes.c_double,
+                            ctypes.c_double, ctypes.c_double, c_vp],
+    "arl_heads_backward_streams": [c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_vp],
+    "arl_fc_backward_streams": [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_int, c_vp],
+    "arl_backward_streams": [c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                             c_vp, c_vp, c_vp, c_vp, c_f32, c_int, c_vp],
+}
+STREAMS_OTHER = {
+    "arl_streams_prepared_floats": ([], c_i64),
+    "arl_streams_workspace_bytes": ([c_int], c_i64),
+}
+
 
 class ArlError(RuntimeError):
     pass
@@ -145,10 +164,11 @@ def load():
                        "(or __graft_entry__.build()); there is no CPU fallback" % LIB_PATH)
     lib = ctypes.CDLL(LIB_PATH)
     for name, argtypes in (list(SIGNATURES.items()) + list(SARSA_SIGNATURES.items())
-                           + list(DUELING_SIGNATURES.items()) + list(DOUBLE_SIGNATURES.items())):
+                           + list(DUELING_SIGNATURES.items()) + list(DOUBLE_SIGNATURES.items())
+                           + list(STREAMS_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes, fn.restype = argtypes, c_int
-    for name, (argtypes, restype) in OTHER.items():
+    for name, (argtypes, restype) in list(OTHER.items()) + list(STREAMS_OTHER.items()):
         fn = getattr(lib, name)
         fn.argtypes, fn.restype = argtypes, restype
     _lib = lib
@@ -206,6 +226,14 @@ def nature_param_layout(action_size):
     return list(off)
 
 
+def streams_param_layout(action_size):
+    """Offsets (13) of the dueling streams' flat parameter buffer: arl_param_layout's 10 tensors, then la_w,
+    la_b."""
+    off = (c_i64 * 13)()
+    check(load().arl_streams_param_layout(int(action_size), off), "arl_streams_param_layout")
+    return list(off)
+
+
 def a2_block_rows(num_envs):
     """Rows of one a2 block (envs per forward launch): see arl_a2_block_rows."""
     return int(load().arl_a2_block_rows(int(num_envs)))
@@ -216,12 +244,17 @@ def launch_count(reset=False):
     return int(load().arl_launch_count(1 if reset else 0))
 
 
-def prepared_floats():
-    """Size (floats) of the prepared-weights buffer arl_prepare_weights fills."""
+def prepared_floats(streams=False):
+    """Size (floats) of the prepared-weights buffer arl_prepare_weights (``streams``:
+    arl_prepare_weights_streams) fills."""
+    if streams:
+        return int(load().arl_streams_prepared_floats())
     return int(load().arl_prepared_floats())
 
 
-def workspace_bytes(action_size):
+def workspace_bytes(action_size, streams=False):
+    if streams:
+        return int(load().arl_streams_workspace_bytes(int(action_size)))
     return int(load().arl_backward_workspace_bytes(int(action_size)))
 
 

@@ -5,6 +5,7 @@
 
 #include "common.cuh"
 #include "../../include/asyncrl_b200_dueling.h"
+#include "../../include/asyncrl_b200_dueling_streams.h"
 
 namespace arl {
 
@@ -105,11 +106,17 @@ template <class Draw, bool Dueling>
 int fc_heads_forward(const float* params, const float* prepared, int action_size, const float* a2, float* h,
                      float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base, int64_t step,
                      const int64_t* step_dev, uint64_t seed, int64_t num_samples, Draw draw, void* stream);
+template <class Draw>
+int fc_heads_forward_streams(const float* params, const float* prepared, int action_size, const float* a2, float* h,
+                             float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base,
+                             int64_t step, const int64_t* step_dev, uint64_t seed, int64_t num_samples, Draw draw,
+                             void* stream);
 }
 
 // One env step of the forward, env range by env range; `draw` is the action draw of the heads launch
-// (common.cuh: SampleDraw with actions == NULL draws nothing), Dueling the head kind (heads.cu)
-template <bool Dueling = false, class Draw>
+// (common.cuh: SampleDraw with actions == NULL draws nothing), Dueling the head kind (heads.cu),
+// Streams the dueling streams' network (h rows of 512)
+template <bool Dueling = false, class Draw, bool Streams = false>
 static int forward_step(const float* params, float* prepared, int action_size, const uint8_t* ring,
                         int num_envs, int ring_slots, int first_slot, float* a1, float* a2, float* h,
                         float* logits, float* probs, float* value, int32_t* actions, int64_t env_id_base,
@@ -119,17 +126,23 @@ static int forward_step(const float* params, float* prepared, int action_size, c
     const int n = num_envs - off < chunk ? num_envs - off : chunk;
     float* a1c = a1 + (size_t)off * 3200;                       // 12 800 bytes of fp16 per sample
     float* a2c = a2 + (size_t)off * ARL_A2_ELEMS;
-    float* hc = h + (size_t)off * ARL_FC;
+    float* hc = h + (size_t)off * (Streams ? 2 * ARL_FC : ARL_FC);
     int rc = arl_conv1_forward(prepared, ring + (size_t)off * ring_slots * kPlane, a1c, n, ring_slots,
                                first_slot, 1, stream);
     if (rc) return rc;
     rc = arl_conv2_forward(prepared, a1c, a2c, n, stream);
     if (rc) return rc;
     // fc256, then heads + softmax (+ the action draw) in one launch
-    rc = fc_heads_forward<Draw, Dueling>(params, prepared, action_size, a2c, hc, logits + (size_t)off * action_size,
-                                         probs + (size_t)off * action_size, value + off,
-                                         actions ? actions + off : nullptr, env_id_base + off, step, step_dev, seed,
-                                         n, draw, stream);
+    if constexpr (Streams)
+      rc = fc_heads_forward_streams<Draw>(params, prepared, action_size, a2c, hc, logits + (size_t)off * action_size,
+                                          probs + (size_t)off * action_size, value + off,
+                                          actions ? actions + off : nullptr, env_id_base + off, step, step_dev, seed,
+                                          n, draw, stream);
+    else
+      rc = fc_heads_forward<Draw, Dueling>(params, prepared, action_size, a2c, hc, logits + (size_t)off * action_size,
+                                           probs + (size_t)off * action_size, value + off,
+                                           actions ? actions + off : nullptr, env_id_base + off, step, step_dev, seed,
+                                           n, draw, stream);
     if (rc) return rc;
   }
   return ARL_OK;
@@ -287,4 +300,84 @@ extern "C" int arl_backward(const float* params, const float* prepared, int acti
   rc = arl_allreduce_begin(grads, 0, L.off[T_L4W], stream);        // l1_w .. l2_b
   if (rc) return rc;
   return arl_allreduce_end(stream);
+}
+
+// ---- dueling streams (include/asyncrl_b200_dueling_streams.h) ---------------------------------
+extern "C" int arl_streams_param_layout(int action_size, int64_t* offsets) {
+  ARL_REQUIRE(offsets, "arl_streams_param_layout: null pointer");
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_streams_param_layout: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
+  const StreamsLayout L = streams_layout(action_size);
+  memcpy(offsets, L.off, sizeof(L.off));
+  return ARL_OK;
+}
+
+extern "C" int64_t arl_streams_workspace_bytes(int action_size) {
+  // largest user: the fc weight-gradient split-K partials of both streams (8 x 2592 x 512 floats)
+  (void)action_size;
+  return (int64_t)8 * ARL_A2_ELEMS * 2 * ARL_FC * sizeof(float) + (1 << 20);
+}
+
+extern "C" int arl_forward_streams(const float* params, float* prepared, int refresh_prepared, int action_size,
+                                   const uint8_t* ring, int num_envs, int ring_slots, int first_slot, int steps,
+                                   float* a1, float* a2, float* h, float* logits, float* probs, float* value,
+                                   int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev,
+                                   uint64_t seed, float ep, double ep_start, double ep_end, double ep_end_t,
+                                   double learn_start, void* stream) {
+  int rc = ARL_OK;
+  if (actions != nullptr) {                       // one env step + the draw of arl_forward_egreedy
+    ARL_REQUIRE(steps == 1, "arl_forward_streams: the action draw needs steps == 1, got %d", steps);
+    rc = egreedy_args("arl_forward_streams", params, prepared, action_size, ring, a1, a2, h, logits, probs, value,
+                      actions, num_envs, env_id_base, step, step_dev, ep, ep_start, ep_end, ep_end_t);
+    if (rc || num_envs == 0) return rc;
+    if (refresh_prepared) rc = arl_prepare_weights_streams(params, prepared, action_size, stream);
+    if (rc) return rc;
+    return forward_step<true, EgreedyDraw, true>(params, prepared, action_size, ring, num_envs, ring_slots,
+                                                 first_slot, a1, a2, h, logits, probs, value, actions, env_id_base,
+                                                 step, step_dev, seed,
+                                                 EgreedyDraw{ep, ep_start, ep_end, ep_end_t, learn_start}, stream);
+  }
+  ARL_REQUIRE(params && prepared && ring && a1 && a2 && h && logits && probs && value,
+              "arl_forward_streams: null pointer");
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_forward_streams: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
+  ARL_REQUIRE(num_envs >= 0 && steps >= 0, "arl_forward_streams: negative size");
+  if (num_envs == 0 || steps == 0) return ARL_OK;
+  if (refresh_prepared) rc = arl_prepare_weights_streams(params, prepared, action_size, stream);
+  if (rc) return rc;
+  if (steps == 1)
+    return forward_step<true, SampleDraw, true>(params, prepared, action_size, ring, num_envs, ring_slots, first_slot,
+                                                a1, a2, h, logits, probs, value, nullptr, 0, 0, nullptr, 0,
+                                                SampleDraw{}, stream);
+  const int64_t N = (int64_t)num_envs * steps;
+  rc = arl_conv1_forward(prepared, ring, a1, num_envs, ring_slots, first_slot, steps, stream);
+  if (rc) return rc;
+  rc = arl_conv2_forward(prepared, a1, a2, N, stream);
+  if (rc) return rc;
+  return fc_heads_forward_streams<SampleDraw>(params, prepared, action_size, a2, h, logits, probs, value, nullptr, 0,
+                                              0, nullptr, 0, N, SampleDraw{}, stream);
+}
+
+// arl_backward with the streams' heads and fc256 backward; the conv backward and the exchange are
+// arl_backward's, over all 12 tensors
+extern "C" int arl_backward_streams(const float* params, const float* prepared, int action_size,
+                                    const uint8_t* ring, int num_envs, int ring_slots, int first_slot,
+                                    int steps, const float* a1, const float* a2, const float* h,
+                                    const float* dlogits, const float* dvalue, float* d_h, float* d_a2,
+                                    float* d_a1, float* grads, void* workspace, float tensor_scale,
+                                    int allreduce, void* stream) {
+  ARL_REQUIRE(tensor_scale > 0.f, "arl_backward_streams: tensor_scale must be > 0");
+  const int64_t N = (int64_t)num_envs * steps;
+  const float unscale = 1.0f / tensor_scale;
+  int rc = arl_heads_backward_streams(params, action_size, h, dlogits, dvalue, d_h, grads, workspace, N,
+                                      tensor_scale, stream);
+  if (rc) return rc;
+  rc = arl_fc_backward_streams(prepared, a2, arl_a2_block_rows(num_envs), d_h, d_a2, grads, workspace, N, unscale,
+                               action_size, stream);
+  if (rc) return rc;
+  rc = arl_conv2_backward(prepared, a1, d_a2, d_a1, grads, workspace, N, unscale, stream);
+  if (rc) return rc;
+  rc = arl_conv1_backward(ring, d_a1, grads, workspace, num_envs, ring_slots, first_slot, steps, unscale, stream);
+  if (rc || !(allreduce && arl_comm_size() > 1)) return rc;
+  return arl_allreduce_grads(grads, streams_layout(action_size).off[kStreamsTensors], stream);
 }

@@ -78,6 +78,29 @@ constexpr int64_t kPrepW2DBytes = 33024;
 constexpr int64_t kPrepFcWT = kPrepW2D + kPrepW2DBytes;           // l4_w TRANSPOSED as a split block [256 rows][2592]
 constexpr int64_t kPrepBytes = kPrepFcWT + kPrepFcWBytes;
 
+// Dueling streams (include/asyncrl_b200_dueling_streams.h): the advantage stream's hidden layer
+// la_w [2592,256], la_b [256] follows q_b; the ten tensors before it keep their offsets.
+enum { T_LAW = ARL_NUM_TENSORS, T_LAB };
+constexpr int kStreamsTensors = ARL_NUM_TENSORS + 2;
+struct StreamsLayout {
+  int64_t off[kStreamsTensors + 1];
+};
+inline StreamsLayout streams_layout(int A) {
+  const ParamLayout P = param_layout(A);
+  StreamsLayout L;
+  for (int i = 0; i <= ARL_NUM_TENSORS; ++i) L.off[i] = P.off[i];
+  L.off[T_LAW + 1] = L.off[T_LAW] + (int64_t)ARL_A2_ELEMS * ARL_FC;
+  L.off[T_LAB + 1] = L.off[T_LAB] + ARL_FC;
+  return L;
+}
+// The streams' prepared images: the plain ones at the plain offsets (kPrepFcW is not written), then
+constexpr int64_t kPrepLaWT = kPrepBytes;                         // la_w TRANSPOSED [256 rows][2592], right behind
+                                                                  // l4_w^T: the two read as ONE operand of 512 rows
+                                                                  // (a SplitMat of two blocks of 256 rows)
+constexpr int64_t kPrepSW = kPrepLaWT + kPrepFcWBytes;            // [l4_w | la_w] as one split block [2592 rows][512]
+constexpr int64_t kPrepSB = kPrepSW + 2 * kPrepFcWBytes;          // [l4_b | la_b], 512 floats
+constexpr int64_t kPrepStreamsBytes = kPrepSB + 2 * ARL_FC * 4;
+
 // Peer-memory exchange state (comm.cu): every rank's gradient slots and flag words mapped into this
 // process (CUDA IPC over NVLink); see arl_comm_enable_p2p.
 constexpr int kMaxRanks = 16;

@@ -371,6 +371,9 @@ struct PolicyBase {
   // custom_epilogue leaves each CTA's partial in its own shared memory and, after a cluster
   // barrier, cluster_reduce (epilogue warps) combines them through distributed shared memory
   static constexpr int CLUSTER = 1;
+  // MULTI_WAVE (CLUSTER > 1): still one work item per CTA, but the grid may exceed the SM count and
+  // run in several waves of clusters (launch() does not clamp it)
+  static constexpr bool MULTI_WAVE = false;
   template <class Args>
   static __device__ __forceinline__ void cluster_reduce(const Args&, uint8_t*, int, int) {}
   // CLUSTER_PHASES == 2: after another cluster barrier cluster_reduce2 (epilogue warps) may read what
@@ -759,7 +762,7 @@ int launch(const typename P::Args& g, int items, cudaStream_t stream) {
     attr_set.fetch_or(bit, std::memory_order_release);
   }
   if (items <= 0) return ARL_OK;
-  const int grid = items < num_sms() ? items : num_sms();
+  const int grid = items < num_sms() || (P::CLUSTER > 1 && P::MULTI_WAVE) ? items : num_sms();
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(cta_threads<P>());

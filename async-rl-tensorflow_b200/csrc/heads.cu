@@ -11,6 +11,7 @@
 #include "../../include/asyncrl_b200_sarsa.h"
 #include "../../include/asyncrl_b200_dueling.h"
 #include "../../include/asyncrl_b200_double.h"
+#include "../../include/asyncrl_b200_dueling_streams.h"
 
 namespace arl {
 
@@ -51,6 +52,8 @@ __device__ __forceinline__ void philox_two(uint32_t c0, uint32_t c1, uint32_t c2
 // EgreedyDraw).  Dueling (Wang et al. 2016, "average" aggregator) makes the A-wide head the advantage
 // stream and the 1-wide head the value stream: the row written to `logits` (and softmaxed into
 // `probs`, and drawn from) is then Q_j = v + (adv_j - mean_k adv_k); `value` is v either way.
+// Streams (dueling only): each stream has its own hidden layer, h is [N][512] = [h_v | h_a]; the
+// advantage head reads h_a, the value head h_v, and the rest is the dueling kernel's.
 
 // agent.py:142-144  ep_end + max(0., (ep_start - ep_end) * (ep_end_t - max(0., step - learn_start))
 // / ep_end_t), in double, one correctly rounded operation at a time in Python's order (the _rn
@@ -64,7 +67,7 @@ __device__ __forceinline__ float egreedy_epsilon(const EgreedyDraw& d, int64_t s
 }
 
 constexpr int kHfThreads = 256;
-template <class Draw, bool Dueling>
+template <class Draw, bool Dueling, bool Streams = false>
 __global__ void __launch_bounds__(kHfThreads)
 heads_fwd_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
                  const float* __restrict__ qw, const float* __restrict__ qb,
@@ -94,15 +97,21 @@ heads_fwd_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
   if constexpr (Draw::kEgreedy) ep = step_dev != nullptr ? egreedy_epsilon(draw, (int64_t)step) : draw.ep;
   const int64_t stride = (int64_t)gridDim.x * (kHfThreads / 32);
   for (int64_t n = (int64_t)blockIdx.x * (kHfThreads / 32) + warp; n < num_samples; n += stride) {
-    const float4* hp = reinterpret_cast<const float4*>(h + n * 256) + lane * 2;
+    const float4* hp = reinterpret_cast<const float4*>(h + n * (Streams ? 512 : 256) + (Streams ? 256 : 0)) + lane * 2;
     const float4 x0 = hp[0], x1 = hp[1];
+    float4 v0 = x0, v1 = x1;                       // the value head's input: h_v with Streams
+    if constexpr (Streams) {
+      const float4* vp = reinterpret_cast<const float4*>(h + n * 512) + lane * 2;
+      v0 = vp[0]; v1 = vp[1];
+    }
     float z = 0.f, zv = 0.f;
     for (int j = 0; j < J; ++j) {
       const float* w = sm + j * 256 + lane;
-      float a0 = x0.x * w[0], a1 = x0.y * w[32];
-      a0 = fmaf(x0.z, w[64], a0);  a1 = fmaf(x0.w, w[96], a1);
-      a0 = fmaf(x1.x, w[128], a0); a1 = fmaf(x1.y, w[160], a1);
-      a0 = fmaf(x1.z, w[192], a0); a1 = fmaf(x1.w, w[224], a1);
+      const float4 y0 = Streams && j == A ? v0 : x0, y1 = Streams && j == A ? v1 : x1;
+      float a0 = y0.x * w[0], a1 = y0.y * w[32];
+      a0 = fmaf(y0.z, w[64], a0);  a1 = fmaf(y0.w, w[96], a1);
+      a0 = fmaf(y1.x, w[128], a0); a1 = fmaf(y1.y, w[160], a1);
+      a0 = fmaf(y1.z, w[192], a0); a1 = fmaf(y1.w, w[224], a1);
       const float t = warp_sum(a0 + a1);           // every lane gets the total
       if (j == lane) z = t;
       if (j == A) zv = t;
@@ -560,6 +569,119 @@ heads_bwd_kernel(const float* __restrict__ pw, const float* __restrict__ qw,
   else if (k == A) out[256 * A + A + 256] = bacc;
 }
 
+// heads_bwd_kernel for the dueling streams: h [N][512] = [h_v | h_a]; the advantage head (p_w, j < A)
+// reads and feeds h_a, the value head (q_w, j = A) h_v.  d_h = [d_h_v | d_h_a] leaves as ONE split
+// block of 512 columns, twice, as there:
+//   dhs  [hi|lo][64 column chunks: 32 of d_h_v, then 32 of d_h_a][num_samples rows][8 columns]
+//   dhsT [hi|lo][ceil(N/8) sample chunks][512 column rows][8 samples]
+// 16 samples are staged per stream (two staging tiles of kHbSub rows would not fit 48 KB).
+constexpr int kHbSubS = 16;
+template <int JMAX>
+__global__ void __launch_bounds__(256, 1)
+heads_bwd_streams_kernel(const float* __restrict__ pw, const float* __restrict__ qw,
+                         const float* __restrict__ h, const float* __restrict__ dlogits,
+                         const float* __restrict__ dvalue, uint8_t* __restrict__ dhs,
+                         uint8_t* __restrict__ dhsT, float* __restrict__ partials, int64_t num_samples,
+                         int64_t per, int A, float tensor_scale) {
+  __shared__ float dzs[kHbChunk][JMAX];
+  __shared__ float dt[2][kHbSubS][257];               // [stream: 0 = v, 1 = a][sample][column]
+  const int J = A + 1;
+  const int k = threadIdx.x;
+  pdl_wait();
+  float w[JMAX], acc[JMAX];                          // the advantage head's columns (j < A)
+#pragma unroll
+  for (int j = 0; j < JMAX; ++j) {
+    w[j] = j < A ? pw[k * A + j] : 0.f;
+    acc[j] = 0.f;
+  }
+  const float wv = qw[k];                            // the value head's column
+  float accv = 0.f, bacc = 0.f;
+  const int64_t beg = per * blockIdx.x;
+  const int64_t end = beg + per < num_samples ? beg + per : num_samples;
+  const int64_t lo_part = (int64_t)64 * num_samples * 16;
+  const int64_t lo_partT = ((num_samples + 7) / 8) * 512 * 16;
+  for (int64_t c0 = beg; c0 < end; c0 += kHbChunk) {
+    const int nc = (int)(end - c0 < kHbChunk ? end - c0 : kHbChunk);
+    __syncthreads();
+    for (int i = k; i < nc * J; i += 256) {
+      const int s = i / J, j = i - s * J;
+      dzs[s][j] = j < A ? dlogits[(c0 + s) * A + j] : dvalue[c0 + s];
+    }
+    __syncthreads();
+    for (int s0 = 0; s0 < nc; s0 += kHbSubS) {
+      const int ns = nc - s0 < kHbSubS ? nc - s0 : kHbSubS;
+      float hvs[kHbSubS], has[kHbSubS];
+#pragma unroll
+      for (int s = 0; s < kHbSubS; ++s) {
+        hvs[s] = s < ns ? h[(c0 + s0 + s) * 512 + k] : 0.f;
+        has[s] = s < ns ? h[(c0 + s0 + s) * 512 + 256 + k] : 0.f;
+      }
+#pragma unroll
+      for (int s = 0; s < kHbSubS; ++s) {
+        if (s < ns) {
+          const float hv = hvs[s], ha = has[s];
+          float da = 0.f;
+#pragma unroll
+          for (int j = 0; j < JMAX; ++j) {
+            if (j < A) {
+              const float g = dzs[s0 + s][j];
+              da = fmaf(g, w[j], da);
+              acc[j] = fmaf(ha, g, acc[j]);
+            }
+          }
+          const float gv = dzs[s0 + s][A], dv = gv * wv;
+          accv = fmaf(hv, gv, accv);
+          dt[0][s][k] = hv > 0.f ? dv * tensor_scale : 0.f;     // d_h leaves scaled (arl_backward)
+          dt[1][s][k] = ha > 0.f ? da * tensor_scale : 0.f;
+        }
+      }
+      __syncthreads();
+      for (int v = k; v < 64 * kHbSubS; v += 256) {
+        const int s = v % kHbSubS, kc = v / kHbSubS;           // kc: chunk of [d_h_v | d_h_a]
+        if (s < ns) {
+          const float* x = &dt[kc >> 5][s][(kc & 31) * 8];
+          uint4 hi, lo;
+          tc_split2(x[0], x[1], hi.x, lo.x);
+          tc_split2(x[2], x[3], hi.y, lo.y);
+          tc_split2(x[4], x[5], hi.z, lo.z);
+          tc_split2(x[6], x[7], hi.w, lo.w);
+          uint8_t* d = dhs + ((int64_t)kc * num_samples + c0 + s0 + s) * 16;
+          *reinterpret_cast<uint4*>(d) = hi;
+          *reinterpret_cast<uint4*>(d + lo_part) = lo;
+        }
+      }
+      // transposed copy: thread k = column k of each stream and each of the (up to 2) sample chunks
+      for (int sc = 0; sc * 8 < ns; ++sc) {
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+          float x[8];
+#pragma unroll
+          for (int e = 0; e < 8; ++e) x[e] = sc * 8 + e < ns ? dt[q][sc * 8 + e][k] : 0.f;
+          uint4 hi, lo;
+          tc_split2(x[0], x[1], hi.x, lo.x);
+          tc_split2(x[2], x[3], hi.y, lo.y);
+          tc_split2(x[4], x[5], hi.z, lo.z);
+          tc_split2(x[6], x[7], hi.w, lo.w);
+          uint8_t* d = dhsT + (((c0 + s0) / 8 + sc) * 512 + q * 256 + k) * 16;
+          *reinterpret_cast<uint4*>(d) = hi;
+          *reinterpret_cast<uint4*>(d + lo_partT) = lo;
+        }
+      }
+      __syncthreads();
+    }
+    if (k < J)
+      for (int s = 0; s < nc; ++s) bacc += dzs[s][k];
+  }
+  float* out = partials + (size_t)blockIdx.x * (256 * J + J);
+  // layout of a partial: p_w [256][A] | p_b [A] | q_w [256] | q_b [1]  (flat-buffer order)
+#pragma unroll
+  for (int j = 0; j < JMAX; ++j)
+    if (j < A) out[k * A + j] = acc[j];
+  out[256 * A + A + k] = accv;
+  if (k < A) out[256 * A + k] = bacc;
+  else if (k == A) out[256 * A + A + 256] = bacc;
+}
+
 // ------------------------------- env-step bookkeeping --------------------------------------
 // GymEnvironment.act for action_repeat == 1 (environment.py:78-96): a life lost in training costs
 // one reward point and ends the episode.  One launch instead of five elementwise ones.
@@ -593,6 +715,10 @@ int heads_init() {
   ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<EgreedyDraw, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<SampleDraw, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<EgreedyDraw, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<SampleDraw, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                smem));
+  ARL_CUDA(cudaFuncSetAttribute(heads_fwd_kernel<EgreedyDraw, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                smem));
   return ARL_OK;
 }
 
@@ -604,8 +730,8 @@ static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 
 namespace arl {
 // heads + softmax + the draw; wait_first = 0 behind the fc256 kernel (fc_heads_forward), 1 stand-alone;
-// Dueling: the Q row of the dueling combine (heads_fwd_kernel)
-template <class Draw, bool Dueling>
+// Dueling: the Q row of the dueling combine (heads_fwd_kernel); Streams: h is [N][512] = [h_v | h_a]
+template <class Draw, bool Dueling, bool Streams = false>
 int heads_forward(const float* params, int action_size, const float* h, float* logits, float* probs, float* value,
                   int32_t* actions, int64_t env_id_base, int64_t step, const int64_t* step_dev, uint64_t seed,
                   int64_t num_samples, int wait_first, Draw draw, cudaStream_t st) {
@@ -615,7 +741,7 @@ int heads_forward(const float* params, int action_size, const float* h, float* l
   // up to 4 CTAs per SM: one env step of 4096 samples is ONE round of warps (two rounds cost a second
   // exposed load latency)
   const int grid = (int)(ctas < 4LL * num_sms() ? ctas : 4LL * num_sms());
-  ARL_CUDA(launch_pdl(heads_fwd_kernel<Draw, Dueling>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
+  ARL_CUDA(launch_pdl(heads_fwd_kernel<Draw, Dueling, Streams>, dim3(grid), dim3(kHfThreads), smem, st, params + L.off[T_PW],
                       params + L.off[T_PB], params + L.off[T_QW], params + L.off[T_QB], h, logits, probs, value,
                       num_samples, action_size, actions, (uint64_t)env_id_base, (uint64_t)step, seed, step_dev,
                       wait_first, draw));
@@ -634,6 +760,12 @@ template int heads_forward<SampleDraw, true>(const float*, int, const float*, fl
 template int heads_forward<EgreedyDraw, true>(const float*, int, const float*, float*, float*, float*, int32_t*,
                                              int64_t, int64_t, const int64_t*, uint64_t, int64_t, int, EgreedyDraw,
                                              cudaStream_t);
+template int heads_forward<SampleDraw, true, true>(const float*, int, const float*, float*, float*, float*, int32_t*,
+                                                  int64_t, int64_t, const int64_t*, uint64_t, int64_t, int,
+                                                  SampleDraw, cudaStream_t);
+template int heads_forward<EgreedyDraw, true, true>(const float*, int, const float*, float*, float*, float*,
+                                                   int32_t*, int64_t, int64_t, const int64_t*, uint64_t, int64_t, int,
+                                                   EgreedyDraw, cudaStream_t);
 }  // namespace arl
 
 extern "C" int arl_heads_forward(const float* params, int action_size, const float* h,
@@ -979,5 +1111,40 @@ extern "C" int arl_heads_backward(const float* params, int action_size, const fl
   ARL_CUDA(launch_pdl(kern, dim3(grid), dim3(256), 0, st, params + L.off[T_PW], params + L.off[T_QW], h, dlogits,
                       dvalue, dhs, dhsT, part, num_samples, per, A, tensor_scale));
   ARL_LAUNCH_CHECK("heads_bwd_kernel");
+  return reduce_partials(part, g, grid, 256 * J + J, st);
+}
+
+extern "C" int arl_heads_backward_streams(const float* params, int action_size, const float* h,
+                                          const float* dlogits, const float* dvalue, float* d_h,
+                                          float* grads, void* workspace, int64_t num_samples,
+                                          float tensor_scale, void* stream) {
+  ARL_REQUIRE(params && h && dlogits && dvalue && d_h && grads && workspace,
+              "arl_heads_backward_streams: null pointer");
+  ARL_REQUIRE(tensor_scale > 0.f, "arl_heads_backward_streams: tensor_scale must be > 0");
+  ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
+              "arl_heads_backward_streams: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
+  ARL_REQUIRE(num_samples >= 0, "arl_heads_backward_streams: negative size");
+  cudaStream_t st = (cudaStream_t)stream;
+  const ParamLayout L = param_layout(action_size);
+  const int A = action_size, J = A + 1;
+  float* g = grads + L.off[T_PW];
+  if (num_samples == 0) {
+    ARL_CUDA(cudaMemsetAsync(g, 0, (size_t)(256 * J + J) * sizeof(float), st));
+    return ARL_OK;
+  }
+  // arl_heads_backward's grid: whole sample chunks (8) per CTA, every CTA non-empty
+  int grid = 2 * num_sms();
+  if ((int64_t)grid > (num_samples + kHbChunk - 1) / kHbChunk)
+    grid = (int)((num_samples + kHbChunk - 1) / kHbChunk);
+  const int64_t per = ((num_samples + grid - 1) / grid + 7) / 8 * 8;
+  grid = (int)((num_samples + per - 1) / per);
+  float* part = (float*)workspace;
+  uint8_t* dhs = (uint8_t*)d_h;
+  uint8_t* dhsT = dhs + (size_t)num_samples * 512 * sizeof(float);
+  auto kern = J <= 8 ? heads_bwd_streams_kernel<8>
+                     : J <= 20 ? heads_bwd_streams_kernel<20> : heads_bwd_streams_kernel<ARL_MAX_ACTIONS + 1>;
+  ARL_CUDA(launch_pdl(kern, dim3(grid), dim3(256), 0, st, params + L.off[T_PW], params + L.off[T_QW], h, dlogits,
+                      dvalue, dhs, dhsT, part, num_samples, per, A, tensor_scale));
+  ARL_LAUNCH_CHECK("heads_bwd_streams_kernel");
   return reduce_partials(part, g, grid, 256 * J + J, st);
 }

@@ -75,6 +75,35 @@ int reduce_partials(const float* partials, float* out, int num_partials, int n,
   return reduce_partials_scaled(partials, out, num_partials, n, 1.0f, stream);
 }
 
+// reduce_partials_kernel's sums over partials [P][rows][2w], written as two matrices: columns < w to
+// out0 [rows][w], the others to out1 (the dueling streams' fc weight gradient: l4_w and la_w)
+__global__ void reduce_partials_cols_kernel(const float* __restrict__ partials, float* __restrict__ out0,
+                                            float* __restrict__ out1, int num_partials, int n, int w, float alpha) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  pdl_wait();
+  if (i >= n) return;
+  float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
+  int p = 0;
+  for (; p + 4 <= num_partials; p += 4) {
+    a0 += partials[(size_t)p * n + i];
+    a1 += partials[(size_t)(p + 1) * n + i];
+    a2 += partials[(size_t)(p + 2) * n + i];
+    a3 += partials[(size_t)(p + 3) * n + i];
+  }
+  for (; p < num_partials; ++p) a0 += partials[(size_t)p * n + i];
+  const int r = i / (2 * w), c = i - r * 2 * w;
+  (c < w ? out0 + (size_t)r * w + c : out1 + (size_t)r * w + (c - w))[0] = ((a0 + a1) + (a2 + a3)) * alpha;
+}
+
+int reduce_partials_cols(const float* partials, float* out0, float* out1, int num_partials, int rows, int w,
+                         float alpha, cudaStream_t stream) {
+  const int n = rows * 2 * w;
+  ARL_CUDA(launch_pdl(reduce_partials_cols_kernel, dim3((n + 255) / 256), dim3(256), 0, stream, partials, out0, out1,
+                      num_partials, n, w, alpha));
+  ARL_LAUNCH_CHECK("reduce_partials_cols_kernel");
+  return ARL_OK;
+}
+
 int conv_init() { return ARL_OK; }
 
 }  // namespace arl

@@ -46,6 +46,15 @@ class Agent(BaseModel):
         if self.dueling and getattr(config, 'loss_mode', 'a3c') == 'a3c':
             raise ValueError("dueling=True needs a Q learner (loss_mode 'async_q', 'nstep_q' or 'sarsa'); "
                              "loss_mode 'a3c' trains a policy/value network, which has no dueling form")
+        # config.py dueling_streams: the dueling architecture with a hidden layer per stream
+        # (Network.dueling_streams), an option of the dueling heads
+        self.dueling_streams = bool(getattr(config, 'dueling_streams', False))
+        if self.dueling_streams and getattr(config, 'loss_mode', 'a3c') == 'a3c':
+            raise ValueError("dueling_streams=True needs a Q learner (loss_mode 'async_q', 'nstep_q' or 'sarsa'); "
+                             "loss_mode 'a3c' trains a policy/value network, which has no dueling form")
+        if self.dueling_streams and not self.dueling:
+            raise ValueError("dueling_streams=True gives the dueling heads a hidden layer per stream; it needs "
+                             "dueling=True")
         # config.py:35 double_q: Double DQN targets (van Hasselt et al. 2016) for the learners that
         # bootstrap from a max; a3c has no max to decouple, sarsa bootstraps from the action taken in s'
         self.double_q = bool(getattr(config, 'double_q', False))
@@ -60,7 +69,8 @@ class Agent(BaseModel):
             screen_width=self.screen_width, gamma=self.discount, beta=self.beta,
             num_envs=self.num_envs, t_max=self.t_max, device=self.device, seed=self.seed,
             decay=self.decay, epsilon=self.epsilon, clip_norm=self.clip_norm,
-            min_reward=self.min_reward, max_reward=self.max_reward, dueling=self.dueling, double_q=self.double_q)
+            min_reward=self.min_reward, max_reward=self.max_reward, dueling=self.dueling, double_q=self.double_q,
+            dueling_streams=self.dueling_streams)
         self.w = self.network.w
         # the per-cycle exchange runs inside the library (arl_comm_init / arl_backward(allreduce=1):
         # NCCL, bucketed so that the fc256 gradient travels while the conv backward kernels run);

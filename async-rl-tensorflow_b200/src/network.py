@@ -17,6 +17,8 @@ import torch
 from .. import _cabi
 
 PARAM_NAMES = ("l1_w", "l1_b", "l2_w", "l2_b", "l4_w", "l4_b", "p_w", "p_b", "q_w", "q_b")
+# dueling streams (include/asyncrl_b200_dueling_streams.h): the advantage stream's hidden layer follows q_b
+STREAMS_PARAM_NAMES = PARAM_NAMES + ("la_w", "la_b")
 A1_ELEMS, A2_ELEMS, FC, DA1_ELEMS = 6400, 2592, 256, 7056
 A1_STORE = 3200                                               # float32 words of storage per sample of a1 (fp16)
 DA1_STORE = 3528                                              # ... of d_a1 (fp16 on the 21x21 grid)
@@ -61,19 +63,23 @@ def decode_da1(raw, n):
     return b.float().permute(1, 2, 3, 0, 4).reshape(n, 21, 21, 16)[:, :20, :20]
 
 
-def param_shapes(action_size):
-    return OrderedDict([
+def param_shapes(action_size, streams=False):
+    shapes = OrderedDict([
         ("l1_w", (8, 8, 4, 16)), ("l1_b", (16,)), ("l2_w", (4, 4, 16, 32)), ("l2_b", (32,)),
         ("l4_w", (A2_ELEMS, FC)), ("l4_b", (FC,)), ("p_w", (FC, action_size)),
         ("p_b", (action_size,)), ("q_w", (FC, 1)), ("q_b", (1,))])
+    if streams:
+        shapes["la_w"], shapes["la_b"] = (A2_ELEMS, FC), (FC,)
+    return shapes
 
 
-def initial_weights(action_size, seed=123, stddev=0.02):
+def initial_weights(action_size, seed=123, stddev=0.02, streams=False):
     """network.py:10 truncated_normal(0,.02) for convs, ops.py:36-39 normal(.02) for ``linear``
-    matrices, zero biases (ops.py:24,38-39).  Returns an OrderedDict of CPU float32 tensors."""
+    matrices, zero biases (ops.py:24,38-39).  Returns an OrderedDict of CPU float32 tensors.
+    ``streams``: la_w / la_b too, drawn after the others (a plain network's weights do not change)."""
     g = torch.Generator().manual_seed(int(seed))
     out = OrderedDict()
-    for name, shape in param_shapes(action_size).items():
+    for name, shape in param_shapes(action_size, streams).items():
         if name.endswith("_b"):
             out[name] = torch.zeros(shape)
         elif name in ("l1_w", "l2_w"):
@@ -94,12 +100,17 @@ class Network(object):
     # nstep_q losses bootstrap from Q(s', a*; theta^-), a* = argmax_a Q(s'; theta); one more forward per
     # update gives Q(s_T; theta) (``q_online_T``).  No parameter or stored state: fixed for the network's life.
     double_q = False
+    # dueling streams (Wang et al. 2016's architecture, include/asyncrl_b200_dueling_streams.h): with
+    # ``dueling``, each stream on its own fc256 layer on a2 -- l4_w/l4_b the value stream's, la_w/la_b
+    # (appended to the parameters) the advantage stream's; h (``l4``) is [N, 512] = [h_v | h_a].
+    dueling_streams = False
 
     def __init__(self, sess=None, data_format='NHWC', history_length=4, screen_height=84,
                  screen_width=84, action_size=6, activation_fn='relu', initializer=None,
                  gamma=0.99, beta=0.01, global_network=None, global_optim=None, DQN_type='nips',
                  num_envs=256, t_max=5, device='cuda', seed=123, decay=0.99, epsilon=0.1,
-                 clip_norm=40.0, min_reward=-1.0, max_reward=1.0, dueling=False, double_q=False):
+                 clip_norm=40.0, min_reward=-1.0, max_reward=1.0, dueling=False, double_q=False,
+                 dueling_streams=False):
         if DQN_type.lower() != 'nips':
             raise ValueError("Network is the 'nips' trunk (network.py:43-52); DQN_type='nature' "
                              "(network.py:30-42) is network_nature.NatureNetwork -- use "
@@ -120,31 +131,38 @@ class Network(object):
         self.global_network = global_network
         self.dueling = bool(dueling)
         self.double_q = bool(double_q)
+        self.dueling_streams = bool(dueling_streams)
+        if self.dueling_streams and not self.dueling:
+            raise ValueError("dueling_streams=True gives the dueling heads a hidden layer per stream; it needs "
+                             "dueling=True")
+        S = self.dueling_streams
+        self.param_names = STREAMS_PARAM_NAMES if S else PARAM_NAMES
 
         A, B, T = self.action_size, self.num_envs, self.t_max
-        self.offsets = _cabi.param_layout(A)
+        self.offsets = _cabi.streams_param_layout(A) if S else _cabi.param_layout(A)
         n_params = self.offsets[-1]
         dev = self.device
         self.params = torch.zeros(n_params, device=dev)
         self.grads = torch.zeros(n_params, device=dev)
         self.rms = torch.ones(n_params, device=dev)           # TF RMSProp slot starts at 1.0
         self.w, self.g = OrderedDict(), OrderedDict()
-        for i, (name, shape) in enumerate(param_shapes(A).items()):
+        for i, (name, shape) in enumerate(param_shapes(A, S).items()):
             self.w[name] = self.params[self.offsets[i]:self.offsets[i + 1]].view(shape)
             self.g[name] = self.grads[self.offsets[i]:self.offsets[i + 1]].view(shape)
         # the weights as the tensor-core kernels keep them resident (arl_prepare_weights); refreshed
         # lazily: the key is (tensor version, number of C-ABI writes) of the parameters it was made from
-        self.fc_w = torch.empty(_cabi.prepared_floats(), device=dev)
+        self.fc_w = torch.empty(_cabi.prepared_floats(S), device=dev)
         self._fc_w_key = None
         self._param_writes = 0
-        self.set_weights(initial_weights(A, seed))
+        self.set_weights(initial_weights(A, seed, streams=S))
+        H = 2 * FC if S else FC                               # width of h (streams: [h_v | h_a])
 
         N = B * T
         f32 = dict(device=dev, dtype=torch.float32)
         # rollout activations, t-major: sample n = t*B + b
         self.l1 = torch.empty(N, A1_STORE, **f32)             # network.py:47-48, stored as blocked fp16: see a1()
         self.l2 = torch.empty(N, A2_ELEMS, **f32)             # network.py:49-50 (flattened NHWC), one split block per step: see a2()
-        self.l4 = torch.empty(N, FC, **f32)                   # network.py:51-52
+        self.l4 = torch.empty(N, H, **f32)                    # network.py:51-52
         self.policy_logits = torch.empty(N, A, **f32)         # network.py:62
         self.policy = torch.empty(N, A, **f32)                # network.py:65
         self.value = torch.empty(N, **f32)                    # network.py:79
@@ -152,25 +170,25 @@ class Network(object):
         self.R = torch.empty(N, **f32)                        # network.py:82
         # bootstrap-state scratch (not kept for backward)
         self._b = dict(l1=torch.empty(B, A1_STORE, **f32), l2=torch.empty(B, A2_ELEMS, **f32),
-                       l4=torch.empty(B, FC, **f32), logits=torch.empty(B, A, **f32),
+                       l4=torch.empty(B, H, **f32), logits=torch.empty(B, A, **f32),
                        probs=torch.empty(B, A, **f32), value=torch.empty(B, **f32))
         # backward scratch
         self.d_logits = torch.empty(N, A, **f32)
         self.d_value = torch.empty(N, **f32)
         # d_h twice (include/asyncrl_b200.h): a split block of N rows, then its transposed copy
         # (groups of 8 samples x 256 columns) for the fc256 weight gradient: see d_h()
-        self.d_l4 = torch.empty(N + (N + 7) // 8 * 8, FC, **f32)
+        self.d_l4 = torch.empty(N + (N + 7) // 8 * 8, H, **f32)
         self.d_l2 = torch.empty(N, A2_ELEMS, **f32)
         self.d_l1 = torch.empty(N, DA1_STORE, **f32)          # fp16 on the 21x21 grid: see decode_da1
-        self.workspace = torch.empty(_cabi.workspace_bytes(A), dtype=torch.uint8, device=dev)
+        self.workspace = torch.empty(_cabi.workspace_bytes(A, S), dtype=torch.uint8, device=dev)
         self.loss_sums = torch.zeros(3, **f32)                # sum policy / value loss, entropy
-        self.grad_norms = torch.zeros(len(PARAM_NAMES), **f32)
+        self.grad_norms = torch.zeros(len(self.param_names), **f32)
         self.events = {}
         self.tensor_scale = 1.0                               # set by compute_gradients
 
     # -- parameters -----------------------------------------------------------------------
     def set_weights(self, weights):
-        for name in PARAM_NAMES:
+        for name in self.param_names:
             self.w[name].copy_(torch.as_tensor(np.asarray(weights[name]), dtype=torch.float32))
 
     def get_weights(self):
@@ -210,6 +228,14 @@ class Network(object):
         self._fc_w_key = key
         return stale
 
+    def _prepare(self, params, fc_w):
+        """Rebuild the prepared weight images ``fc_w`` from ``params``."""
+        P, st = _cabi.ptr, _cabi.stream_ptr()
+        if self.dueling_streams:
+            _cabi.call("arl_prepare_weights_streams", P(params), P(fc_w), self.action_size, st)
+        else:
+            _cabi.call("arl_prepare_weights", P(params), P(fc_w), st)
+
     def _refresh(self, refresh):
         """A ``refresh`` argument as the C-ABI's int, None decided from the parameter version."""
         return (1 if self._fc_w_stale() else 0) if refresh is None else int(bool(refresh))
@@ -230,17 +256,18 @@ class Network(object):
                        P(logits), P(probs), P(value), st)
             return
         if refresh:
-            _cabi.call("arl_prepare_weights", P(self.params), P(self.fc_w), st)
+            self._prepare(self.params, self.fc_w)
         self._timed_layers(history, l1, l2, l4, logits, probs, value, None, 0, 0, None, 0)
 
     def _forward_dueling(self, params, fc_w, refresh, history, first_slot, steps, l1, l2, l4, logits, probs, value,
                          actions=None, env_id_base=0, step=0, step_dev=None, seed=0, ep=0.0, ep_sched=None):
-        """arl_forward_dueling: ``steps`` env steps from ``first_slot`` under ``params`` with the dueling Q
-        row into ``logits``; with ``actions`` (one step) also the epsilon-greedy draw of
-        ``forward_egreedy``.  One entry under ``timed``."""
+        """arl_forward_dueling (arl_forward_streams with ``dueling_streams``): ``steps`` env steps from
+        ``first_slot`` under ``params`` with the dueling Q row into ``logits``; with ``actions`` (one step)
+        also the epsilon-greedy draw of ``forward_egreedy``.  One entry under ``timed``."""
         P = _cabi.ptr
         e0, e1, et, ls = (float(x) for x in (ep_sched if ep_sched is not None else (0.0, 0.0, 1.0, 0.0)))
-        self._timed_call("arl_forward_dueling", P(params), P(fc_w), int(bool(refresh)), self.action_size,
+        entry = "arl_forward_streams" if self.dueling_streams else "arl_forward_dueling"
+        self._timed_call(entry, P(params), P(fc_w), int(bool(refresh)), self.action_size,
                          P(history.ring), self.num_envs, history.ring_slots, first_slot, steps, P(l1), P(l2), P(l4),
                          P(logits), P(probs), P(value), P(actions), int(env_id_base), int(step), P(step_dev),
                          int(seed), float(ep), e0, e1, et, ls, _cabi.stream_ptr())
@@ -313,9 +340,10 @@ class Network(object):
         return float(2.0 ** max(-20, min(40, e)))
 
     def d_h(self):
-        """Gradient w.r.t. the fc256 output of the last backward as float32 [N,256]."""
+        """Gradient w.r.t. the fc256 output of the last backward as float32 [N,256] ([N,512] =
+        [d_h_v | d_h_a] with ``dueling_streams``)."""
         N = self.num_envs * self.t_max
-        return decode_split(self.d_l4[:N], N, FC) / self.tensor_scale
+        return decode_split(self.d_l4[:N], N, self.l4.shape[1]) / self.tensor_scale
 
     def d_a2(self):
         """Gradient w.r.t. the conv2 output (pre-relu) of the last backward, float32 [N,2592]."""
@@ -328,9 +356,9 @@ class Network(object):
     def d_h_transposed(self):
         """The same gradient decoded from its second, transposed copy (what fc wgrad reads)."""
         N = self.num_envs * self.t_max
-        n8 = (N + 7) // 8 * 8
-        b = self.d_l4[N:].reshape(-1).view(torch.bfloat16).reshape(2, n8 // 8, FC, 8)
-        return (b[0].float() + b[1].float()).permute(0, 2, 1).reshape(n8, FC)[:N] / self.tensor_scale
+        n8, H = (N + 7) // 8 * 8, self.l4.shape[1]
+        b = self.d_l4[N:].reshape(-1).view(torch.bfloat16).reshape(2, n8 // 8, H, 8)
+        return (b[0].float() + b[1].float()).permute(0, 2, 1).reshape(n8, H)[:N] / self.tensor_scale
 
     def sample(self, t, step, seed, env_id_base=0):
         """network.py:72-73 sampled_action for rollout slot t."""
@@ -421,8 +449,14 @@ class Network(object):
         T, B, A = self.t_max, self.num_envs, self.action_size
         P, st = _cabi.ptr, _cabi.stream_ptr()
         if self._refresh(refresh):
-            _cabi.call("arl_prepare_weights", P(self.params), P(self.fc_w), st)
+            self._prepare(self.params, self.fc_w)
         S = self.tensor_scale = self.pick_tensor_scale(grad_scale)
+        if self.dueling_streams:                               # one entry, the exchange inside
+            self._timed_call("arl_backward_streams", P(self.params), P(self.fc_w), A, P(history.ring), B,
+                             history.ring_slots, history.first_slot(T), T, P(self.l1), P(self.l2), P(self.l4),
+                             P(self.d_logits), P(self.d_value), P(self.d_l4), P(self.d_l2), P(self.d_l1),
+                             P(self.grads), P(self.workspace), S, 1 if allreduce else 0, st)
+            return self.grads
         if self.timed is None:
             _cabi.call("arl_backward", P(self.params), P(self.fc_w), A, P(history.ring), B,
                        history.ring_slots, history.first_slot(T), T, P(self.l1), P(self.l2),
@@ -476,7 +510,7 @@ class Network(object):
         if self.double_q:                                     # Q(s_T; theta) + its probs / value scratch
             self.q_online_T = torch.empty(B, A, **f32)
             self._online_scratch = (torch.empty(B, A, **f32), torch.empty(B, **f32))
-        self.target_fc_w = torch.empty(_cabi.prepared_floats(), device=self.device)
+        self.target_fc_w = torch.empty(_cabi.prepared_floats(self.dueling_streams), device=self.device)
         return self.target_params
 
     def update_target(self):
@@ -685,11 +719,24 @@ class Network(object):
                          float(base_lr), int(max_step), self.decay, self.epsilon, self.clip_norm,
                          _cabi.ptr(self.grad_norms), _cabi.ptr(self.workspace), _cabi.stream_ptr())
 
+    def _layout_update(self, lr, step_dev, step_offset, base_lr, max_step):
+        """K5 over the tensors of ``offsets`` (arl_clip_rmsprop_layout): the dueling streams' 12 tensors."""
+        import ctypes
+        if not hasattr(self, '_offsets_c'):
+            self._offsets_c = (ctypes.c_int64 * len(self.offsets))(*self.offsets)
+        self._timed_call("arl_clip_rmsprop_layout", _cabi.ptr(self.params), _cabi.ptr(self.rms),
+                         _cabi.ptr(self.grads), self._offsets_c, len(self.offsets) - 1, float(lr),
+                         _cabi.ptr(step_dev) if step_dev is not None else None, int(step_offset),
+                         float(base_lr), int(max_step), self.decay, self.epsilon, self.clip_norm,
+                         _cabi.ptr(self.grad_norms), _cabi.ptr(self.workspace), _cabi.stream_ptr())
+
     def apply_gradients(self, lr, exchange=False):
         """agent.py:316-321: per-tensor clip_by_norm(40) + shared RMSProp (K5).  ``exchange``: sum
         the gradient over the ranks first, inside the same kernels (NVLink peer memory)."""
         if exchange:
             self._exchange_update(lr, None, 0, 0.0, 1)
+        elif self.dueling_streams:
+            self._layout_update(lr, None, 0, 0.0, 1)
         else:
             self._timed_call("arl_clip_rmsprop", _cabi.ptr(self.params), _cabi.ptr(self.rms),
                              _cabi.ptr(self.grads), self.action_size, float(lr), self.decay, self.epsilon,
@@ -703,6 +750,8 @@ class Network(object):
         from the int64 step counter ``step_dev`` (+ ``step_offset``): replayable by a CUDA graph."""
         if exchange:
             self._exchange_update(0.0, step_dev, step_offset, base_lr, max_step)
+        elif self.dueling_streams:
+            self._layout_update(0.0, step_dev, step_offset, base_lr, max_step)
         else:
             self._timed_call("arl_clip_rmsprop_sched", _cabi.ptr(self.params), _cabi.ptr(self.rms),
                              _cabi.ptr(self.grads), self.action_size, _cabi.ptr(step_dev), int(step_offset),
@@ -720,6 +769,8 @@ class Network(object):
         blobs["step"] = np.int64(step if step is not None else 0)
         if self.dueling:                                       # absent = not dueling: older files load as such
             blobs["dueling"] = np.bool_(True)
+        if self.dueling_streams:                               # absent = no hidden layer per stream
+            blobs["dueling_streams"] = np.bool_(True)
         np.savez(path, **blobs)
         return path
 
@@ -736,7 +787,12 @@ class Network(object):
             raise ValueError("checkpoint %s was written by a %s network; this network is %s"
                              % (files[-1], "dueling" if saved else "non-dueling",
                                 "dueling" if self.dueling else "non-dueling"))
-        self.set_weights({k: z[k] for k in PARAM_NAMES})
+        saved = bool(z["dueling_streams"]) if "dueling_streams" in z.files else False
+        if saved != self.dueling_streams:                      # other parameters: refuse
+            raise ValueError("checkpoint %s was written by a %s network; this network is %s"
+                             % (files[-1], "dueling_streams" if saved else "non-dueling_streams",
+                                "dueling_streams" if self.dueling_streams else "non-dueling_streams"))
+        self.set_weights({k: z[k] for k in self.param_names})
         self.rms.copy_(torch.as_tensor(z["rms"]))
         self.loaded_step = int(z["step"])
         return True
@@ -751,6 +807,9 @@ def make_network(DQN_type='nips', **kw):
     if kind == 'nature':
         if kw.pop('dueling', False):
             raise NotImplementedError("dueling Q heads are built on the nips trunk (agent.py:226-252); the "
+                                      "nature trunk is A3C-only")
+        if kw.pop('dueling_streams', False):
+            raise NotImplementedError("dueling streams are built on the nips trunk (agent.py:226-252); the "
                                       "nature trunk is A3C-only")
         if kw.pop('double_q', False):
             raise NotImplementedError("double Q-learning targets are built on the nips trunk (agent.py:226-252); "

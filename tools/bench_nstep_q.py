@@ -3,7 +3,7 @@ async_q eager (its own path: host epsilon, a separate draw launch, a target forw
 states; sarsa runs that target forward too, inside its graph).
 
     python tools/bench_nstep_q.py [--rounds R] [--cycles K] [--modes a3c,nstep_q,...] [--dueling off|on|both]
-                                  [--double off|on|both] [--out FILE]
+                                  [--double off|on|both] [--dueling-streams off|on|both] [--out FILE]
 
 For each shape (envs x t_max x actions: 4096 x 5 x 6 and 16384 x 20 x 18) one agent per mode is built
 and warmed up until a whole ring period has replayed without a new graph capture; then the modes take
@@ -56,12 +56,17 @@ def main():
                     help="dueling Q heads for the Q learners: off, on, or both (each Q learner twice)")
     ap.add_argument("--double", default="off", choices=("off", "on", "both"),
                     help="double Q-learning targets for async_q and nstep_q: off, on, or both")
+    ap.add_argument("--dueling-streams", default="off", choices=("off", "on", "both"),
+                    help="a hidden layer per dueling stream (reported as \"<mode>+streams\"): off, on, or both "
+                         "(each Q learner plain, with dueling heads and with dueling streams)")
     ap.add_argument("--out", default=None, help="default: profiles/r05_sarsa_bench.json, "
-                                                "profiles/r06_dueling_bench.json with --dueling on|both, or "
-                                                "profiles/r08_double_q_bench.json with --double on|both")
+                                                "profiles/r06_dueling_bench.json with --dueling on|both, "
+                                                "profiles/r08_double_q_bench.json with --double on|both, or "
+                                                "profiles/r09_dueling_streams_bench.json with --dueling-streams on|both")
     args = ap.parse_args()
     if args.out is None:
-        args.out = os.path.join(ROOT, "profiles", "r08_double_q_bench.json" if args.double != "off"
+        args.out = os.path.join(ROOT, "profiles", "r09_dueling_streams_bench.json" if args.dueling_streams != "off"
+                                else "r08_double_q_bench.json" if args.double != "off"
                                 else "r05_sarsa_bench.json" if args.dueling == "off" else "r06_dueling_bench.json")
     if not torch.cuda.is_available():
         sys.exit("bench_nstep_q: needs a CUDA device")
@@ -71,6 +76,8 @@ def main():
     modes = []
     for m in args.modes.split(","):
         heads = [""] if m == "a3c" else {"off": [""], "on": ["+dueling"], "both": ["", "+dueling"]}[args.dueling]
+        if m != "a3c" and args.dueling_streams != "off":
+            heads = {"on": ["+streams"], "both": ["", "+dueling", "+streams"]}[args.dueling_streams]
         targets = ([""] if m not in ("async_q", "nstep_q")
                    else {"off": [""], "on": ["+double"], "both": ["", "+double"]}[args.double])
         modes += [m + h + d for h in heads for d in targets]
@@ -82,7 +89,8 @@ def main():
         agents = {}
         for mode in modes:
             cfg = pkg.config.get_config({"model": "m1", "num_envs": B, "t_max": T, "loss_mode": mode.split("+")[0],
-                                         "dueling": "+dueling" in mode, "double_q": mode.endswith("+double")})
+                                         "dueling": "+dueling" in mode or "+streams" in mode,
+                                         "dueling_streams": "+streams" in mode, "double_q": mode.endswith("+double")})
             env = pkg.GymEnvironment(cfg, env=pkg.SyntheticAtari(B, A, seed=123, pool=pool, device=dev), device=dev)
             agent = pkg.Agent(cfg, env, device=dev)
             random.seed(cfg.seed)
