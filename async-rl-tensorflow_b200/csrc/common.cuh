@@ -191,6 +191,23 @@ __device__ __forceinline__ void bulk_s2g(void* dst_gmem, const void* src_smem, u
                "r"(smem_u32(src_smem)), "r"(bytes)
                : "memory");
 }
+// L2 eviction priority of the lines a copy touches, as a 64-bit cache policy for bulk_g2s_hint.
+// evict_first: data read once (K1's frames) goes first, so a stream of it does not push out the
+// lines the next kernels re-read or the dirty lines of the previous ones.
+__device__ __forceinline__ uint64_t l2_policy_evict_first() {
+  uint64_t p;
+  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
+  return p;
+}
+// bulk_g2s with an L2 cache policy (SASS: UBLKCP with a desc[UR] policy operand)
+__device__ __forceinline__ void bulk_g2s_hint(void* dst_smem, const void* src_gmem, uint32_t bytes,
+                                              uint64_t* bar, uint64_t policy) {
+  asm volatile(
+      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
+      " [%0], [%1], %2, [%3], %4;" ::"r"(smem_u32(dst_smem)),
+      "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
+      : "memory");
+}
 __device__ __forceinline__ void bulk_commit() {
   asm volatile("cp.async.bulk.commit_group;" ::: "memory");
 }

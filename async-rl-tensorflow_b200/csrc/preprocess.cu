@@ -3,7 +3,7 @@
 // expression, truncated) -> cv2 INTER_LINEAR 84x84 (fixed point) -> ring slot.
 //
 // Layout / data flow per frame (one persistent CTA per SM, every compute warp a 2-stage bulk-copy pipeline):
-//   HBM --cp.async.bulk (43 copies: the 168 source rows cv2 actually reads)--> smem raw[stage]
+//   HBM --cp.async.bulk (43 copies: the 168 source rows cv2 actually reads; L2 evict_first up to 8192 frames)--> smem raw[stage]
 //   raw --luma, 8 px / lane-iteration, dp2a--> smem Y [168][160] u8 (8 rows private to a warp)
 //   Y   --dp2a x taps, packed vertical terms--> smem out[ob] [84*84] u8 --cp.async.bulk--> ring[b][slot]
 // Algorithmic HBM bytes per frame: 80 640 read + 7 056 written (x replicate).
@@ -78,6 +78,13 @@ static void linear_taps(int src, int dst, uint32_t* packed) {
 //                 iterations) into its private Y slice, then its 4 x 84 outputs.
 //   store warp  : the 7056-B plane store(s) out[ob] -> ring (out_full/out_empty mbarriers).
 constexpr int kComputeWarps = kS / 4;                       // 21
+// Up to this many frames per launch K1 loads them with an L2 evict_first policy.  The forward
+// kernels before it leave ~100 MB of dirty lines in the 126 MB L2 whatever the batch; streaming the
+// frames past them moves that write-back into the forward kernels, which have DRAM bandwidth to
+// spare.  On a B200 at 1000 W: 82 -> 71 us per launch at 4096 frames, 137 -> 129 us at 8192.  At
+// 16 384 frames the hint cost K1 1-4 us per launch at t_max 20 on a power-capped card (268 -> 271 us,
+// cycle +0.4 %), so launches that long load as before.  DESIGN.md §3.1.
+constexpr int kK1EvictFirstMaxEnvs = 8192;
 constexpr int kK1Threads = (kComputeWarps + 1) * 32;        // 704
 
 struct __align__(16) K1Smem {
@@ -145,6 +152,8 @@ __device__ __forceinline__ uint2 luma_8px(const uint32_t (&w)[6], const LumaCoef
                     __byte_perm(__byte_perm(h[4], h[5], 0x0062), __byte_perm(h[6], h[7], 0x0062), 0x5410));
 }
 
+// kEvictFirst: the frame loads carry an L2 evict_first policy (arl_preprocess_push picks it by batch size)
+template <bool kEvictFirst>
 __global__ void __launch_bounds__(kK1Threads, 1)
 preprocess_kernel(const uint8_t* __restrict__ frames, uint8_t* __restrict__ ring, int num_envs,
                   int ring_slots, int slot, int replicate) {
@@ -156,18 +165,26 @@ preprocess_kernel(const uint8_t* __restrict__ frames, uint8_t* __restrict__ ring
   // A compute warp's load barriers are private to it: lane 0 initialises them and issues the
   // copies of its first two frames before anything else happens in the CTA (the 8-KB correction
   // bitmap and the output barriers are set up while those copies are in flight).
+  // The frames are read once per step: evict_first lets their stream pass through L2 without
+  // evicting the previous kernels' dirty lines (whose write-back would then fall into this kernel)
+  // or the ring planes the next kernel reads.
   auto issue_loads = [&](int f) {                               // lane 0 of a compute warp only
     const int stage = f & 1;
     uint64_t* bar = &sm.full[stage][warp];
     mbar_expect_tx(bar, 4 * kPairBytes);
+    const uint64_t once = kEvictFirst ? l2_policy_evict_first() : 0;
+    auto load = [&](uint8_t* dst, const uint8_t* src, uint32_t bytes) {
+      if (kEvictFirst) bulk_g2s_hint(dst, src, bytes, bar, once);
+      else bulk_g2s(dst, src, bytes, bar);
+    };
     const uint8_t* src = frames + (size_t)(blockIdx.x + (size_t)f * gridDim.x) * kFrameBytes;
     uint8_t* dst = sm.raw[stage] + warp * (4 * kPairBytes);
-    bulk_g2s(dst, src + (10 * warp + 3) * kRowBytes, 2 * kPairBytes, bar);
+    load(dst, src + (10 * warp + 3) * kRowBytes, 2 * kPairBytes);
     if (warp < kComputeWarps - 1) {
-      bulk_g2s(dst + 2 * kPairBytes, src + (10 * warp + 8) * kRowBytes, 2 * kPairBytes, bar);
+      load(dst + 2 * kPairBytes, src + (10 * warp + 8) * kRowBytes, 2 * kPairBytes);
     } else {
-      bulk_g2s(dst + 2 * kPairBytes, src + (kH - 2) * kRowBytes, kPairBytes, bar);
-      bulk_g2s(dst + 3 * kPairBytes, src, kPairBytes, bar);
+      load(dst + 2 * kPairBytes, src + (kH - 2) * kRowBytes, kPairBytes);
+      load(dst + 3 * kPairBytes, src, kPairBytes);
     }
   };
   if (warp < kComputeWarps && lane == 0) {
@@ -369,8 +386,10 @@ preprocess_pil_kernel(const uint8_t* __restrict__ frames, uint8_t* __restrict__ 
       bulk_wait_read<0>();                                    // previous plane store has read sm.out
       mbar_expect_tx(&sm.full, kFrameBytes);
       const uint8_t* src = frames + (size_t)env * kFrameBytes;
+      const uint64_t once = l2_policy_evict_first();          // frames are read once (see issue_loads)
       for (int c = 0; c < 4; ++c)                             // 4 x 25 200 B
-        bulk_g2s(sm.raw + c * (kFrameBytes / 4), src + c * (kFrameBytes / 4), kFrameBytes / 4, &sm.full);
+        bulk_g2s_hint(sm.raw + c * (kFrameBytes / 4), src + c * (kFrameBytes / 4), kFrameBytes / 4, &sm.full,
+                      once);
     }
     mbar_wait(&sm.full, it & 1);
     // luma of all 210 x 160 pixels, 8 per thread-iteration
@@ -480,7 +499,9 @@ int preprocess_init(int device) {
   ARL_CUDA(cudaMemset(fix, 0, sizeof(uint32_t) * kBitmapWords));
   luma_fix_init_kernel<<<65536 / 256, 256>>>();
   ARL_LAUNCH_CHECK("luma_fix_init_kernel");
-  ARL_CUDA(cudaFuncSetAttribute(preprocess_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  ARL_CUDA(cudaFuncSetAttribute(preprocess_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)sizeof(K1Smem)));
+  ARL_CUDA(cudaFuncSetAttribute(preprocess_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)sizeof(K1Smem)));
   {
     static PilTaps pt;
@@ -516,7 +537,8 @@ extern "C" int arl_preprocess_push(const uint8_t* frames, uint8_t* ring, int num
               "arl_preprocess_push: frames and ring must be 16-byte aligned");
   if (num_envs == 0) return ARL_OK;
   const int grid = num_envs < num_sms() ? num_envs : num_sms();
-  ARL_CUDA(launch_pdl(preprocess_kernel, dim3(grid), dim3(kK1Threads), sizeof(K1Smem), (cudaStream_t)stream,
+  ARL_CUDA(launch_pdl(num_envs <= kK1EvictFirstMaxEnvs ? preprocess_kernel<true> : preprocess_kernel<false>,
+                      dim3(grid), dim3(kK1Threads), sizeof(K1Smem), (cudaStream_t)stream,
                       frames, ring, num_envs, ring_slots, slot, replicate));
   ARL_LAUNCH_CHECK("preprocess_kernel");
   return ARL_OK;
