@@ -1,5 +1,6 @@
 """ctypes binding of libasyncrl_b200.so (include/asyncrl_b200.h, include/asyncrl_b200_sarsa.h,
-include/asyncrl_b200_dueling.h, include/asyncrl_b200_double.h, include/asyncrl_b200_dueling_streams.h).
+include/asyncrl_b200_dueling.h, include/asyncrl_b200_double.h, include/asyncrl_b200_dueling_streams.h,
+include/asyncrl_b200_lstm.h).
 
 The product path has no CPU fallback: if the shared library is missing or a call
 fails, this module raises.  PyTorch is only the carrier of device memory and
@@ -145,6 +146,27 @@ STREAMS_OTHER = {
     "arl_streams_workspace_bytes": ([c_int], c_i64),
 }
 
+# the A3C LSTM agent: its own header (include/asyncrl_b200_lstm.h), its own tables
+LSTM_SIGNATURES = {
+    "arl_lstm_param_layout": [c_int, ctypes.POINTER(c_i64)],
+    "arl_prepare_weights_lstm": [c_vp, c_vp, c_int, c_vp],
+    "arl_lstm_step": [c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int,
+                      c_vp],
+    "arl_forward_lstm": [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                         c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_u64,
+                         c_vp],
+    "arl_heads_backward_lstm": [c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_vp],
+    "arl_lstm_backward": [c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                          c_vp, c_vp, c_vp, c_vp, c_f32, c_vp],
+    "arl_backward_lstm": [c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                          c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_f32,
+                          c_int, c_vp],
+}
+LSTM_OTHER = {
+    "arl_lstm_prepared_floats": ([], c_i64),
+    "arl_lstm_workspace_bytes": ([c_int], c_i64),
+}
+
 
 class ArlError(RuntimeError):
     pass
@@ -165,10 +187,10 @@ def load():
     lib = ctypes.CDLL(LIB_PATH)
     for name, argtypes in (list(SIGNATURES.items()) + list(SARSA_SIGNATURES.items())
                            + list(DUELING_SIGNATURES.items()) + list(DOUBLE_SIGNATURES.items())
-                           + list(STREAMS_SIGNATURES.items())):
+                           + list(STREAMS_SIGNATURES.items()) + list(LSTM_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes, fn.restype = argtypes, c_int
-    for name, (argtypes, restype) in list(OTHER.items()) + list(STREAMS_OTHER.items()):
+    for name, (argtypes, restype) in list(OTHER.items()) + list(STREAMS_OTHER.items()) + list(LSTM_OTHER.items()):
         fn = getattr(lib, name)
         fn.argtypes, fn.restype = argtypes, restype
     _lib = lib
@@ -234,6 +256,14 @@ def streams_param_layout(action_size):
     return list(off)
 
 
+def lstm_param_layout(action_size):
+    """Offsets (13) of the LSTM network's flat parameter buffer: arl_param_layout's 10 tensors, then lstm_w,
+    lstm_b."""
+    off = (c_i64 * 13)()
+    check(load().arl_lstm_param_layout(int(action_size), off), "arl_lstm_param_layout")
+    return list(off)
+
+
 def a2_block_rows(num_envs):
     """Rows of one a2 block (envs per forward launch): see arl_a2_block_rows."""
     return int(load().arl_a2_block_rows(int(num_envs)))
@@ -244,15 +274,19 @@ def launch_count(reset=False):
     return int(load().arl_launch_count(1 if reset else 0))
 
 
-def prepared_floats(streams=False):
+def prepared_floats(streams=False, lstm=False):
     """Size (floats) of the prepared-weights buffer arl_prepare_weights (``streams``:
-    arl_prepare_weights_streams) fills."""
+    arl_prepare_weights_streams, ``lstm``: arl_prepare_weights_lstm) fills."""
+    if lstm:
+        return int(load().arl_lstm_prepared_floats())
     if streams:
         return int(load().arl_streams_prepared_floats())
     return int(load().arl_prepared_floats())
 
 
-def workspace_bytes(action_size, streams=False):
+def workspace_bytes(action_size, streams=False, lstm=False):
+    if lstm:
+        return int(load().arl_lstm_workspace_bytes(int(action_size)))
     if streams:
         return int(load().arl_streams_workspace_bytes(int(action_size)))
     return int(load().arl_backward_workspace_bytes(int(action_size)))

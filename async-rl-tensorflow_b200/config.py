@@ -40,6 +40,9 @@ class AgentConfig(object):
                                          # Q learners (async_q, nstep_q, sarsa) on the nips trunk: p_w/p_b is the
                                          # advantage stream, q_w/q_b the value stream, both on fc256's output
                                          # (no hidden layer per stream); a3c refuses it
+    lstm = False                         # a3c only: Mnih et al. 2016's A3C LSTM agent, 256 LSTM cells between fc256
+                                         # and the heads (lstm_w/lstm_b), stepped in the rollout and trained by
+                                         # truncated BPTT over t_max steps; Q learners and the nature trunk refuse it
     dueling_streams = False              # with dueling: Wang et al.'s dueling architecture, each stream on its own
                                          # 256-wide hidden layer on conv2's output (value: l4_w/l4_b, advantage:
                                          # la_w/la_b); needs dueling=True, a3c and the nature trunk refuse it

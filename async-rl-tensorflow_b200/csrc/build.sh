@@ -4,7 +4,7 @@ set -euo pipefail
 cd "$(dirname "$0")"
 OUT=../libasyncrl_b200.so
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
-SRCS="api.cu preprocess.cu convs_tc.cu reduce.cu fc.cu heads.cu update.cu comm.cu nature.cu"
+SRCS="api.cu preprocess.cu convs_tc.cu reduce.cu fc.cu heads.cu update.cu comm.cu nature.cu lstm.cu"
 FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xcompiler -fvisibility=hidden"
 mkdir -p build
 pids=()

@@ -289,27 +289,11 @@ struct FcFwdClusterStreams : FcFwdCluster {
   }
 };
 
-template <class P>
-int run_gemm(tc::BulkGemmArgs& g, int k_splits, cudaStream_t st) {
-  if (k_splits < 1) k_splits = 1;
-  g.k_chunk = ((g.K + k_splits - 1) / k_splits + P::KB - 1) / P::KB * P::KB;
-  g.k_splits = (g.K + g.k_chunk - 1) / g.k_chunk;
-  g.m_tiles = (g.M + tc::kTileM - 1) / tc::kTileM;
-  g.n_tiles = (g.N + P::N_TILE - 1) / P::N_TILE;
-  return tc::launch<P>(g, g.m_tiles * g.n_tiles * g.k_splits, st);
-}
-
 // number of split-K slices the wgrad produces for K samples and a request of `want`
 int fc_wgrad_splits(int K, int want) {
   const int kb = FcWgrad::KB;
   const int k_chunk = ((K + want - 1) / want + kb - 1) / kb * kb;
   return (K + k_chunk - 1) / k_chunk;
-}
-
-static tc::SplitMat mat(const void* base, int rows, int block_rows, int chunks) {
-  tc::SplitMat m;
-  m.base = (const uint8_t*)base; m.rows = rows; m.block_rows = block_rows; m.chunks = chunks;
-  return m;
 }
 
 }  // namespace arl

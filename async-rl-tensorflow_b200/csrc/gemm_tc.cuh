@@ -1017,4 +1017,23 @@ struct BulkGemm : PolicyBase {
 };
 
 }  // namespace tc
+
+// Launch a BulkGemm instance on g (M, N, K, operands, D filled in): k_splits split-K slices over K,
+// slice z writing D + z*M*ldd
+template <class P>
+int run_gemm(tc::BulkGemmArgs& g, int k_splits, cudaStream_t st) {
+  if (k_splits < 1) k_splits = 1;
+  g.k_chunk = ((g.K + k_splits - 1) / k_splits + P::KB - 1) / P::KB * P::KB;
+  g.k_splits = (g.K + g.k_chunk - 1) / g.k_chunk;
+  g.m_tiles = (g.M + tc::kTileM - 1) / tc::kTileM;
+  g.n_tiles = (g.N + P::N_TILE - 1) / P::N_TILE;
+  return tc::launch<P>(g, g.m_tiles * g.n_tiles * g.k_splits, st);
+}
+
+inline tc::SplitMat mat(const void* base, int rows, int block_rows, int chunks) {
+  tc::SplitMat m;
+  m.base = (const uint8_t*)base; m.rows = rows; m.block_rows = block_rows; m.chunks = chunks;
+  return m;
+}
+
 }  // namespace arl

@@ -12,6 +12,7 @@
 #include "../../include/asyncrl_b200_dueling.h"
 #include "../../include/asyncrl_b200_double.h"
 #include "../../include/asyncrl_b200_dueling_streams.h"
+#include "../../include/asyncrl_b200_lstm.h"
 
 namespace arl {
 
@@ -469,8 +470,11 @@ __global__ void sarsa_lossgrad_kernel(const float* __restrict__ rewards,
 //   dhsT [hi|lo][ceil(N/8) sample chunks][256 column rows][8 samples]   fc wgrad's B operand
 //        (K-major over samples: one run = all 256 columns of 8 samples = 4 KB; samples >= N zero)
 // 32 samples are staged in shared memory so that a warp writes 512 contiguous bytes either way.
+// Relu = false (the LSTM network, include/asyncrl_b200_lstm.h: h = sigmoid(o) tanh(c) can be negative):
+// no mask, and d_h leaves as plain f32 [num_samples][256] in dhs (times tensor_scale), the form the
+// LSTM cell backward reads; dhsT is not written.
 constexpr int kHbChunk = 64, kHbSub = 32;
-template <int JMAX>
+template <int JMAX, bool Relu = true>
 __global__ void __launch_bounds__(256)
 heads_bwd_kernel(const float* __restrict__ pw, const float* __restrict__ qw,
                  const float* __restrict__ h, const float* __restrict__ dlogits,
@@ -521,8 +525,13 @@ heads_bwd_kernel(const float* __restrict__ pw, const float* __restrict__ qw,
               acc[j] = fmaf(hv, g, acc[j]);
             }
           }
-          dt[s][k] = hv > 0.f ? d * tensor_scale : 0.f;       // d_h leaves scaled (arl_backward)
+          dt[s][k] = !Relu || hv > 0.f ? d * tensor_scale : 0.f;       // d_h leaves scaled (arl_backward)
         }
+      }
+      if constexpr (!Relu) {                          // column k of the staging tile is this thread's own
+        __syncthreads();
+        for (int s = 0; s < ns; ++s) reinterpret_cast<float*>(dhs)[(c0 + s0 + s) * 256 + k] = dt[s][k];
+        continue;
       }
       __syncthreads();
       for (int v = k; v < 32 * kHbSub; v += 256) {
@@ -1079,16 +1088,16 @@ extern "C" int arl_observe_store_advance(const float* reward, const uint8_t* ter
   return ARL_OK;
 }
 
-extern "C" int arl_heads_backward(const float* params, int action_size, const float* h,
-                                  const float* dlogits, const float* dvalue, float* d_h,
-                                  float* grads, void* workspace, int64_t num_samples,
-                                  float tensor_scale, void* stream) {
-  ARL_REQUIRE(params && h && dlogits && dvalue && d_h && grads && workspace,
-              "arl_heads_backward: null pointer");
-  ARL_REQUIRE(tensor_scale > 0.f, "arl_heads_backward: tensor_scale must be > 0");
+// arl_heads_backward (Relu) and arl_heads_backward_lstm (fn: the entry's name, for errors)
+template <bool Relu>
+static int heads_backward(const char* fn, const float* params, int action_size, const float* h,
+                          const float* dlogits, const float* dvalue, float* d_h, float* grads, void* workspace,
+                          int64_t num_samples, float tensor_scale, void* stream) {
+  ARL_REQUIRE(params && h && dlogits && dvalue && d_h && grads && workspace, "%s: null pointer", fn);
+  ARL_REQUIRE(tensor_scale > 0.f, "%s: tensor_scale must be > 0", fn);
   ARL_REQUIRE(action_size >= 1 && action_size <= ARL_MAX_ACTIONS,
-              "arl_heads_backward: action_size %d outside [1,%d]", action_size, ARL_MAX_ACTIONS);
-  ARL_REQUIRE(num_samples >= 0, "arl_heads_backward: negative size");
+              "%s: action_size %d outside [1,%d]", fn, action_size, ARL_MAX_ACTIONS);
+  ARL_REQUIRE(num_samples >= 0, "%s: negative size", fn);
   cudaStream_t st = (cudaStream_t)stream;
   const ParamLayout L = param_layout(action_size);
   const int A = action_size, J = A + 1;
@@ -1107,11 +1116,27 @@ extern "C" int arl_heads_backward(const float* params, int action_size, const fl
   float* part = (float*)workspace;
   uint8_t* dhs = (uint8_t*)d_h;
   uint8_t* dhsT = dhs + (size_t)num_samples * 256 * sizeof(float);
-  auto kern = J <= 8 ? heads_bwd_kernel<8> : J <= 20 ? heads_bwd_kernel<20> : heads_bwd_kernel<ARL_MAX_ACTIONS + 1>;
+  auto kern = J <= 8 ? heads_bwd_kernel<8, Relu> : J <= 20 ? heads_bwd_kernel<20, Relu>
+                                                   : heads_bwd_kernel<ARL_MAX_ACTIONS + 1, Relu>;
   ARL_CUDA(launch_pdl(kern, dim3(grid), dim3(256), 0, st, params + L.off[T_PW], params + L.off[T_QW], h, dlogits,
                       dvalue, dhs, dhsT, part, num_samples, per, A, tensor_scale));
   ARL_LAUNCH_CHECK("heads_bwd_kernel");
   return reduce_partials(part, g, grid, 256 * J + J, st);
+}
+
+extern "C" int arl_heads_backward(const float* params, int action_size, const float* h,
+                                  const float* dlogits, const float* dvalue, float* d_h,
+                                  float* grads, void* workspace, int64_t num_samples,
+                                  float tensor_scale, void* stream) {
+  return heads_backward<true>("arl_heads_backward", params, action_size, h, dlogits, dvalue, d_h, grads, workspace,
+                              num_samples, tensor_scale, stream);
+}
+
+extern "C" int arl_heads_backward_lstm(const float* params, int action_size, const float* h_lstm,
+                                       const float* dlogits, const float* dvalue, float* d_h_lstm, float* grads,
+                                       void* workspace, int64_t num_samples, float tensor_scale, void* stream) {
+  return heads_backward<false>("arl_heads_backward_lstm", params, action_size, h_lstm, dlogits, dvalue, d_h_lstm,
+                               grads, workspace, num_samples, tensor_scale, stream);
 }
 
 extern "C" int arl_heads_backward_streams(const float* params, int action_size, const float* h,

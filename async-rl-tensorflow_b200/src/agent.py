@@ -62,6 +62,11 @@ class Agent(BaseModel):
             raise ValueError("double_q=True needs a learner that bootstraps from max_a Q (loss_mode 'async_q' or "
                              "'nstep_q'); loss_mode %r has no max to decouple"
                              % (getattr(config, 'loss_mode', 'a3c'),))
+        # config.py lstm: Mnih et al. 2016's A3C LSTM agent (Network.lstm), a policy/value network
+        self.lstm = bool(getattr(config, 'lstm', False))
+        if self.lstm and getattr(config, 'loss_mode', 'a3c') != 'a3c':
+            raise ValueError("lstm=True is the A3C LSTM agent (loss_mode 'a3c'); loss_mode %r has no recurrent form"
+                             % (getattr(config, 'loss_mode', 'a3c'),))
         # network.py:30-55: 'nips' (what agent.py:226-252 wires, the default) or 'nature'
         self.network = make_network(
             DQN_type=getattr(config, 'DQN_type', 'nips'), action_size=self.env.action_size, data_format=self.cnn_format,
@@ -70,7 +75,7 @@ class Agent(BaseModel):
             num_envs=self.num_envs, t_max=self.t_max, device=self.device, seed=self.seed,
             decay=self.decay, epsilon=self.epsilon, clip_norm=self.clip_norm,
             min_reward=self.min_reward, max_reward=self.max_reward, dueling=self.dueling, double_q=self.double_q,
-            dueling_streams=self.dueling_streams)
+            dueling_streams=self.dueling_streams, lstm=self.lstm)
         self.w = self.network.w
         # the per-cycle exchange runs inside the library (arl_comm_init / arl_backward(allreduce=1):
         # NCCL, bucketed so that the fc256 gradient travels while the conv backward kernels run);
@@ -139,6 +144,7 @@ class Agent(BaseModel):
         # agent.py:37-38: the stack starts as 4 copies of the first screen (K1, replicate=4)
         self.history.add(self.env.frames, replicate=self.history_length)
         self.t = 0
+        self.network.reset_lstm_state()                          # every game starts over: (h, c) = 0
         self.update_target_q_network()                           # main.py:92
         if self.has_target:
             self._last_target_sync = self.T
@@ -349,9 +355,14 @@ class Agent(BaseModel):
                                     ep_sched=self._ep_sched(), refresh=refresh)
             else:
                 net.forward_sample(self.history, t, 0, self.seed, self.env_id_base, step_dev=self.step_dev,
-                                   refresh=refresh)
+                                   refresh=refresh, **self._lstm_reset(t))
         self._run(('predict', t, self.history.head, refresh, take_pending), launches)
         return net.sampled_action[net._rows(t)]
+
+    def _lstm_reset(self, t):
+        """The ``reset`` argument of the LSTM forward entering rollout step ``t`` (none without an LSTM): the
+        terminal row of step t-1, for step 0 the previous rollout's last (a fixed row: the graph key t covers it)."""
+        return dict(reset=self.batch_terminal[(t - 1) % self.t_max]) if self.lstm else {}
 
     def _ep_sched(self):
         """agent.py:142-144's constants, for the epsilon the kernels evaluate from ``step_dev``."""
@@ -375,6 +386,7 @@ class Agent(BaseModel):
         for idx in range(int(n_episode)):
             self.env.new_random_game()
             test_history.add(self.env.frames, replicate=self.history_length)
+            self.network.reset_lstm_state(play=True)
             current = torch.zeros(self.num_envs, device=self.device)
             alive = torch.ones(self.num_envs, dtype=torch.bool, device=self.device)
             for _ in range(int(n_step)):
@@ -476,7 +488,8 @@ class Agent(BaseModel):
                                         self.seed, self._ep_sched(), self.env_id_base, allreduce=in_lib,
                                         target_refresh=target_refresh, refresh=refresh)
         else:
-            v_boot = net.bootstrap_value(hist, refresh=refresh)          # R = V(s_T), masked if terminal
+            v_boot = net.bootstrap_value(hist, refresh=refresh,          # R = V(s_T), masked if terminal
+                                         **self._lstm_reset(self.t_max))
             net.compute_gradients(hist, self.batch_reward, self.batch_terminal, v_boot, grad_scale=scale,
                                   allreduce=in_lib, refresh=False)
         if self.world_size > 1 and self.collective == 'torch':

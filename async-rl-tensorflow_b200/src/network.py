@@ -19,6 +19,9 @@ from .. import _cabi
 PARAM_NAMES = ("l1_w", "l1_b", "l2_w", "l2_b", "l4_w", "l4_b", "p_w", "p_b", "q_w", "q_b")
 # dueling streams (include/asyncrl_b200_dueling_streams.h): the advantage stream's hidden layer follows q_b
 STREAMS_PARAM_NAMES = PARAM_NAMES + ("la_w", "la_b")
+# the A3C LSTM agent (include/asyncrl_b200_lstm.h): the LSTM layer's kernel and bias follow q_b
+LSTM_PARAM_NAMES = PARAM_NAMES + ("lstm_w", "lstm_b")
+LSTM_CELLS = 256
 A1_ELEMS, A2_ELEMS, FC, DA1_ELEMS = 6400, 2592, 256, 7056
 A1_STORE = 3200                                               # float32 words of storage per sample of a1 (fp16)
 DA1_STORE = 3528                                              # ... of d_a1 (fp16 on the 21x21 grid)
@@ -63,23 +66,26 @@ def decode_da1(raw, n):
     return b.float().permute(1, 2, 3, 0, 4).reshape(n, 21, 21, 16)[:, :20, :20]
 
 
-def param_shapes(action_size, streams=False):
+def param_shapes(action_size, streams=False, lstm=False):
     shapes = OrderedDict([
         ("l1_w", (8, 8, 4, 16)), ("l1_b", (16,)), ("l2_w", (4, 4, 16, 32)), ("l2_b", (32,)),
         ("l4_w", (A2_ELEMS, FC)), ("l4_b", (FC,)), ("p_w", (FC, action_size)),
         ("p_b", (action_size,)), ("q_w", (FC, 1)), ("q_b", (1,))])
     if streams:
         shapes["la_w"], shapes["la_b"] = (A2_ELEMS, FC), (FC,)
+    if lstm:
+        shapes["lstm_w"], shapes["lstm_b"] = (FC + LSTM_CELLS, 4 * LSTM_CELLS), (4 * LSTM_CELLS,)
     return shapes
 
 
-def initial_weights(action_size, seed=123, stddev=0.02, streams=False):
+def initial_weights(action_size, seed=123, stddev=0.02, streams=False, lstm=False):
     """network.py:10 truncated_normal(0,.02) for convs, ops.py:36-39 normal(.02) for ``linear``
     matrices, zero biases (ops.py:24,38-39).  Returns an OrderedDict of CPU float32 tensors.
-    ``streams``: la_w / la_b too, drawn after the others (a plain network's weights do not change)."""
+    ``streams``: la_w / la_b too, drawn after the others (a plain network's weights do not change);
+    ``lstm``: lstm_w (like the ``linear`` matrices) / lstm_b the same way."""
     g = torch.Generator().manual_seed(int(seed))
     out = OrderedDict()
-    for name, shape in param_shapes(action_size, streams).items():
+    for name, shape in param_shapes(action_size, streams, lstm).items():
         if name.endswith("_b"):
             out[name] = torch.zeros(shape)
         elif name in ("l1_w", "l2_w"):
@@ -104,13 +110,17 @@ class Network(object):
     # ``dueling``, each stream on its own fc256 layer on a2 -- l4_w/l4_b the value stream's, la_w/la_b
     # (appended to the parameters) the advantage stream's; h (``l4``) is [N, 512] = [h_v | h_a].
     dueling_streams = False
+    # the A3C LSTM agent (Mnih et al. 2016, include/asyncrl_b200_lstm.h): 256 LSTM cells between fc256 and
+    # the heads, lstm_w/lstm_b appended to the parameters; each env carries (h, c) (``lstm_state``) from
+    # step to step, reset where the previous step was terminal.  a3c only; fixed for the network's life.
+    lstm = False
 
     def __init__(self, sess=None, data_format='NHWC', history_length=4, screen_height=84,
                  screen_width=84, action_size=6, activation_fn='relu', initializer=None,
                  gamma=0.99, beta=0.01, global_network=None, global_optim=None, DQN_type='nips',
                  num_envs=256, t_max=5, device='cuda', seed=123, decay=0.99, epsilon=0.1,
                  clip_norm=40.0, min_reward=-1.0, max_reward=1.0, dueling=False, double_q=False,
-                 dueling_streams=False):
+                 dueling_streams=False, lstm=False):
         if DQN_type.lower() != 'nips':
             raise ValueError("Network is the 'nips' trunk (network.py:43-52); DQN_type='nature' "
                              "(network.py:30-42) is network_nature.NatureNetwork -- use "
@@ -135,26 +145,31 @@ class Network(object):
         if self.dueling_streams and not self.dueling:
             raise ValueError("dueling_streams=True gives the dueling heads a hidden layer per stream; it needs "
                              "dueling=True")
-        S = self.dueling_streams
-        self.param_names = STREAMS_PARAM_NAMES if S else PARAM_NAMES
+        self.lstm = bool(lstm)
+        if self.lstm and (self.dueling or self.dueling_streams or self.double_q):
+            raise ValueError("lstm=True is the A3C LSTM agent (a policy/value network); it has no dueling or "
+                             "double-Q form")
+        S, L = self.dueling_streams, self.lstm
+        self.param_names = STREAMS_PARAM_NAMES if S else LSTM_PARAM_NAMES if L else PARAM_NAMES
 
         A, B, T = self.action_size, self.num_envs, self.t_max
-        self.offsets = _cabi.streams_param_layout(A) if S else _cabi.param_layout(A)
+        self.offsets = (_cabi.streams_param_layout(A) if S else _cabi.lstm_param_layout(A) if L
+                        else _cabi.param_layout(A))
         n_params = self.offsets[-1]
         dev = self.device
         self.params = torch.zeros(n_params, device=dev)
         self.grads = torch.zeros(n_params, device=dev)
         self.rms = torch.ones(n_params, device=dev)           # TF RMSProp slot starts at 1.0
         self.w, self.g = OrderedDict(), OrderedDict()
-        for i, (name, shape) in enumerate(param_shapes(A, S).items()):
+        for i, (name, shape) in enumerate(param_shapes(A, S, L).items()):
             self.w[name] = self.params[self.offsets[i]:self.offsets[i + 1]].view(shape)
             self.g[name] = self.grads[self.offsets[i]:self.offsets[i + 1]].view(shape)
         # the weights as the tensor-core kernels keep them resident (arl_prepare_weights); refreshed
         # lazily: the key is (tensor version, number of C-ABI writes) of the parameters it was made from
-        self.fc_w = torch.empty(_cabi.prepared_floats(S), device=dev)
+        self.fc_w = torch.empty(_cabi.prepared_floats(S, L), device=dev)
         self._fc_w_key = None
         self._param_writes = 0
-        self.set_weights(initial_weights(A, seed, streams=S))
+        self.set_weights(initial_weights(A, seed, streams=S, lstm=L))
         H = 2 * FC if S else FC                               # width of h (streams: [h_v | h_a])
 
         N = B * T
@@ -180,11 +195,56 @@ class Network(object):
         self.d_l4 = torch.empty(N + (N + 7) // 8 * 8, H, **f32)
         self.d_l2 = torch.empty(N, A2_ELEMS, **f32)
         self.d_l1 = torch.empty(N, DA1_STORE, **f32)          # fp16 on the 21x21 grid: see decode_da1
-        self.workspace = torch.empty(_cabi.workspace_bytes(A, S), dtype=torch.uint8, device=dev)
+        self.workspace = torch.empty(_cabi.workspace_bytes(A, S, L), dtype=torch.uint8, device=dev)
         self.loss_sums = torch.zeros(3, **f32)                # sum policy / value loss, entropy
         self.grad_norms = torch.zeros(len(self.param_names), **f32)
         self.events = {}
         self.tensor_scale = 1.0                               # set by compute_gradients
+        if L:
+            C = LSTM_CELLS
+            # the recurrent state the next rollout step reads (fixed addresses: CUDA-graph replay), and
+            # play's own, which Agent.play resets per episode
+            self.state_h, self.state_c = torch.zeros(B, C, **f32), torch.zeros(B, C, **f32)
+            self.play_h, self.play_c = torch.zeros(B, C, **f32), torch.zeros(B, C, **f32)
+            # per rollout step (include/asyncrl_b200_lstm.h): x = h_fc is ``l4``; xh one split block per step
+            self.xh = torch.empty(N, 2 * C, **f32)
+            self.lstm_z = torch.empty(B, 4 * C, **f32)
+            self.gates = torch.empty(N, 4 * C, **f32)
+            self.c_prev = torch.empty(N, C, **f32)
+            self.c_seq = torch.empty(N, C, **f32)
+            self.h_lstm = torch.empty(N, C, **f32)            # the heads' input
+            self._b.update(xh=torch.empty(B, 2 * C, **f32), h=torch.empty(B, C, **f32), c=torch.empty(B, C, **f32))
+            # BPTT scratch
+            self.d_h_lstm = torch.empty(N, C, **f32)
+            self.dz = torch.empty(N, 4 * C, **f32)
+            self.dxh = torch.empty(N, 2 * C, **f32)
+            self.dc = torch.empty(B, C, **f32)
+
+    # -- the LSTM state ---------------------------------------------------------------------
+    def lstm_state(self, play=False):
+        """(h, c) of every env, float32 [B, 256] each (copies): the state the next step reads; ``play``:
+        Agent.play's."""
+        if play:
+            return self.play_h.clone(), self.play_c.clone()
+        return self.state_h.clone(), self.state_c.clone()
+
+    def reset_lstm_state(self, play=False):
+        """Zero the recurrent state (a new game for every env)."""
+        if self.lstm:
+            for t in ((self.play_h, self.play_c) if play else (self.state_h, self.state_c)):
+                t.zero_()
+
+    def _forward_lstm(self, history, refresh, l1, l2, h_fc, state, reset, advance, xh, gates, c_prev, c, h, logits,
+                      probs, value, actions=None, env_id_base=0, step=0, step_dev=None, seed=0):
+        """arl_forward_lstm: one env step of the trunk, the LSTM step from ``state`` = (h, c) (``reset``: u8 [B],
+        nonzero = the env's previous step was terminal; advanced when ``advance``) and the heads on h."""
+        P = _cabi.ptr
+        self._timed_call("arl_forward_lstm", P(self.params), P(self.fc_w), int(bool(refresh)), self.action_size,
+                         P(history.ring), self.num_envs, history.ring_slots, history.first_slot(0), P(l1), P(l2),
+                         P(h_fc), P(state[0]), P(state[1]),
+                         P(reset), int(bool(advance)), P(xh), P(self.lstm_z), P(gates), P(c_prev), P(c), P(h),
+                         P(logits), P(probs), P(value), P(actions), int(env_id_base), int(step), P(step_dev),
+                         int(seed), _cabi.stream_ptr())
 
     # -- parameters -----------------------------------------------------------------------
     def set_weights(self, weights):
@@ -233,6 +293,8 @@ class Network(object):
         P, st = _cabi.ptr, _cabi.stream_ptr()
         if self.dueling_streams:
             _cabi.call("arl_prepare_weights_streams", P(params), P(fc_w), self.action_size, st)
+        elif self.lstm:
+            _cabi.call("arl_prepare_weights_lstm", P(params), P(fc_w), self.action_size, st)
         else:
             _cabi.call("arl_prepare_weights", P(params), P(fc_w), st)
 
@@ -292,20 +354,29 @@ class Network(object):
 
     def forward(self, history, t, refresh=None):
         """Forward of the current stack into rollout slot ``t``; returns (logits, policy, value)."""
+        self._not_lstm("forward")
         r = self._rows(t)
         self._forward_into(history, self.l1[r], self.l2[r], self.l4[r], self.policy_logits[r],
                            self.policy[r], self.value[r], refresh)
         return self.policy_logits[r], self.policy[r], self.value[r]
 
-    def forward_sample(self, history, t, step, seed, env_id_base=0, step_dev=None, refresh=None):
+    def forward_sample(self, history, t, step, seed, env_id_base=0, step_dev=None, refresh=None, reset=None):
         """``forward`` into rollout slot t + ``sample`` (network.py:72) as one composed call: the
         heads and the Philox draw run inside the fc256 kernel (arl_forward_sample).  The Philox step
-        is ``step`` (+ the int64 device counter ``step_dev`` when given)."""
+        is ``step`` (+ the int64 device counter ``step_dev`` when given).  ``lstm``: the LSTM step runs
+        between fc256 and the heads and advances the state; ``reset`` (u8 [B], None = none) marks the envs
+        whose previous step was terminal (arl_forward_lstm)."""
         self._policy_value_only("forward_sample")
         r = self._rows(t)
         P, st = _cabi.ptr, _cabi.stream_ptr()
         B, A = self.num_envs, self.action_size
         refresh = self._refresh(refresh)
+        if self.lstm:
+            self._forward_lstm(history, refresh, self.l1[r], self.l2[r], self.l4[r], (self.state_h, self.state_c),
+                               reset, True, self.xh[r], self.gates[r], self.c_prev[r], self.c_seq[r], self.h_lstm[r],
+                               self.policy_logits[r], self.policy[r], self.value[r], self.sampled_action[r],
+                               env_id_base, step, step_dev, seed)
+            return self.sampled_action[r]
         sd = P(step_dev) if step_dev is not None else None
         if self.timed is None:
             _cabi.call("arl_forward_sample", P(self.params), P(self.fc_w), refresh, A, P(history.ring), B,
@@ -368,10 +439,16 @@ class Network(object):
                          int(env_id_base), int(step), int(seed), _cabi.stream_ptr())
         return self.sampled_action[r]
 
-    def bootstrap_value(self, history, refresh=None):
-        """V(s_T) under the same theta (Algorithm 3: R = V(s_t, theta'_v))."""
+    def bootstrap_value(self, history, refresh=None, reset=None):
+        """V(s_T) under the same theta (Algorithm 3: R = V(s_t, theta'_v)).  ``lstm``: from the state after
+        the rollout's last step (with ``reset`` applied as in forward_sample), which is not advanced."""
         self._policy_value_only("bootstrap_value")
         b = self._b
+        if self.lstm:
+            self._forward_lstm(history, self._refresh(refresh), b['l1'], b['l2'], b['l4'],
+                               (self.state_h, self.state_c), reset, False, b['xh'], None, None, b['c'], b['h'],
+                               b['logits'], b['probs'], b['value'])
+            return b['value']
         self._forward_into(history, b['l1'], b['l2'], b['l4'], b['logits'], b['probs'], b['value'],
                            refresh)
         return b['value']
@@ -390,7 +467,11 @@ class Network(object):
         touched) and one action per env: epsilon-greedy over the Q values when ``ep`` is given
         (agent.py:141-151), else a sample from the policy (network.py:72).  Used by Agent.play."""
         b = self._b
-        self._forward_into(history, b['l1'], b['l2'], b['l4'], b['logits'], b['probs'], b['value'])
+        if self.lstm:                                          # play's own state (reset_lstm_state(play=True))
+            self._forward_lstm(history, self._refresh(None), b['l1'], b['l2'], b['l4'], (self.play_h, self.play_c),
+                               None, True, b['xh'], None, None, b['c'], b['h'], b['logits'], b['probs'], b['value'])
+        else:
+            self._forward_into(history, b['l1'], b['l2'], b['l4'], b['logits'], b['probs'], b['value'])
         if 'action' not in b:
             b['action'] = torch.zeros(self.num_envs, dtype=torch.int32, device=self.device)
         if ep is not None:
@@ -432,7 +513,33 @@ class Network(object):
                          _cabi.ptr(v_boot), _cabi.ptr(self.R), _cabi.ptr(self.d_logits),
                          _cabi.ptr(self.d_value), _cabi.ptr(self.loss_sums), T, B, A, self.gamma,
                          self.beta, self.min_reward, self.max_reward, float(grad_scale), st)
+        if self.lstm:
+            return self._backward_lstm(history, terminals, grad_scale, allreduce, refresh)
         return self._backward(history, grad_scale, allreduce, refresh)
+
+    def _backward_lstm(self, history, terminals, grad_scale, allreduce, refresh):
+        """arl_backward_lstm: heads (unmasked), truncated BPTT over the rollout (``terminals`` u8 [T, B] reset
+        the state between steps) and the LSTM weight gradient, then the trunk's backward; one entry."""
+        T, B, A = self.t_max, self.num_envs, self.action_size
+        P = _cabi.ptr
+        if self._refresh(refresh):
+            self._prepare(self.params, self.fc_w)
+        S = self.tensor_scale = self.pick_tensor_scale(grad_scale)
+        self._timed_call("arl_backward_lstm", P(self.params), P(self.fc_w), A, P(history.ring), B, history.ring_slots,
+                         history.first_slot(T), T, P(terminals), P(self.l1), P(self.l2), P(self.l4), P(self.xh),
+                         P(self.gates), P(self.c_prev), P(self.c_seq), P(self.h_lstm), P(self.d_logits),
+                         P(self.d_value), P(self.d_h_lstm), P(self.dz), P(self.dxh), P(self.dc), P(self.d_l4),
+                         P(self.d_l2), P(self.d_l1), P(self.grads), P(self.workspace), S, 1 if allreduce else 0,
+                         _cabi.stream_ptr())
+        return self.grads
+
+    def _not_lstm(self, entry):
+        """The Q-learner entry points and the plain forward run the heads on fc256's output; an LSTM network's
+        heads read the LSTM's h, which only the A3C entries (forward_sample, bootstrap_value, evaluate,
+        compute_gradients) compute."""
+        if self.lstm:
+            raise ValueError("Network.%s has no LSTM form; an LSTM network (lstm=True) serves the A3C learner "
+                             "only" % entry)
 
     def _policy_value_only(self, entry):
         """The A3C entry points (policy sample, V(s_T) bootstrap, policy/value loss) have no dueling
@@ -492,6 +599,7 @@ class Network(object):
         evaluates the target network on the B states s_T only (``q_boot``).  ``next_actions``
         (sarsa): the rollout's actions get one more row, a_T, the action taken in s_T
         (``sarsa_actions`` [(T+1)*B]; ``sampled_action`` becomes a view of its first T rows)."""
+        self._not_lstm("make_target")
         self.target_params = self.params.clone()
         B, A = self.num_envs, self.action_size
         N = B * self.t_max
@@ -545,6 +653,7 @@ class Network(object):
         """agent.py:186-197: target-network forward over s_1..s_T, 1-step targets, MSE gradient,
         backward.  The backward scratch buffers hold the target activations meanwhile.  Double Q: the
         online rows of s_1..s_{T-1} are the rollout's own Q rows, Q(s_T; theta) one more forward."""
+        self._not_lstm("compute_q_gradients")
         T, B, A = self.t_max, self.num_envs, self.action_size
         P, st = _cabi.ptr, _cabi.stream_ptr()
         probs, value = self._tq_scratch
@@ -602,6 +711,7 @@ class Network(object):
         int64 device counter ``step_dev`` the step is ``step`` + *step_dev and epsilon is agent.py:142-144
         evaluated on the device from it with ``ep_sched`` = (ep_start, ep_end, ep_end_t, learn_start);
         without it the step is ``step`` and epsilon is ``ep``."""
+        self._not_lstm("forward_egreedy")
         r = self._rows(t)
         P, st = _cabi.ptr, _cabi.stream_ptr()
         refresh = self._refresh(refresh)
@@ -628,6 +738,7 @@ class Network(object):
         actions (arl_nstep_q_lossgrad), then the backward (agent.py:317).  ``history`` must have had
         exactly t_max pushes since s_0.  Double Q: first the online forward of s_T (``q_online_T``,
         with ``refresh``), and R_T = q_boot[a*], a* = argmax_a q_online_T (arl_double_nstep_q_lossgrad)."""
+        self._not_lstm("compute_nstep_q_gradients")
         T, B, A = self.t_max, self.num_envs, self.action_size
         P, st = _cabi.ptr, _cabi.stream_ptr()
         b = self._b
@@ -673,6 +784,7 @@ class Network(object):
              (arl_sarsa_lossgrad);
           4. the backward (agent.py:317).
         ``history`` must have had exactly t_max pushes since s_0."""
+        self._not_lstm("compute_sarsa_gradients")
         T, B, A = self.t_max, self.num_envs, self.action_size
         P, st = _cabi.ptr, _cabi.stream_ptr()
         b = self._b
@@ -720,7 +832,8 @@ class Network(object):
                          _cabi.ptr(self.grad_norms), _cabi.ptr(self.workspace), _cabi.stream_ptr())
 
     def _layout_update(self, lr, step_dev, step_offset, base_lr, max_step):
-        """K5 over the tensors of ``offsets`` (arl_clip_rmsprop_layout): the dueling streams' 12 tensors."""
+        """K5 over the tensors of ``offsets`` (arl_clip_rmsprop_layout): the dueling streams' or the LSTM
+        network's 12 tensors."""
         import ctypes
         if not hasattr(self, '_offsets_c'):
             self._offsets_c = (ctypes.c_int64 * len(self.offsets))(*self.offsets)
@@ -735,7 +848,7 @@ class Network(object):
         the gradient over the ranks first, inside the same kernels (NVLink peer memory)."""
         if exchange:
             self._exchange_update(lr, None, 0, 0.0, 1)
-        elif self.dueling_streams:
+        elif self.dueling_streams or self.lstm:
             self._layout_update(lr, None, 0, 0.0, 1)
         else:
             self._timed_call("arl_clip_rmsprop", _cabi.ptr(self.params), _cabi.ptr(self.rms),
@@ -750,7 +863,7 @@ class Network(object):
         from the int64 step counter ``step_dev`` (+ ``step_offset``): replayable by a CUDA graph."""
         if exchange:
             self._exchange_update(0.0, step_dev, step_offset, base_lr, max_step)
-        elif self.dueling_streams:
+        elif self.dueling_streams or self.lstm:
             self._layout_update(0.0, step_dev, step_offset, base_lr, max_step)
         else:
             self._timed_call("arl_clip_rmsprop_sched", _cabi.ptr(self.params), _cabi.ptr(self.rms),
@@ -771,6 +884,8 @@ class Network(object):
             blobs["dueling"] = np.bool_(True)
         if self.dueling_streams:                               # absent = no hidden layer per stream
             blobs["dueling_streams"] = np.bool_(True)
+        if self.lstm:                                          # absent = no LSTM; the (h, c) state is not saved
+            blobs["lstm"] = np.bool_(True)
         np.savez(path, **blobs)
         return path
 
@@ -792,6 +907,10 @@ class Network(object):
             raise ValueError("checkpoint %s was written by a %s network; this network is %s"
                              % (files[-1], "dueling_streams" if saved else "non-dueling_streams",
                                 "dueling_streams" if self.dueling_streams else "non-dueling_streams"))
+        saved = bool(z["lstm"]) if "lstm" in z.files else False
+        if saved != self.lstm:                                 # other parameters: refuse
+            raise ValueError("checkpoint %s was written by a %s network; this network is %s"
+                             % (files[-1], "lstm" if saved else "non-lstm", "lstm" if self.lstm else "non-lstm"))
         self.set_weights({k: z[k] for k in self.param_names})
         self.rms.copy_(torch.as_tensor(z["rms"]))
         self.loaded_step = int(z["step"])
@@ -811,6 +930,9 @@ def make_network(DQN_type='nips', **kw):
         if kw.pop('dueling_streams', False):
             raise NotImplementedError("dueling streams are built on the nips trunk (agent.py:226-252); the "
                                       "nature trunk is A3C-only")
+        if kw.pop('lstm', False):
+            raise NotImplementedError("the A3C LSTM agent is built on the nips trunk (agent.py:226-252); the nature "
+                                      "trunk has no LSTM")
         if kw.pop('double_q', False):
             raise NotImplementedError("double Q-learning targets are built on the nips trunk (agent.py:226-252); "
                                       "the nature trunk is A3C-only")

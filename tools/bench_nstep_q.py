@@ -3,7 +3,8 @@ async_q eager (its own path: host epsilon, a separate draw launch, a target forw
 states; sarsa runs that target forward too, inside its graph).
 
     python tools/bench_nstep_q.py [--rounds R] [--cycles K] [--modes a3c,nstep_q,...] [--dueling off|on|both]
-                                  [--double off|on|both] [--dueling-streams off|on|both] [--out FILE]
+                                  [--double off|on|both] [--dueling-streams off|on|both] [--lstm off|on|both]
+                                  [--out FILE]
 
 For each shape (envs x t_max x actions: 4096 x 5 x 6 and 16384 x 20 x 18) one agent per mode is built
 and warmed up until a whole ring period has replayed without a new graph capture; then the modes take
@@ -46,6 +47,49 @@ def card():
         return {"name": torch.cuda.get_device_name(), "power_limit": "unknown (%s)" % str(e)[:80]}
 
 
+def lstm_entry_times(pkg, agent, reps):
+    """GPU time of each new LSTM entry on the network's own buffers after the timed cycles (a CUDA event pair
+    around ``reps`` back-to-back calls; the state is not advanced), with the bytes each must move at the
+    least, counted from the shapes, and the rate that gives.  Per row of B envs (one step) or N = T*B samples:
+      arl_lstm_step      read h_fc, h (2 KB), write xh (2 KB); GEMM read xh (2 KB), write z (4 KB); cell read
+                         z, c (5 KB), write gates, c_prev, c, h (7 KB)                                = 22 KB
+      arl_heads_backward_lstm  read h (1 KB), write d_h_lstm (1 KB)                                 =  2 KB
+      arl_lstm_backward  cell bwd read d_h_lstm, dh_rec, dc, gates, c_prev, c (9 KB), write dz, dc (5 KB);
+                         dgrad read dz (4 KB), write dxh (2 KB); wgrad read xh, dz (6 KB); dx hand-over read
+                         dx, h_fc (2 KB), write d_h twice (2 KB)                                      = 30 KB
+    (+ the 4 MB of weight images and the wgrad's 8 MB of partials, read back once)."""
+    P, st, net = pkg._cabi.ptr, pkg._cabi.stream_ptr(), agent.network
+    B, T, A = net.num_envs, net.t_max, net.action_size
+    N, b = B * T, net._b
+    calls = {
+        "arl_lstm_step": (lambda: pkg._cabi.call(
+            "arl_lstm_step", P(net.params), P(net.fc_w), A, P(net.l4[:B]), P(net.state_h), P(net.state_c), None, 0,
+            P(b["xh"]), P(net.lstm_z), P(net.gates[:B]), P(net.c_prev[:B]), P(b["c"]), P(b["h"]), B, st),
+            B * 22 * 1024 + 4 * 2 ** 20),
+        "arl_heads_backward_lstm": (lambda: pkg._cabi.call(
+            "arl_heads_backward_lstm", P(net.params), A, P(net.h_lstm), P(net.d_logits), P(net.d_value),
+            P(net.d_h_lstm), P(net.grads), P(net.workspace), N, 64.0, st), N * 2 * 1024),
+        "arl_lstm_backward": (lambda: pkg._cabi.call(
+            "arl_lstm_backward", P(net.params), P(net.fc_w), A, B, T, P(agent.batch_terminal), P(net.l4), P(net.xh),
+            P(net.gates), P(net.c_prev), P(net.c_seq), P(net.d_h_lstm), P(net.dz), P(net.dxh), P(net.dc),
+            P(net.d_l4), P(net.grads), P(net.workspace), 64.0, st), N * 30 * 1024 + 12 * 2 ** 20),
+    }
+    out = {}
+    for name, (fn, nbytes) in calls.items():
+        fn()                                                     # warm
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(reps):
+            fn()
+        e1.record()
+        torch.cuda.synchronize()
+        ms = e0.elapsed_time(e1) / reps
+        out[name] = {"ms": round(ms, 4), "min_bytes": nbytes, "GB_per_s": round(nbytes / ms / 1e6, 1),
+                     "launches_per_call": {"arl_lstm_step": 3, "arl_heads_backward_lstm": 2,
+                                           "arl_lstm_backward": 2 * T + 4}[name]}
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rounds", type=int, default=5)
@@ -59,13 +103,18 @@ def main():
     ap.add_argument("--dueling-streams", default="off", choices=("off", "on", "both"),
                     help="a hidden layer per dueling stream (reported as \"<mode>+streams\"): off, on, or both "
                          "(each Q learner plain, with dueling heads and with dueling streams)")
+    ap.add_argument("--lstm", default="off", choices=("off", "on", "both"),
+                    help="the A3C LSTM agent for the a3c mode (reported as \"a3c+lstm\"): off, on, or both; with the "
+                         "flag on, the GPU time of each new LSTM entry is recorded too")
     ap.add_argument("--out", default=None, help="default: profiles/r05_sarsa_bench.json, "
                                                 "profiles/r06_dueling_bench.json with --dueling on|both, "
                                                 "profiles/r08_double_q_bench.json with --double on|both, or "
-                                                "profiles/r09_dueling_streams_bench.json with --dueling-streams on|both")
+                                                "profiles/r09_dueling_streams_bench.json with --dueling-streams on|both, "
+                                                "or profiles/r11_lstm_bench.json with --lstm on|both")
     args = ap.parse_args()
     if args.out is None:
-        args.out = os.path.join(ROOT, "profiles", "r09_dueling_streams_bench.json" if args.dueling_streams != "off"
+        args.out = os.path.join(ROOT, "profiles", "r11_lstm_bench.json" if args.lstm != "off"
+                                else "r09_dueling_streams_bench.json" if args.dueling_streams != "off"
                                 else "r08_double_q_bench.json" if args.double != "off"
                                 else "r05_sarsa_bench.json" if args.dueling == "off" else "r06_dueling_bench.json")
     if not torch.cuda.is_available():
@@ -75,7 +124,8 @@ def main():
     torch.cuda.set_device(dev)
     modes = []
     for m in args.modes.split(","):
-        heads = [""] if m == "a3c" else {"off": [""], "on": ["+dueling"], "both": ["", "+dueling"]}[args.dueling]
+        heads = ({"off": [""], "on": ["+lstm"], "both": ["", "+lstm"]}[args.lstm] if m == "a3c"
+                 else {"off": [""], "on": ["+dueling"], "both": ["", "+dueling"]}[args.dueling])
         if m != "a3c" and args.dueling_streams != "off":
             heads = {"on": ["+streams"], "both": ["", "+dueling", "+streams"]}[args.dueling_streams]
         targets = ([""] if m not in ("async_q", "nstep_q")
@@ -90,7 +140,8 @@ def main():
         for mode in modes:
             cfg = pkg.config.get_config({"model": "m1", "num_envs": B, "t_max": T, "loss_mode": mode.split("+")[0],
                                          "dueling": "+dueling" in mode or "+streams" in mode,
-                                         "dueling_streams": "+streams" in mode, "double_q": mode.endswith("+double")})
+                                         "dueling_streams": "+streams" in mode, "double_q": mode.endswith("+double"),
+                                         "lstm": "+lstm" in mode})
             env = pkg.GymEnvironment(cfg, env=pkg.SyntheticAtari(B, A, seed=123, pool=pool, device=dev), device=dev)
             agent = pkg.Agent(cfg, env, device=dev)
             random.seed(cfg.seed)
@@ -133,6 +184,9 @@ def main():
             entry["modes"][mode] = {"ms_per_cycle": round(med, 4), "ms_min": round(min(ms[mode]), 4),
                                     "ms_max": round(max(ms[mode]), 4), "frames_per_sec": round(B * T / med * 1e3),
                                     "graph_replayed": bool(agent.graph_replays), "graphs": len(agent._graphs)}
+        for mode in modes:
+            if "+lstm" in mode:
+                entry["modes"][mode]["entries"] = lstm_entry_times(pkg, agents[mode][0], args.cycles)
         if "a3c" in modes:
             for mode in modes:
                 entry["modes"][mode]["vs_a3c"] = round(entry["modes"][mode]["ms_per_cycle"] /
